@@ -3,6 +3,8 @@
 
   python bench.py --gpus N --steps K --warmup W            # this repo (hand-written sm_100a kernels)
   python bench.py --impl reference --gpus N --steps K ...  # the UNMODIFIED reference's torch code on the host cores
+  python bench.py ... --dump-outputs DIR                   # also write the last timed step's outputs as DIR/<name>.npy, so
+                                                           # that two builds can be compared on identical seeded inputs
 
 Workload (BASELINE.json configs[3], one rank's share = configs[2] plus the device-side reset path): 131,072 envs per GPU
 (`--envs`; 65,536 when the GPU has less than 60 GB free; `--envs 4096` = configs[1]), full dense+sparse heightmap (1634
@@ -32,6 +34,8 @@ PEAKS_FILE = os.path.join(ROOT, "MEASURED_PEAKS.json")
 FALLBACK_HBM_GBS = 6650.0                 # /opt/skills/guides/B200_PROFILING.md fallback
 METRIC = "env-steps/sec (obs+kinematics+reward)"
 C4_ENVS_PER_GPU = 131072                  # BASELINE.json configs[3]: 1,048,576 envs over 8 GPUs
+DUMP_ENVS = 8192                          # --dump-outputs: envs sampled; their obs rows alone are 8192 x 1750 f32 = 57 MB
+DUMP_MAX_BYTES = 64 * 10 ** 6
 
 
 _JSON_FD = None
@@ -331,6 +335,26 @@ def time_policy_epilogue(R, obs, steps=20, warmup=3):
 
 
 # ------------------------------------------------------------------------------------------------ B200 arm
+def last_step_outputs(task, stats):
+    """What the last timed step returned to its caller (hot_step: obs, rew, reset, extras), the joint targets it computed for
+    the simulator and the step's reduced statistics, as host arrays (float32; float64 for the statistics and for integers).
+    The per-env arrays keep a fixed, seeded sample of DUMP_ENVS envs, sorted; `env_ids` holds their indices."""
+    N = task.num_envs
+    ids = torch.randperm(N, generator=torch.Generator().manual_seed(0))[:DUMP_ENVS].sort().values
+    ids_d = ids.to(task.obs_buf.device)
+    per_env = {"obs": task.obs_buf, "rew": task.rew_buf, "reset": task.reset_buf,
+               "joint_position_targets": task.joint_position_targets, "joint_velocity_targets": task.joint_velocity_targets}
+    per_env.update({"extras_" + k: v for k, v in task.extras.items()})
+    out = {"env_ids": ids.double().numpy(), "stats": stats.double().cpu().numpy()}
+    for name, t in per_env.items():
+        t = t[ids_d].cpu()
+        out[name] = (t.float() if t.is_floating_point() and t.dtype != torch.float64 else t.double()).numpy()
+    nbytes = sum(a.nbytes for a in out.values())
+    if nbytes > DUMP_MAX_BYTES:
+        raise RuntimeError("--dump-outputs: %d bytes exceed the %d-byte limit" % (nbytes, DUMP_MAX_BYTES))
+    return out
+
+
 def run_b200(args, rank, world, local):
     import isaac_rover_b200 as R
     from isaac_rover_b200 import synth
@@ -399,6 +423,10 @@ def run_b200(args, rank, world, local):
     torch.cuda.synchronize()
     R.dist.barrier()
     launches = R._lib.launch_count - launches0
+    # taken before the passes below reuse the task's buffers
+    dumped = None
+    if args.dump_outputs and rank == 0:
+        dumped = last_step_outputs(task, task.stats if args.sync_reduce else reducer.result((reducer.i - 1) % reducer.depth))
     dt = R.dist.max_over_ranks(e0.elapsed_time(e1) * 1e-3, dev)
     reset_counts = task.reset_counters.cpu().tolist()
     ray_ms = [a.elapsed_time(b) for a, b in task.Camera.timing]
@@ -563,6 +591,11 @@ def run_b200(args, rank, world, local):
             line["policy_epilogue"] = time_policy_epilogue(R, task.obs_buf)
         except Exception as e:          # reported beside the step, never a reason to lose the bench line
             line["policy_epilogue"] = {"unavailable": str(e)[:200]}
+    if dumped is not None:
+        import numpy as np
+        os.makedirs(args.dump_outputs, exist_ok=True)
+        for name, a in dumped.items():
+            np.save(os.path.join(args.dump_outputs, name + ".npy"), a)
     emit(line)
 
 
@@ -586,7 +619,13 @@ def main():
     ap.add_argument("--no-numa", action="store_true", help="do not bind the process to the CPUs local to its GPU")
     ap.add_argument("--unfused", action="store_true", help="one library call per reference call instead of rvb_env_step")
     ap.add_argument("--sync-reduce", action="store_true", help="all-reduce the statistics on the compute stream every step")
+    ap.add_argument("--dump-outputs", metavar="DIR", help="write what the last timed step computed as DIR/<name>.npy (rank 0's "
+                    "envs; obs, rew, reset, extras and joint targets of %d seeded sample envs, the reduced statistics)" % DUMP_ENVS)
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl != "b200":
+        ap.error("--dump-outputs writes the outputs of --impl b200")
     args.warmup = max(args.warmup, 1 if args.impl == "reference" else 3)
     rank = int(os.environ.get("RANK", "0"))
     world = int(os.environ.get("WORLD_SIZE", "1"))

@@ -142,16 +142,14 @@ def test_oracle_matches_reference_fresh_world():
     assert torch.equal(s2, steer) and torch.equal(v2, vel)
 
 
-@needs_ref
-@pytest.mark.reference
-def test_product_pattern_matches_reference():
-    import isaac_rover_b200
+def test_product_pattern_matches_reference(golden):
+    """The product's pattern against the reference Heightmap's distribution / coarse_idx / fine_idx, as make_golden.py stored
+    them."""
+    import isaac_rover_b200  # noqa: F401
     from isaac_rover_b200.heightmap_distribution import build_pattern
-    ns = ref_import.load("cpu")
-    hm = ns.Heightmap("cpu")
     pts, ci, fi = build_pattern()
-    assert torch.equal(torch.from_numpy(pts), hm.distribution)
-    assert torch.equal(torch.from_numpy(ci), hm.coarse_idx) and torch.equal(torch.from_numpy(fi), hm.fine_idx)
+    assert torch.equal(torch.from_numpy(pts), golden["ref_pattern"])
+    assert torch.equal(torch.from_numpy(ci), golden["ref_coarse_idx"]) and torch.equal(torch.from_numpy(fi), golden["ref_fine_idx"])
 
 
 def test_golden_spawn_direct_path():

@@ -11,6 +11,7 @@ sys.path.insert(0, ROOT)
 from oracle import policy_oracle, ref_import  # noqa: E402
 
 GOLDEN = os.path.join(ROOT, "tests", "golden", "policy_golden.pt")
+GOLDEN_THREADS = 8
 
 
 def _gen():
@@ -21,9 +22,16 @@ def _gen():
 
 
 def test_golden_fixture_matches_oracle_bit_for_bit():
+    """The fixture was computed by torch's fp32 CPU matmul on GOLDEN_THREADS threads; the CPU BLAS splits the work by thread
+    count, so the same bits come out only with that count."""
     g = torch.load(GOLDEN)["leakyrelu"]
-    mean = policy_oracle.forward(g["actor_sd"], g["obs"], 4, 634, 1112, "leakyrelu", actor=True)
-    value = policy_oracle.forward(g["critic_sd"], g["obs"], 4, 634, 1112, "leakyrelu", actor=False)
+    threads = torch.get_num_threads()
+    torch.set_num_threads(GOLDEN_THREADS)
+    try:
+        mean = policy_oracle.forward(g["actor_sd"], g["obs"], 4, 634, 1112, "leakyrelu", actor=True)
+        value = policy_oracle.forward(g["critic_sd"], g["obs"], 4, 634, 1112, "leakyrelu", actor=False)
+    finally:
+        torch.set_num_threads(threads)
     assert mean.shape == (70, 2) and value.shape == (70, 1)
     assert torch.equal(mean, g["mean"]) and torch.equal(value, g["value"])
     assert torch.equal(g["log_std"], torch.zeros(2))                       # model.py:178
