@@ -194,6 +194,15 @@ __device__ __forceinline__ uint32_t min_key(__half k, uint32_t slot) {
     return (key << 16) | slot;
 }
 
+// Two fp32 FMAs in one issue slot (Blackwell FFMA2: d.xy = a.xy * b + d.xy; ptxas folds the {b, b} pair into the
+// instruction's broadcast operand).  Each half is an IEEE fma, so the result equals two fmaf() calls bit for bit.
+__device__ __forceinline__ void ffma2(float& d0, float& d1, float a0, float a1, float b) {
+    asm("{\n\t.reg .b64 ra, rb, rc;\n\tmov.b64 ra, {%2, %3};\n\tmov.b64 rb, {%4, %4};\n\tmov.b64 rc, {%0, %1};\n\t"
+        "fma.rn.f32x2 rc, ra, rb, rc;\n\tmov.b64 {%0, %1}, rc;\n\t}"
+        : "+f"(d0), "+f"(d1)
+        : "f"(a0), "f"(a1), "f"(b));
+}
+
 // f64 -> fp16 the way torch casts (double -> float -> half, two roundings) (camera.py:212)
 __device__ __forceinline__ __half h_from_double(double v) { return __float2half_rn(__double2float_rn(v)); }
 

@@ -96,15 +96,6 @@ __device__ __forceinline__ void pl_act16(float* v, int kind) {
     }
 }
 
-// Two fp32 FMAs in one issue slot (Blackwell FFMA2: d.xy = a.xy * b + c.xy; ptxas folds the {b, b} pair into the
-// instruction's broadcast operand).  Each half is an IEEE fma, so the result equals two fmaf() calls bit for bit.
-__device__ __forceinline__ void ffma2(float& d0, float& d1, float a0, float a1, float b) {
-    asm("{\n\t.reg .b64 ra, rb, rc;\n\tmov.b64 ra, {%2, %3};\n\tmov.b64 rb, {%4, %4};\n\tmov.b64 rc, {%0, %1};\n\t"
-        "fma.rn.f32x2 rc, ra, rb, rc;\n\tmov.b64 {%0, %1}, rc;\n\t}"
-        : "+f"(d0), "+f"(d1)
-        : "f"(a0), "f"(a1), "f"(b));
-}
-
 // torch [out][in] -> k-major padded panel
 __global__ void pl_pack_kernel(const float* __restrict__ w, const float* __restrict__ b, int in, int out, int outp,
                                float* __restrict__ wt, float* __restrict__ bias) {
@@ -232,7 +223,7 @@ template <bool F2>
 __global__ void __launch_bounds__(PL_THREADS, 2)
 policy_forward_kernel(const PolicyDev* __restrict__ p0, const PolicyDev* __restrict__ p1, const float* __restrict__ obs,
                       int64_t obs_ld, int64_t N, float* __restrict__ out0, int64_t out0_ld, float* __restrict__ out1,
-                      int64_t out1_ld, const float* __restrict__ h1, int h1_nets) {
+                      int64_t out1_ld) {
     // blockIdx.y selects the network (actor / critic of one PPO step read the same obs tile, hot in L2)
     const PolicyDev& P = *(blockIdx.y ? p1 : p0);
     float* __restrict__ out = blockIdx.y ? out1 : out0;
@@ -252,24 +243,11 @@ policy_forward_kernel(const PolicyDev* __restrict__ p0, const PolicyDev* __restr
         const int m = tid & 31, k = tid >> 5;
         A[k * PL_LDA + m] = (m0 + m < N) ? __ldg(obs + (m0 + m) * obs_ld + k) : 0.f;
     }
-    // h1 (optional): the first layer of both encoders, already computed by policy_l1_tc_kernel:
-    // h1[env][enc * 80 * nets + net * 80 + k] -> Cb[k][env]
-    auto load_h1 = [&](int enc) {
-        const int ld = 2 * PL_E1 * h1_nets, off = enc * PL_E1 * h1_nets + (int)blockIdx.y * PL_E1;
-        for (int i = tid; i < PL_TM * PL_E1; i += PL_THREADS) {
-            const int m = i / PL_E1, k = i % PL_E1;
-            Cb[k * PL_LDA + m] = (m0 + m < N) ? __ldg(h1 + (m0 + m) * ld + off + k) : 0.f;
-        }
-    };
     // sparse encoder (model.py:186) -> concat rows p .. p+59
-    if (h1) load_h1(0);
-    else pl_dense<3, true, F2>(nullptr, obs, obs_ld, m0, N, p, P.n_sparse, P.es1, xs, ws, Cb, P.act);
+    pl_dense<3, true, F2>(nullptr, obs, obs_ld, m0, N, p, P.n_sparse, P.es1, xs, ws, Cb, P.act);
     pl_dense<2, false, F2>(Cb, nullptr, 0, 0, 0, 0, PL_E1, P.es2, xs, ws, A + p * PL_LDA, P.act);
     // dense encoder (model.py:187) -> concat rows p+60 .. p+119
-    if (h1) {
-        __syncthreads();          // every thread is done reading Cb
-        load_h1(1);
-    } else pl_dense<3, true, F2>(nullptr, obs, obs_ld, m0, N, p + P.n_sparse, P.n_dense, P.ed1, xs, ws, Cb, P.act);
+    pl_dense<3, true, F2>(nullptr, obs, obs_ld, m0, N, p + P.n_sparse, P.n_dense, P.ed1, xs, ws, Cb, P.act);
     pl_dense<2, false, F2>(Cb, nullptr, 0, 0, 0, 0, PL_E1, P.ed2, xs, ws, A + (p + PL_E2) * PL_LDA, P.act);
     // MLP (model.py:190-191)
     pl_dense<8, false, F2>(A, nullptr, 0, 0, 0, 0, p + 2 * PL_E2, P.m1, xs, ws, B, P.act);
@@ -304,7 +282,7 @@ policy_forward_kernel(const PolicyDev* __restrict__ p0, const PolicyDev* __restr
 //     stage's mbarrier; warp 4 issues the MMAs (M = 128, N = 80 per network, K = 8) and commits them to the stage's "empty"
 //     barrier.  Three stages of 32 KB (A hi + lo) + 20 KB per network (W hi + lo).  Both networks of a PPO step share the A tiles.
 // Output: h1 [N][nets * 160] = act(obs_sparse . W^T + b) | act(obs_dense . W^T + b) per network; the rest of the network (42 % of
-// the multiply-adds) runs in policy_forward_kernel from there.
+// the multiply-adds) runs in policy_tail_tc_kernel from there.
 // ------------------------------------------------------------------------------------------------------------
 #define TC_M 128
 #define TC_KC 32
@@ -606,7 +584,7 @@ __global__ void pl_tail_image_kernel(const float* __restrict__ w, int in, int ou
 
 __global__ void __launch_bounds__(TT_THREADS, 1)
 policy_tail_tc_kernel(const PolicyDev* __restrict__ p0, const PolicyDev* __restrict__ p1, const float* __restrict__ obs, int64_t obs_ld,
-                      int64_t N, const float* __restrict__ h1, int h1_nets, float* __restrict__ out0, int64_t out0_ld,
+                      int64_t N, const float* h1, int h1_nets, float* __restrict__ out0, int64_t out0_ld,
                       float* __restrict__ out1, int64_t out1_ld) {
     const PolicyDev& P = *(blockIdx.y ? p1 : p0);
     float* __restrict__ out = blockIdx.y ? out1 : out0;
@@ -717,7 +695,9 @@ policy_tail_tc_kernel(const PolicyDev* __restrict__ p0, const PolicyDev* __restr
             const float4* src = reinterpret_cast<const float4*>(hrow + enc * PL_E1 * h1_nets);
 #pragma unroll 5
             for (int g = half; g < PL_E1 / 4; g += 2) {
-                const float4 x = live ? __ldg(src + g) : make_float4(0.f, 0.f, 0.f, 0.f);
+                // a plain (coherent) load, and h1 is not __restrict__: under programmatic dependent launch the producer grid was
+                // still writing h1 while this one was resident, so the non-coherent read-only path is not allowed here
+                const float4 x = live ? src[g] : make_float4(0.f, 0.f, 0.f, 0.f);
                 store4(4 * g, x.x, x.y, x.z, x.w);
             }
             for (int f = PL_E1 + 4 * half; f < 96; f += 8) store4(f, 0.f, 0.f, 0.f, 0.f);
@@ -947,7 +927,7 @@ extern "C" int64_t rvb_policy_bytes(const rvb_policy* P) { return P ? P->storage
 // 2 (default) = the whole network on tcgen05 (policy_l1_tc_kernel + policy_tail_tc_kernel: faster than the FFMA path from a single
 // 128-env tile upwards); 3 = the same (kept for the tests that force the path); 1 = packed FFMA2 throughout (round 1's kernel);
 // 0 = scalar FFMA throughout.  1 and 0 are bit-identical; 2 / 3 differ from them in the summation order (all within 2e-5 of the
-// fp64 oracle, the gate of the tests).  RVB_TC_TAIL=0 keeps the FFMA kernel for the layers after the first (A/B switch).
+// fp64 oracle, the gate of the tests).
 static int g_policy_variant = 2;
 extern "C" int rvb_policy_variant(int v) {
     const int prev = g_policy_variant;
@@ -970,10 +950,9 @@ static int check_forward(const rvb_policy* P, const float* obs, int64_t obs_ld, 
     return RVB_OK;
 }
 
-// The tail kernel as a programmatic dependent of the first-layer kernel in front of it on `st` (RVB_POLICY_PDL=0: plain launch).
+// The tail kernel as a programmatic dependent of the first-layer kernel in front of it on `st`.
 static cudaError_t launch_tail_tc(dim3 grid, cudaStream_t st, const PolicyDev* a, const PolicyDev* b, const float* obs, int64_t obs_ld,
                                   int64_t N, const float* h1, int nets, float* out0, int64_t out0_ld, float* out1, int64_t out1_ld) {
-    static const bool pdl = !(getenv("RVB_POLICY_PDL") && atoi(getenv("RVB_POLICY_PDL")) == 0);
     cudaLaunchConfig_t cfg = {};
     cfg.gridDim = grid;
     cfg.blockDim = dim3(TT_THREADS);
@@ -983,7 +962,7 @@ static cudaError_t launch_tail_tc(dim3 grid, cudaStream_t st, const PolicyDev* a
     at[0].id = cudaLaunchAttributeProgrammaticStreamSerialization;
     at[0].val.programmaticStreamSerializationAllowed = 1;
     cfg.attrs = at;
-    cfg.numAttrs = pdl ? 1 : 0;
+    cfg.numAttrs = 1;
     return cudaLaunchKernelEx(&cfg, policy_tail_tc_kernel, a, b, obs, obs_ld, N, h1, nets, out0, out0_ld, out1, out1_ld);
 }
 
@@ -997,16 +976,16 @@ extern "C" int rvb_policy_forward(const rvb_policy* P, const float* obs, int64_t
     auto kern = g_policy_variant ? policy_forward_kernel<true> : policy_forward_kernel<false>;
     cudaStream_t st = as_stream(stream);
     float* h1 = nullptr;
+    cudaError_t le = cudaSuccess;
     if (tc_usable(P, obs, obs_ld, N)) {
         RVB_CUDA(rvb_scratch_alloc((void**)&h1, sizeof(float) * (size_t)N * 2 * PL_E1, st));
         policy_l1_tc_kernel<1><<<dim3((unsigned)ceil_div(N, TC_M), 2), TC_THREADS, tc_smem_bytes(1), st>>>(P->dev, nullptr, obs, obs_ld, N, h1);
+        le = launch_tail_tc(dim3((unsigned)ceil_div(N, TC_M), 1), st, P->dev, nullptr, obs, obs_ld, N, h1, 1, out, out_ld, nullptr, 0);
+    } else {
+        kern<<<dim3((unsigned)ceil_div(N, PL_TM), 1), PL_THREADS, PL_SMEM_BYTES, st>>>(P->dev, nullptr, obs, obs_ld, N, out, out_ld, nullptr, 0);
     }
-    const bool tc_tail = h1 && !(getenv("RVB_TC_TAIL") && atoi(getenv("RVB_TC_TAIL")) == 0);      // A/B switch: FFMA tail after the TC first layers
-    if (tc_tail)
-        launch_tail_tc(dim3((unsigned)ceil_div(N, TC_M), 1), st, P->dev, nullptr, obs, obs_ld, N, h1, 1, out, out_ld, nullptr, 0);
-    else
-        kern<<<dim3((unsigned)ceil_div(N, PL_TM), 1), PL_THREADS, PL_SMEM_BYTES, st>>>(P->dev, nullptr, obs, obs_ld, N, out, out_ld, nullptr, 0, h1, 1);
-    const cudaError_t le = cudaGetLastError();
+    const cudaError_t last = cudaGetLastError();          // also clears the error state of a failed launch
+    if (le == cudaSuccess) le = last;
     if (h1) cudaFreeAsync(h1, st);
     if (le != cudaSuccess) return rvb_set_error(RVB_ERR_CUDA, "rvb_policy_forward", cudaGetErrorString(le));
     return RVB_OK;
@@ -1027,17 +1006,16 @@ extern "C" int rvb_policy_forward_pair(const rvb_policy* A, const rvb_policy* B,
     auto kern = g_policy_variant ? policy_forward_kernel<true> : policy_forward_kernel<false>;
     cudaStream_t st = as_stream(stream);
     float* h1 = nullptr;
+    cudaError_t le = cudaSuccess;
     if (tc_usable(A, obs, obs_ld, N)) {          // both networks' first layers in one launch: they share the observation tiles
         RVB_CUDA(rvb_scratch_alloc((void**)&h1, sizeof(float) * (size_t)N * 4 * PL_E1, st));
         policy_l1_tc_kernel<2><<<dim3((unsigned)ceil_div(N, TC_M), 2), TC_THREADS, tc_smem_bytes(2), st>>>(A->dev, B->dev, obs, obs_ld, N, h1);
+        le = launch_tail_tc(dim3((unsigned)ceil_div(N, TC_M), 2), st, A->dev, B->dev, obs, obs_ld, N, h1, 2, out_a, out_a_ld, out_b, out_b_ld);
+    } else {
+        kern<<<dim3((unsigned)ceil_div(N, PL_TM), 2), PL_THREADS, PL_SMEM_BYTES, st>>>(A->dev, B->dev, obs, obs_ld, N, out_a, out_a_ld, out_b, out_b_ld);
     }
-    const bool tc_tail = h1 && !(getenv("RVB_TC_TAIL") && atoi(getenv("RVB_TC_TAIL")) == 0);
-    if (tc_tail)
-        launch_tail_tc(dim3((unsigned)ceil_div(N, TC_M), 2), st, A->dev, B->dev, obs, obs_ld, N, h1, 2, out_a, out_a_ld, out_b, out_b_ld);
-    else
-        kern<<<dim3((unsigned)ceil_div(N, PL_TM), 2), PL_THREADS, PL_SMEM_BYTES, st>>>(A->dev, B->dev, obs, obs_ld, N, out_a, out_a_ld, out_b, out_b_ld,
-                                                                                       h1, 2);
-    const cudaError_t le = cudaGetLastError();
+    const cudaError_t last = cudaGetLastError();          // also clears the error state of a failed launch
+    if (le == cudaSuccess) le = last;
     if (h1) cudaFreeAsync(h1, st);
     if (le != cudaSuccess) return rvb_set_error(RVB_ERR_CUDA, "rvb_policy_forward_pair", cudaGetErrorString(le));
     return RVB_OK;

@@ -4,9 +4,7 @@
 // variant 1 ("simple"): one warp per ray, lanes stride over the K candidates of the ray's cell, every
 // (ray, candidate) pair evaluated with the literal op sequence of ray_casting.py.  Kept as the on-device
 // cross-check for the production kernel (raycast_tiled.cu).
-#include <stdlib.h>
-
-#include "common.cuh"
+#include "raycast_common.cuh"
 
 int launch_heightmap_tiled(const rvb_terrain* t, const float* pos, const float* euler, const float* trig,
                            const double* pattern, int64_t P, int64_t N, uint16_t* dist, int32_t* hit_slot,
@@ -15,10 +13,8 @@ int launch_heightmap_tiled(const rvb_terrain* t, const float* pos, const float* 
 int launch_heightmap_shadow(const rvb_terrain* t, const float* pos, const float* euler, const float* trig,
                            const double* pattern, int64_t P, int64_t N, uint16_t* dist, int32_t* hit_slot,
                            int32_t* hit_tri, uint16_t* pt, uint16_t* sources, float* obs, int64_t obs_ld,
-                           const int32_t* col_a, const int32_t* col_b, float cos_steep, const RvbObs16* o16, cudaStream_t st);
-// envs whose ray direction has |d_z| below this are ray-cast by the tiled kernel (their prisms are long slivers)
-#define RVB_COS_STEEP 0.7f
-
+                           const int32_t* col_a, const int32_t* col_b, const RaycastKnobs& knobs, const RvbObs16* o16,
+                           cudaStream_t st);
 
 // ------------------------------------------------------------------------------------------------
 // setup: sources (fp64 transform -> fp16), per-env direction, per-ray cell
@@ -165,16 +161,15 @@ extern "C" int rvb_heightmap_raycast2(const rvb_terrain* t, const float* pos, co
     RVB_REQUIRE(variant != 2 || t->index != nullptr, "rvb_heightmap_raycast: variant 2 reads the index the layer released (rvb_terrain_release_index)");
     const RvbObs16 o16v = {obs_h16, obs_h16_ld, obs_h16_col0};
     const RvbObs16* o16 = obs_h16 ? &o16v : nullptr;
+    RaycastKnobs knobs;
+    const int krc = read_raycast_knobs(knobs);
+    if (krc != RVB_OK) return krc;
     cudaStream_t st = as_stream(stream);
     // a layer with more than 2 % of triangles the shadow kernel has no bound for (terrain.cu: n_ill): the tiled kernel is the faster one
-    bool shadow_ok = t->n_ill * 50 <= t->T;
-    if (const char* ev = getenv("RVB_SHADOW_FORCE")) shadow_ok = atoi(ev) != 0;      // tuning hook
-    if (variant == 0 && t->sb_ids != nullptr && shadow_ok) {
-        float cos_steep = RVB_COS_STEEP;
-        if (const char* ev = getenv("RVB_COS_STEEP")) cos_steep = (float)atof(ev);      // tuning hook; results do not depend on it
+    const bool shadow_ok = knobs.force >= 0 ? knobs.force == 1 : t->n_ill * 50 <= t->T;
+    if (variant == 0 && t->sb_ids != nullptr && shadow_ok)
         return launch_heightmap_shadow(t, pos, euler, trig, pattern, P, N, dist, hit_slot, hit_tri, pt, sources, obs,
-                                       obs_ld, col_a, col_b, cos_steep, o16, st);
-    }
+                                       obs_ld, col_a, col_b, knobs, o16, st);
     if (variant != 1)
         return launch_heightmap_tiled(t, pos, euler, trig, pattern, P, N, dist, hit_slot, hit_tri, pt, sources, obs,
                                       obs_ld, col_a, col_b, variant == 2, o16, st);
@@ -204,7 +199,6 @@ extern "C" int rvb_cast_rays(const rvb_terrain* t, const uint16_t* sources, cons
     RVB_REQUIRE(t && sources && directions && dist, "rvb_cast_rays: null pointer");
     RVB_REQUIRE(t->index != nullptr, "rvb_cast_rays: the layer released its index (rvb_terrain_release_index)");
     (void)variant;
-    if (R == 0) return RVB_OK;
     cudaStream_t st = as_stream(stream);
     __half* dneg = nullptr;
     RVB_CUDA(rvb_scratch_alloc((void**)&dneg, sizeof(__half) * 3 * (size_t)R, st));
@@ -243,7 +237,6 @@ extern "C" int rvb_ray_distance(const uint16_t* sources, const uint16_t* directi
     RVB_REQUIRE(n >= 0, "rvb_ray_distance: n < 0");
     if (n == 0) return RVB_OK;
     RVB_REQUIRE(sources && directions && triangles && k, "rvb_ray_distance: null pointer");
-    if (n == 0) return RVB_OK;
     ray_distance_kernel<<<(unsigned)ceil_div(n, 256), 256, 0, as_stream(stream)>>>(
         (const __half*)sources, (const __half*)directions, (const __half*)triangles, n, (__half*)k, (__half*)pt);
     RVB_LAUNCH_CHECK();

@@ -2,6 +2,19 @@
 #pragma once
 #include "common.cuh"
 
+// Tuning knobs of the heightmap ray-cast: parameters of the shipped design that tools/ sweep (DESIGN.md 6, "Tuning knobs").
+// read_raycast_knobs (raycast_shadow.cu) takes them from the environment on every call, so a process can change them between
+// calls; an unset variable means the shipped default, a value that does not parse or lies outside its range is RVB_ERR_INVALID.
+struct RaycastKnobs {
+    int force;            // RVB_SHADOW_FORCE: -1 = unset (the layer's count of triangles without a bound decides), 0 / 1 = off / on
+    float cos_steep;      // RVB_COS_STEEP: envs whose ray direction has |d_z| below it are cast by the tiled kernel
+    int min_sh;           // RVB_SHADOW_SH: finest bins of the shadow kernel, 2^sh x 2^sh cells
+    int task_rays;        // RVB_SHADOW_TASK_RAYS: rays per stage-3L task
+    int64_t split;        // RVB_SHADOW_SPLIT: envs cast by two half-ray CTAs at the end of the launch; -1 = unset (depends on N)
+    bool dbg;             // RVB_SHADOW_DBG: per-stage counters of each launch on stderr
+};
+int read_raycast_knobs(RaycastKnobs& k);
+
 namespace rc {
 
 constexpr uint32_t KEY_INIT = 0xC9800000u;     // (11.0, slot 0): the result when every candidate misses
@@ -39,7 +52,7 @@ struct TiledParams {
     const uint32_t* sb_off;
     const int32_t* sb_ids;
     const unsigned char* sb_slot9;
-    const ChunkRec* sb_chunk;   // bounds per window of 32 list entries (chunk culling); NULL = none
+    const ChunkRec* sb_chunk;   // bounds per window of 32 list entries (window cull)
     int nSBy;
     float cos_steep;          // envs whose ray direction is flatter than this go to the fall-back list
     int* fb_count;            // [1]
@@ -52,11 +65,8 @@ struct TiledParams {
     // pre-sorted steep envs (cast by the tiled kernel on a second stream, concurrently); both written by hm_classify_kernel
     const int32_t* order;     // [N] or NULL
     int presorted;            // steep envs are already on a work list: the shadow kernel just skips them
-    int min_sh;               // bins are 2^sh x 2^sh cells, sh >= min_sh (0 = one cell; tuning hook)
-    int spec_slot;            // stage 3b fetches the slot byte before the literal test (tuning hook)
-    int task_rays;            // shadow kernel: rays per task of stage 3L (<= 16; tuning hook)
-    int bulk_obs;             // shadow kernel: observation row leaves through one bulk asynchronous copy (A/B switch)
-    int n_obs_cols;           // number of heightmap observation columns (sparse + dense) when obs is requested
+    int min_sh;               // bins are 2^sh x 2^sh cells, sh >= min_sh (0 = one cell; tuning knob)
+    int task_rays;            // shadow kernel: rays per task of stage 3L (1..32: one mask bit each; tuning knob)
     int64_t split_from;       // shadow kernel: order positions >= split_from are cast by two CTAs (half the rays each); -1 = none
     int split_at;             // first ray of the second half
     unsigned long long* dbg;  // optional [24] work counters / cycle counts of the shadow kernel (RVB_SHADOW_DBG=1)
@@ -201,20 +211,11 @@ static __device__ __noinline__ int32_t tri_of_slot_blk(const int32_t* ids, const
 // Epilogue in ray order: coalesced stores of dist / hit slot / hit triangle / pt / sources and the fused sparse+dense
 // observation columns (heightmap_distribution.py:126-133, rover.py:324-325).  res[p] = best key of local ray p; a set bit
 // in far[] marks a ray that saw a hit beyond the 11.0 miss sentinel (resolved literally here).
-// `stage` (optional, shared memory, 16-byte aligned, >= (ncols + 8) floats): the observation row is assembled there and leaves
-// the SM as ONE bulk asynchronous copy (cp.async.bulk shared -> global, the TMA unit's non-tensor mode) instead of one 4-byte
-// store per column; only when the tile is the whole pattern.  ncols = number of heightmap observation columns.
 __device__ __forceinline__ void epilogue(const TiledParams& q, int64_t n, int p0, int np, const Trig& tr, double tx, double ty,
                                          double tz, __half2 dx2, __half2 dy2, __half2 dz2, const uint32_t* res,
-                                         const uint32_t* far, int tid, int nthreads, float* stage = nullptr, int ncols = 0) {
+                                         const uint32_t* far, int tid, int nthreads) {
     const H3 dlit = {__low2half(dx2), __low2half(dy2), __low2half(dz2)};
     const bool want_geo = q.hit_tri || q.pt || q.sources;
-    // destination of column 4 (the first heightmap column) and how the row splits into an unaligned head, a 16-byte aligned body
-    // (the bulk copy) and a tail
-    const bool bulk = stage != nullptr && q.obs != nullptr && np == q.P && ncols > 8;
-    float* const grow = q.obs ? q.obs + n * q.obs_ld + 4 : nullptr;
-    const int head = bulk ? (int)(((16u - (uint32_t)((uintptr_t)grow & 15u)) & 15u) >> 2) : 0;      // floats before the body
-    float* const srow = bulk ? stage + ((4 - head) & 3) : nullptr;                                    // srow + head is 16-byte aligned
     // Fast path (the production call: distances + observation columns only, no ray of the tile saw a hit beyond the miss sentinel):
     // every load of the thread's <= 8 rays is issued before the first store -- in the general loop below a ray's column indices,
     // its stores and the next ray's loads form one dependent chain, and the CTA sits in this tail at memory latency (the obs
@@ -223,7 +224,7 @@ __device__ __forceinline__ void epilogue(const TiledParams& q, int64_t n, int p0
         bool any_far = false;
         for (int i = tid; i < (np + 31) / 32; i += nthreads) any_far |= far[i] != 0u;
         any_far = __syncthreads_or(any_far ? 1 : 0) != 0;
-        if (!any_far && !want_geo && !q.hit_slot && np <= 8 * nthreads && !bulk && (q.spec_slot & 16)) {
+        if (!any_far && !want_geo && !q.hit_slot && np <= 8 * nthreads) {
             uint32_t key[8];
             int ca[8], cb[8];
             const bool want_cols = q.obs != nullptr || q.obs16 != nullptr;
@@ -305,13 +306,8 @@ __device__ __forceinline__ void epilogue(const TiledParams& q, int64_t n, int p0
         if (q.obs) {
             const float v = __half2float(h_mul(h_from_bits(kb), __float2half_rn(0.5f)));     // fp16(dist / 2) -> f32
             const int ca = q.col_a[p0 + p], cb = q.col_b[p0 + p];
-            if (bulk) {
-                if (ca >= 4) srow[ca - 4] = v;
-                if (cb >= 4) srow[cb - 4] = v;
-            } else {
-                if (ca >= 0) q.obs[n * q.obs_ld + ca] = v;
-                if (cb >= 0) q.obs[n * q.obs_ld + cb] = v;
-            }
+            if (ca >= 0) q.obs[n * q.obs_ld + ca] = v;
+            if (cb >= 0) q.obs[n * q.obs_ld + cb] = v;
         }
         if (q.obs16) {                                                                        // the same value, kept in fp16
             const __half v = h_mul(h_from_bits(kb), __float2half_rn(0.5f));
@@ -319,19 +315,6 @@ __device__ __forceinline__ void epilogue(const TiledParams& q, int64_t n, int p0
             if (ca >= 0) q.obs16[n * q.obs16_ld + (ca - q.obs16_col0)] = v;
             if (cb >= 0) q.obs16[n * q.obs16_ld + (cb - q.obs16_col0)] = v;
         }
-    }
-    if (bulk) {
-        __syncthreads();
-        const int body = ((ncols - head) >> 2) << 2;                  // floats in the 16-byte aligned middle part
-        if (tid == 0) {
-            asm volatile("fence.proxy.async.shared::cta;" ::: "memory");
-            const uint32_t saddr = (uint32_t)__cvta_generic_to_shared(srow + head);
-            asm volatile("cp.async.bulk.global.shared::cta.bulk_group [%0], [%1], %2;" ::"l"(grow + head), "r"(saddr), "r"(body * 4) : "memory");
-            asm volatile("cp.async.bulk.commit_group;" ::: "memory");
-        }
-        if (tid < head) grow[tid] = srow[tid];
-        if (tid >= 32 && tid - 32 < ncols - head - body) grow[head + body + tid - 32] = srow[head + body + tid - 32];
-        if (tid == 0) asm volatile("cp.async.bulk.wait_group.read 0;" ::: "memory");      // the source must outlive the copy
     }
 }
 

@@ -34,6 +34,8 @@
 // tests/test_shadow_bound_cpu.py runs it.  Tiles this kernel cannot group (rays spread over more than 6144 bins or
 // 64 superblocks, a list longer than the queue encoding, fp16 overflow) are handed to the tiled kernel through a second
 // work list.
+#include <ctype.h>
+#include <errno.h>
 #include <stdlib.h>
 #include <string.h>
 
@@ -62,6 +64,9 @@ constexpr int CHUNK_CAP = 1024;    // chunks per tile (u8 chunk -> item table)
 constexpr int QCAP = 64;           // per-warp queues q1, q2 (each drained below 32 after every push of <= 32)
 constexpr int QCAP3 = 128;         // q4 (stage 3L pushes while it holds < 32 entries, stage 3b drains in batches of 32)
 constexpr int TASK_RAYS = 20;      // rays per task (<= 32: one mask bit each); sweep with the shipped kernel: 8 +5 %, 12 +1 %, 16 +0.45 %, 20 best, 24 +0.2 %, 32 +1 %
+constexpr int MIN_SH = 1;          // finest bins: 2x2 cells, 2 % faster than single cells (fewer tasks)
+constexpr float COS_STEEP = 0.7f;  // envs whose ray direction has |d_z| below this go to the tiled kernel (their prisms are long
+                                   // slivers); 0.8 until a sweep: -0.6 % at 0.7.  Results do not depend on it
 constexpr int REL_BITS = 15;        // queue entries name a triangle as item << 15 | position in the item's list
 constexpr int ILL_CAP = 128;        // triangles without a bound ("ill": fp16 determinant within rounding of zero) a tile may meet before it
                                    // is handed to the tiled kernel, whose cost does not depend on them (a 1M-triangle heightfield has ~1
@@ -118,14 +123,6 @@ __device__ __forceinline__ TriF tri_f(const uint4& q0, const uint2& q1) {
     t.bx = hf(q0.y >> 16); t.by = hf(q0.z & 0xffff); t.bz = hf(q0.z >> 16);
     t.cx = hf(q0.w & 0xffff); t.cy = hf(q0.w >> 16); t.cz = hf(q1.x & 0xffff);
     return t;
-}
-
-// Two fp32 FMAs in one issue slot (sm_100 FFMA2): d.xy = a.xy * b + d.xy, b broadcast.
-__device__ __forceinline__ void ffma2(float& d0, float& d1, float a0, float a1, float b) {
-    asm("{\n\t.reg .b64 ra, rb, rc;\n\tmov.b64 ra, {%2, %3};\n\tmov.b64 rb, {%4, %4};\n\tmov.b64 rc, {%0, %1};\n\t"
-        "fma.rn.f32x2 rc, ra, rb, rc;\n\tmov.b64 {%0, %1}, rc;\n\t}"
-        : "+f"(d0), "+f"(d1)
-        : "f"(a0), "f"(a1), "f"(b));
 }
 
 // positive fp32 (or +inf) -> its upper 16 bits, rounded up
@@ -545,22 +542,19 @@ __global__ void __launch_bounds__(TT, RTC <= RT_SMALL ? 4 : 3) hm_shadow_kernel(
         // entries at a time (one thread per window).  The survivors go into the chunk table the warps pull from, the expensive ones
         // (many rays of the item under the window) first: the warps' last chunks are then cheap and they finish together
         const int total = s_nchunks;
-        const bool cull_on = q.sb_chunk != nullptr && (q.spec_slot & 4);
         for (int g = tid; g < total; g += TT) {
             const int item = all_item[g];
             const Item& it = sm.items[item];
-            int key = 0;
-            if (cull_on) {
-                const uint4* rp = reinterpret_cast<const uint4*>(q.sb_chunk + (it.list_off >> 5) + (g - (int)sm.cum[item]));
-                union { uint4 u[4]; ChunkRec c; } rec;
-                uint4 c0, c1, c2, c3;
-                ldg_rec32(rp, c0, c1);
-                ldg_rec32(rp + 2, c2, c3);
-                rec.u[0] = c0; rec.u[1] = c1; rec.u[2] = c2; rec.u[3] = c3;
-                float ov;
-                if (chunk_cull(rec.c, s_env, it.rlox, it.rhix, it.rloy, it.rhiy, ov)) key = 0xFF;
-                else key = 7 - min(7, (int)(sqrtf((float)s_item_rays[item] * ov) * 0.25f));      // bucket 0: >= 784 rays under the window
-            }
+            const uint4* rp = reinterpret_cast<const uint4*>(q.sb_chunk + (it.list_off >> 5) + (g - (int)sm.cum[item]));
+            union { uint4 u[4]; ChunkRec c; } rec;
+            uint4 c0, c1, c2, c3;
+            ldg_rec32(rp, c0, c1);
+            ldg_rec32(rp + 2, c2, c3);
+            rec.u[0] = c0; rec.u[1] = c1; rec.u[2] = c2; rec.u[3] = c3;
+            float ov;
+            int key;
+            if (chunk_cull(rec.c, s_env, it.rlox, it.rhix, it.rloy, it.rhiy, ov)) key = 0xFF;
+            else key = 7 - min(7, (int)(sqrtf((float)s_item_rays[item] * ov) * 0.25f));      // bucket 0: >= 784 rays under the window
             all_key[g] = (unsigned char)key;
             if (key != 0xFF) atomicAdd(&s_bkt[0][key], 1);
         }
@@ -681,7 +675,7 @@ __global__ void __launch_bounds__(TT, RTC <= RT_SMALL ? 4 : 3) hm_shadow_kernel(
                     q1[at] = make_uint2(ent, ((__float_as_uint(gball) + 0x7fu) & ~0x7fu) | (uint32_t)item);
                     q1t[at] = id;
                     // stage 2 will want the triangle's record: start bringing it into L2 now
-                    if (q.spec_slot & 2) asm volatile("prefetch.global.L2 [%0];" ::"l"(q.recs + id));
+                    asm volatile("prefetch.global.L2 [%0];" ::"l"(q.recs + id));
                 }
                 t1 += __popc(m);
                 DBG(0, 1); DBG(1, __popc(m));
@@ -704,7 +698,7 @@ __global__ void __launch_bounds__(TT, RTC <= RT_SMALL ? 4 : 3) hm_shadow_kernel(
             if ((uint32_t)lane < cnt) {
                 const uint2 en = q1[(h1 + lane) & (QCAP - 1)];
                 e_ent = en.x;
-                const int32_t tri = (q.spec_slot & 8) ? q1t[(h1 + lane) & (QCAP - 1)] : __ldg(q.sb_ids + e_ent);
+                const int32_t tri = q1t[(h1 + lane) & (QCAP - 1)];
                 e_tri = tri;
                 const float gball = __uint_as_float(en.y & ~0x7fu);
                 const Item& it = sm.items[en.y & 0x7fu];
@@ -769,8 +763,7 @@ __global__ void __launch_bounds__(TT, RTC <= RT_SMALL ? 4 : 3) hm_shadow_kernel(
                 a_ent = tk.x;
                 a_start = tk.y & 0xffffu;
                 const int c = (int)(tk.y >> 16);
-                const int32_t tri = (q.spec_slot & 8) ? q2t[(h2 + lane) & (QCAP - 1)]
-                                                      : __ldg(q.sb_ids + sm.items[a_ent >> REL_BITS].list_off + (a_ent & ((1u << REL_BITS) - 1u)));
+                const int32_t tri = q2t[(h2 + lane) & (QCAP - 1)];
                 a_tri = tri;
                 const uint4 r0 = __ldg(reinterpret_cast<const uint4*>(q.recs + tri));
                 const uint32_t r1 = __ldg(reinterpret_cast<const uint32_t*>(q.recs + tri) + 4);
@@ -847,7 +840,7 @@ __global__ void __launch_bounds__(TT, RTC <= RT_SMALL ? 4 : 3) hm_shadow_kernel(
                     const uint32_t pc = q4[(h4 + lane) & (QCAP3 - 1)];
                     const uint2 ray = sm.rays[pc & 0x7ffu];
                     const uint32_t ent = sm.items[pc >> (11 + REL_BITS)].list_off + ((pc >> 11) & ((1u << REL_BITS) - 1u));
-                    const int32_t tri = (q.spec_slot & 8) ? q4t[(h4 + lane) & (QCAP3 - 1)] : __ldg(q.sb_ids + ent);
+                    const int32_t tri = q4t[(h4 + lane) & (QCAP3 - 1)];
                     const H3 s = {h_from_bits(ray.x & 0xffff), h_from_bits(ray.x >> 16), h_from_bits(ray.y & 0xffff)};
                     const uint32_t meta = ray.y >> 16, p = meta & 0x7ffu, cym = meta >> 11;
                     // slot of the triangle in the K-list of the ray's own cell (0xFF: not in it): ONE look-up in the superblock entry's
@@ -907,30 +900,66 @@ __global__ void __launch_bounds__(TT, RTC <= RT_SMALL ? 4 : 3) hm_shadow_kernel(
             const float r_ = -ve[0], p_ = -ve[1], y_ = -ve[2];
             tr2 = {sinf(r_), cosf(r_), sinf(p_), cosf(p_), sinf(y_), cosf(y_)};
         }
-        // the sorted rays are dead: their shared memory stages the observation row of the bulk-copy epilogue
-        epilogue(q, n, p0, np, tr2, ex_, ey_, ez_, dx2, dy2, dz2, sm.res, sm.far, tid, TT,
-                 q.bulk_obs ? reinterpret_cast<float*>(sm.rays) : nullptr, q.n_obs_cols);
+        epilogue(q, n, p0, np, tr2, ex_, ey_, ez_, dx2, dy2, dz2, sm.res, sm.far, tid, TT);
     }
 }
 
 }  // namespace
 
+// The whole of `name`'s value as a number in [lo, hi] (an integer if `integer`) into v; unset leaves v alone.  `range` states
+// the accepted values in the error message.
+static int read_knob(const char* name, double lo, double hi, bool integer, const char* range, double& v) {
+    const char* s = getenv(name);
+    if (!s) return RVB_OK;
+    char* end = nullptr;
+    errno = 0;
+    const double x = integer ? (double)strtoll(s, &end, 10) : strtod(s, &end);
+    if (*s == '\0' || isspace((unsigned char)*s) || *end != '\0' || errno != 0 || !(x >= lo && x <= hi)) {
+        char detail[128];
+        snprintf(detail, sizeof(detail), "'%.32s' is not %s", s, range);
+        return rvb_set_error(RVB_ERR_INVALID, name, detail);
+    }
+    v = x;
+    return RVB_OK;
+}
+
+int read_raycast_knobs(RaycastKnobs& k) {
+    double force = -1, cos_steep = COS_STEEP, min_sh = MIN_SH, task_rays = TASK_RAYS, split = -1, dbg = 0;
+    int rc_;
+    if ((rc_ = read_knob("RVB_SHADOW_FORCE", 0, 1, true, "0 or 1", force))) return rc_;
+    if ((rc_ = read_knob("RVB_COS_STEEP", 0, 1, false, "a number in [0, 1]", cos_steep))) return rc_;
+    // 2^3 cells, the coarsest bins phase 1 goes up to; bins must divide the superblock side (24 cells)
+    if ((rc_ = read_knob("RVB_SHADOW_SH", 0, 3, true, "an integer in 0..3", min_sh))) return rc_;
+    if ((rc_ = read_knob("RVB_SHADOW_TASK_RAYS", 1, 32, true, "an integer in 1..32", task_rays))) return rc_;
+    if ((rc_ = read_knob("RVB_SHADOW_SPLIT", 0, 9e18, true, "an integer >= 0", split))) return rc_;
+    if ((rc_ = read_knob("RVB_SHADOW_DBG", 0, 1, true, "0 or 1", dbg))) return rc_;
+    k.force = (int)force;
+    k.cos_steep = (float)cos_steep;
+    k.min_sh = (int)min_sh;
+    k.task_rays = (int)task_rays;
+    k.split = (int64_t)split;
+    k.dbg = dbg != 0;
+    return RVB_OK;
+}
+
 int launch_heightmap_shadow(const rvb_terrain* t, const float* pos, const float* euler, const float* trig,
                             const double* pattern, int64_t P, int64_t N, uint16_t* dist, int32_t* hit_slot,
                             int32_t* hit_tri, uint16_t* pt, uint16_t* sources, float* obs, int64_t obs_ld,
-                            const int32_t* col_a, const int32_t* col_b, float cos_steep, const RvbObs16* o16, cudaStream_t st) {
-    RVB_REQUIRE(t->sb_ids != nullptr && t->sb_slot9 != nullptr && t->blk_ids != nullptr && t->s1recs != nullptr, "heightmap ray-cast (shadow): layer has no block lists");
+                            const int32_t* col_a, const int32_t* col_b, const RaycastKnobs& knobs, const RvbObs16* o16,
+                            cudaStream_t st) {
+    RVB_REQUIRE(t->sb_ids != nullptr && t->sb_slot9 != nullptr && t->sb_chunk != nullptr && t->blk_ids != nullptr && t->s1recs != nullptr,
+                "heightmap ray-cast (shadow): layer has no block lists");
     rc::TiledParams q;
     int rc_ = fill_tiled_params(t, pos, euler, trig, pattern, P, N, dist, hit_slot, hit_tri, pt, sources, obs, obs_ld, col_a,
                                 col_b, o16, q);
     if (rc_ != RVB_OK) return rc_;
     RVB_REQUIRE(q.tile_size <= 2048, "heightmap ray-cast (shadow): tile larger than 2048 rays");
     int64_t nblocks = N * q.tiles;
-    // RVB_SHADOW_SPLIT = number of envs (at the end of the order) cast by two CTAs of half the rays each; default below
+    // the last nsplit envs of the order are cast by two CTAs of half the rays each
     q.split_from = -1;
     {
         int64_t nsplit = N >= 8 * 148 ? 3 * 148 : 0;            // measured at 4096 envs: -2 % (444), -1.2 % (592), -1 % (296)
-        if (const char* ev = getenv("RVB_SHADOW_SPLIT")) nsplit = atoll(ev);
+        if (knobs.split >= 0) nsplit = knobs.split;
         if (q.tiles == 1 && q.P >= 64 && nsplit > 0) {
             if (nsplit > N) nsplit = N;
             q.split_from = N - nsplit;
@@ -949,23 +978,11 @@ int launch_heightmap_shadow(const rvb_terrain* t, const float* pos, const float*
     q.fb_count = scratch + 3;
     q.fb_list = scratch + 4 + nblocks;
     int32_t* order = scratch + 4 + 2 * nblocks;
-    q.cos_steep = cos_steep;
+    q.cos_steep = knobs.cos_steep;
     q.order = order;
     q.presorted = 1;
-    q.min_sh = 1;                                                            // 2x2-cell bins: 2 % faster than single cells (fewer tasks)
-    if (const char* ms = getenv("RVB_SHADOW_SH")) q.min_sh = atoi(ms);      // tuning hook: finest bins to start from
-    q.spec_slot = 31;         // bit 0: (unused since the slot table) bit 1: L2 prefetch of the records, bit 2: window cull,
-                              // bit 3: triangle ids travel through the queues instead of being re-read from sb_ids, bit 4: the epilogue
-                              // issues all of a thread's loads before its first store (raycast_common.cuh)
-    // A/B switch (DESIGN.md 4.1): RVB_SHADOW_BULK = number of heightmap observation columns (1746 for the reference pattern; every
-    // one of them must be named by col_a / col_b) -> the row is staged in shared memory and stored by one cp.async.bulk
-    q.bulk_obs = 0;
-    q.n_obs_cols = 0;
-    if (const char* bo = getenv("RVB_SHADOW_BULK")) q.n_obs_cols = atoi(bo);
-    q.bulk_obs = q.n_obs_cols > 8 && (size_t)(q.n_obs_cols + 8) * 4 <= (size_t)q.tile_size * 8;
-    q.task_rays = TASK_RAYS;
-    if (const char* tr = getenv("RVB_SHADOW_TASK_RAYS")) q.task_rays = min(max(atoi(tr), 1), 32);   // tuning hook
-    if (const char* sp = getenv("RVB_SHADOW_SPEC")) q.spec_slot = atoi(sp); // tuning hook
+    q.min_sh = knobs.min_sh;
+    q.task_rays = knobs.task_rays;
     RvbSide* side_p = nullptr;
     RVB_CUDA(rvb_side_stream(1, &side_p));
     RvbSide& side = *side_p;
@@ -988,29 +1005,24 @@ int launch_heightmap_shadow(const rvb_terrain* t, const float* pos, const float*
         guard.join = side.join;
     }
     if (configured_device != dev) {
-        RVB_CUDA(cudaFuncSetAttribute(hm_shadow_kernel<false, RT_MAX>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)shadow_smem_bytes(RT_MAX) + 48 * 1024));
-        RVB_CUDA(cudaFuncSetAttribute(hm_shadow_kernel<true, RT_MAX>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)shadow_smem_bytes(RT_MAX) + 48 * 1024));
-        RVB_CUDA(cudaFuncSetAttribute(hm_shadow_kernel<false, RT_SMALL>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)shadow_smem_bytes(RT_SMALL) + 48 * 1024));
-        RVB_CUDA(cudaFuncSetAttribute(hm_shadow_kernel<true, RT_SMALL>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)shadow_smem_bytes(RT_SMALL) + 48 * 1024));
+        RVB_CUDA(cudaFuncSetAttribute(hm_shadow_kernel<false, RT_MAX>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)shadow_smem_bytes(RT_MAX)));
+        RVB_CUDA(cudaFuncSetAttribute(hm_shadow_kernel<true, RT_MAX>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)shadow_smem_bytes(RT_MAX)));
+        RVB_CUDA(cudaFuncSetAttribute(hm_shadow_kernel<false, RT_SMALL>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)shadow_smem_bytes(RT_SMALL)));
+        RVB_CUDA(cudaFuncSetAttribute(hm_shadow_kernel<true, RT_SMALL>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)shadow_smem_bytes(RT_SMALL)));
         configured_device = dev;
     }
-    const bool dbg = getenv("RVB_SHADOW_DBG") != nullptr;
+    const bool dbg = knobs.dbg;
     if (dbg) {
         cudaMalloc(&q.dbg, 24 * sizeof(unsigned long long));
         cudaMemset(q.dbg, 0, 24 * sizeof(unsigned long long));
     }
-    // RVB_SHADOW_PAD (bytes, <= 48 KB): extra dynamic shared memory, to measure the kernel at a lower occupancy (tuning hook);
-    // RVB_SHADOW_BIG: force the 2048-ray instantiation (3 CTAs per SM) where the 1664-ray one (4 CTAs per SM) would run
-    const char* pad_s = getenv("RVB_SHADOW_PAD");
-    const size_t pad = pad_s ? (size_t)min(max(atoi(pad_s), 0), 48 * 1024) : 0;
-    const bool small = q.tile_size <= RT_SMALL && getenv("RVB_SHADOW_BIG") == nullptr;
     const unsigned grid = (unsigned)nblocks;
-    if (small) {
-        if (dbg) hm_shadow_kernel<true, RT_SMALL><<<grid, TT, shadow_smem_bytes(RT_SMALL) + pad, st>>>(q);
-        else hm_shadow_kernel<false, RT_SMALL><<<grid, TT, shadow_smem_bytes(RT_SMALL) + pad, st>>>(q);
+    if (q.tile_size <= RT_SMALL) {
+        if (dbg) hm_shadow_kernel<true, RT_SMALL><<<grid, TT, shadow_smem_bytes(RT_SMALL), st>>>(q);
+        else hm_shadow_kernel<false, RT_SMALL><<<grid, TT, shadow_smem_bytes(RT_SMALL), st>>>(q);
     } else {
-        if (dbg) hm_shadow_kernel<true, RT_MAX><<<grid, TT, shadow_smem_bytes(RT_MAX) + pad, st>>>(q);
-        else hm_shadow_kernel<false, RT_MAX><<<grid, TT, shadow_smem_bytes(RT_MAX) + pad, st>>>(q);
+        if (dbg) hm_shadow_kernel<true, RT_MAX><<<grid, TT, shadow_smem_bytes(RT_MAX), st>>>(q);
+        else hm_shadow_kernel<false, RT_MAX><<<grid, TT, shadow_smem_bytes(RT_MAX), st>>>(q);
     }
     if (dbg) {
         unsigned long long h[24];

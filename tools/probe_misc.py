@@ -1,8 +1,6 @@
-"""GPU probes: (1) pinned D2H / H2D bandwidth, (2) shadow kernel time vs occupancy (RVB_SHADOW_PAD)."""
-import os, sys, time
+"""GPU probe: pinned D2H / H2D bandwidth and the host link topology."""
+import os
 import torch
-ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
-sys.path.insert(0, ROOT)
 for mb in (28.7, 256.0):
     n = int(mb * 1e6)
     d = torch.empty(n, dtype=torch.uint8, device="cuda")
@@ -18,21 +16,3 @@ for mb in (28.7, 256.0):
         e1.record(); torch.cuda.synchronize()
         print("%s %.1f MB pinned: %.1f GB/s" % (name, mb, n * 10 / (e0.elapsed_time(e1) * 1e-3) / 1e9))
 os.system("nvidia-smi topo -m 2>&1 | head -20")
-import isaac_rover_b200 as R
-w = R.synth.make_world(length=200.0, nv=708, K=200, n_stones=2000, seed=42, build_index=None)
-w.map_indices = R.build_knn_index(w.triangles, w.vertices, w.G, w.res, w.K, device="cuda:0")
-cam = R.Camera("cuda:0", torch.tensor([0, 0, 0.0]), assets=(w.map_indices, w.triangles, w.vertices))
-for N in (4096, 16384):
-    st = {k: v.cuda() for k, v in R.synth.make_env_state(w, N, seed=100).items()}
-    eul = R.tensor_quat_to_eul(st["quat"])
-    for pad in ("0", "20000", "40000"):
-        os.environ["RVB_SHADOW_PAD"] = pad
-        for _ in range(3):
-            cam.get_depths(st["pos"], eul, want_pt=False)
-        torch.cuda.synchronize()
-        e0, e1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
-        e0.record()
-        for _ in range(10):
-            cam.get_depths(st["pos"], eul, want_pt=False)
-        e1.record(); torch.cuda.synchronize()
-        print("N=%d pad %s: %.3f ms" % (N, pad, e0.elapsed_time(e1) / 10))

@@ -53,16 +53,10 @@ for v in (3, 0, 2):
     d, pt, s = cam.get_depths(st["pos"], eul, want_hits=True, want_pt=False)
     out[v] = (d.clone(), cam.last_hit_slot.clone(), cam.last_hit_tri.clone())
 import os as _os
-for big in ("1", None):
-    if big:
-        _os.environ["RVB_SHADOW_BIG"] = big
-    else:
-        _os.environ.pop("RVB_SHADOW_BIG", None)
-    cam.variant = 0
-    med, mn = timed(lambda: cam.get_depths(st["pos"], eul, want_pt=False))
-    d, _, _ = cam.get_depths(st["pos"], eul, want_pt=False)
-    print("shadow %s instantiation: median %.3f ms, min %.3f ms, equal to variant 3: %s" % ("2048-ray (3 CTAs/SM)" if big else "1664-ray (4 CTAs/SM)", med, mn,
-                                                                        bool(torch.equal(d.view(torch.int16), out[3][0].view(torch.int16)))))
+cam.variant = 0
+med, mn = timed(lambda: cam.get_depths(st["pos"], eul, want_pt=False))
+d, _, _ = cam.get_depths(st["pos"], eul, want_pt=False)
+print("shadow: median %.3f ms, min %.3f ms, equal to variant 3: %s" % (med, mn, bool(torch.equal(d.view(torch.int16), out[3][0].view(torch.int16)))))
 for ns in ("0", "444", "0", "444"):
     _os.environ["RVB_SHADOW_SPLIT"] = ns
     cam.variant = 0
@@ -70,13 +64,6 @@ for ns in ("0", "444", "0", "444"):
     d, _, _ = cam.get_depths(st["pos"], eul, want_pt=False)
     print("split envs %s: median %.3f ms, min %.3f, equal to variant 3: %s" % (ns, med, mn, bool(torch.equal(d.view(torch.int16), out[3][0].view(torch.int16)))))
 _os.environ.pop("RVB_SHADOW_SPLIT")
-for sp in ("3", "7", "3", "7"):
-    _os.environ["RVB_SHADOW_SPEC"] = sp
-    cam.variant = 0
-    med, mn = timed(lambda: cam.get_depths(st["pos"], eul, want_pt=False), reps=30)
-    d, _, _ = cam.get_depths(st["pos"], eul, want_pt=False)
-    print("spec bits (1 slot prefetch, 2 record prefetch, 4 window cull) %s: median %.3f ms, min %.3f, equal to variant 3: %s" % (sp, med, mn, bool(torch.equal(d.view(torch.int16), out[3][0].view(torch.int16)))))
-_os.environ.pop("RVB_SHADOW_SPEC")
 for msh in ("1", "0", "1", "0"):
     _os.environ["RVB_SHADOW_SH"] = msh
     cam.variant = 0
