@@ -29,7 +29,7 @@
 extern "C" {
 #endif
 
-#define RVB_ABI_VERSION 3
+#define RVB_ABI_VERSION 4
 
 typedef enum rvb_status {
     RVB_OK = 0,
@@ -63,20 +63,13 @@ int rvb_terrain_create(rvb_terrain** out,
                        const int32_t* triangles, int64_t T,
                        const uint16_t* vertices, int64_t V,
                        float res, float shift_x, float shift_y,
-                       int sem, void* stream);
-/* flags (rvb_terrain_create2; rvb_terrain_create = flags 0):
+                       int sem, int flags, void* stream);
+/* flags (0 = a heightmap layer with every list):
  *   RVB_LAYER_INDEX_ONLY  build the K-contiguous index and the triangle records only, not the block / superblock lists of the
  *                         heightmap ray-cast's production kernels: the layer of a Rock_Detection (rock_detect.py:151-158), whose
  *                         kernel scans the K-lists themselves -- 3.2 GB instead of 6 GB for the reference's rock index.
  *                         rvb_heightmap_raycast on such a layer runs the per-cell kernels (variants 1 / 2 and what 0 / 3 fall back to). */
 #define RVB_LAYER_INDEX_ONLY 1
-int rvb_terrain_create2(rvb_terrain** out,
-                        const int32_t* map_indices, int64_t G0, int64_t G1, int64_t K,
-                        int64_t stride_g0, int64_t stride_g1, int64_t stride_k,
-                        const int32_t* triangles, int64_t T,
-                        const uint16_t* vertices, int64_t V,
-                        float res, float shift_x, float shift_y,
-                        int sem, int flags, void* stream);
 int rvb_terrain_destroy(rvb_terrain* t);
 /* bytes of device memory owned by the handle */
 int64_t rvb_terrain_bytes(const rvb_terrain* t);
@@ -100,6 +93,10 @@ int64_t rvb_terrain_unbounded_triangles(const rvb_terrain* t);
  *   hit_tri      i32 [N,P]  triangle id        pt, sources f16 [N,P,3] (optional)
  *   obs/obs_ld/col_a/col_b: optional fused Heightmap.get_sparse_vector/get_dense_vector + rover.py:324-325:
  *        obs[n*obs_ld + col_a[p]] = obs[n*obs_ld + col_b[p]] = f32(fp16(dist/2))  for columns >= 0.
+ *   obs_h16/obs_h16_ld/obs_h16_col0: optional PACKED form of the same columns -- they are fp16 values by construction
+ *        (rover.py:324-325 stores fp16(dist / 2) into the f32 obs_buf), so a consumer that wants half the bytes passes
+ *        obs_h16[n*obs_h16_ld + (col - obs_h16_col0)] = fp16(dist/2)  for col in col_a/col_b >= 0  (obs may then be NULL).
+ *        Not available with variant 1.  rvb_env_step uses it for rvb_step_io.obs_h16.
  * `variant`: 0 = production ("shadow" kernel: enumerates triangles, not (ray, candidate) pairs; needs the layer's block
  * lists, i.e. K <= 255, otherwise the tiled kernel on per-cell lists runs), 1 = simple per-pair kernel kept for
  * cross-checking, 2 = tiled kernel on per-cell lists, 3 = tiled kernel on 3x3-cell block lists.  All four are
@@ -108,23 +105,13 @@ int64_t rvb_terrain_unbounded_triangles(const rvb_terrain* t);
 int rvb_heightmap_raycast(const rvb_terrain* t, const float* pos, const float* euler, const float* trig,
                           const double* pattern, int64_t P, int64_t N,
                           uint16_t* dist, int32_t* hit_slot, int32_t* hit_tri, uint16_t* pt, uint16_t* sources,
-                          float* obs, int64_t obs_ld, const int32_t* col_a, const int32_t* col_b,
-                          int variant, void* stream);
-
-/* The same with an optional PACKED observation output: the heightmap observation columns are fp16 values by construction
- * (rover.py:324-325 stores fp16(dist / 2) into the f32 obs_buf), so a consumer that wants half the bytes passes
- *   obs_h16 u16(f16) [N, obs_h16_ld]:  obs_h16[n*obs_h16_ld + (col - obs_h16_col0)] = fp16(dist/2)  for col in col_a/col_b >= 0
- * (obs may then be NULL).  Not available with variant 1.  rvb_env_step uses this entry point for rvb_step_io.obs_h16. */
-int rvb_heightmap_raycast2(const rvb_terrain* t, const float* pos, const float* euler, const float* trig,
-                           const double* pattern, int64_t P, int64_t N,
-                           uint16_t* dist, int32_t* hit_slot, int32_t* hit_tri, uint16_t* pt, uint16_t* sources,
-                           float* obs, int64_t obs_ld, uint16_t* obs_h16, int64_t obs_h16_ld, int obs_h16_col0,
-                           const int32_t* col_a, const int32_t* col_b, int variant, void* stream);
+                          float* obs, int64_t obs_ld, uint16_t* obs_h16, int64_t obs_h16_ld, int obs_h16_col0,
+                          const int32_t* col_a, const int32_t* col_b, int variant, void* stream);
 
 /* Cast pre-computed fp16 rays (sources/directions [R,3], directions NOT normalised, as handed to
  * ray_distance by camera.py:110) against a layer: _height_lookup + gather + ray_distance + min over K. */
 int rvb_cast_rays(const rvb_terrain* t, const uint16_t* sources, const uint16_t* directions, int64_t R,
-                  uint16_t* dist, int32_t* hit_slot, int32_t* hit_tri, uint16_t* pt, int variant, void* stream);
+                  uint16_t* dist, int32_t* hit_slot, int32_t* hit_tri, uint16_t* pt, void* stream);
 
 /* ray_distance(sources, directions, triangles) (utils/camera/ray_casting.py:3-66): n rays vs n triangles,
  * fp16.  sources, directions [n,3]; triangles [n,3,3]; k [n]; pt [n,3] (optional). */
@@ -138,22 +125,17 @@ int rvb_ray_distance(const uint16_t* sources, const uint16_t* directions, const 
  *   joints f32 [N,13] (DOF order rock_detect.py:174-188)    wheel_dist f16 [N,24]   body_dist f16 [N,2]
  *   hit_tri i32 [N,26] optional    collision i64 [N] optional (|min wheel| < 0.8 or |min body| < 0.45)
  *   rays_out f16 [N,26,6] optional (source xyz, direction xyz as fed to the ray-cast; for tests)
+ *   joint_trig f32 [N,18] optional = (sin j_i, cos j_i) for the DOFs i = 0..8 the wheel chain uses (rock_detect.py:248-291),
+ *        NULL = sinf/cosf on the device.  Like `trig` for the body rotation: libm results differ in the last ulp between
+ *        torch-CPU, torch-CUDA and CUDA's sinf, and parity tests that demand bit-identical rays inject the oracle's values.
  * ---------------------------------------------------------------------------------------------- */
 int rvb_rock_collision(const rvb_terrain* rocks, const float* pos, const float* euler, const float* trig,
-                       const float* joints, int64_t N,
-                       uint16_t* wheel_dist, uint16_t* body_dist, int32_t* hit_tri, int64_t* collision,
-                       uint16_t* rays_out, int variant, void* stream);
-/* The same with the joint trigonometry supplied by the caller: joint_trig f32 [N,18] = (sin j_i, cos j_i) for the DOFs
- * i = 0..8 the wheel chain uses (rock_detect.py:248-291), NULL = sinf/cosf on the device.  Like `trig` for the body rotation:
- * libm results differ in the last ulp between torch-CPU, torch-CUDA and CUDA's sinf, and parity tests that demand bit-identical
- * rays inject the oracle's values. */
-int rvb_rock_collision2(const rvb_terrain* rocks, const float* pos, const float* euler, const float* trig,
                        const float* joints, const float* joint_trig, int64_t N,
                        uint16_t* wheel_dist, uint16_t* body_dist, int32_t* hit_tri, int64_t* collision,
-                       uint16_t* rays_out, int variant, void* stream);
-/* check_collision alone (rover.py:663-668) on caller-provided distances. */
-int rvb_check_collision(const uint16_t* wheel_dist, const uint16_t* body_dist, int64_t N, int64_t* collision,
-                        int sem, void* stream);
+                       uint16_t* rays_out, void* stream);
+/* check_collision alone (rover.py:663-668) on caller-provided distances.  Both torch backends round the thresholds to fp16
+ * before the compare, so the flags do not depend on `sem` and the call takes none. */
+int rvb_check_collision(const uint16_t* wheel_dist, const uint16_t* body_dist, int64_t N, int64_t* collision, void* stream);
 
 /* tensor_quat_to_eul (utils/math/tensor_quat_to_euler.py:6-31): wxyz f32 [N,4] -> (roll,pitch,yaw) f32 [N,3] */
 int rvb_quat_to_euler(const float* quat, int64_t N, float* euler, void* stream);
@@ -300,9 +282,12 @@ int rvb_build_knn_index(const int32_t* triangles, int64_t T, const uint16_t* ver
  * borrowed DEVICE pointers that may be released when rvb_policy_create returns (it re-packs them into k-major panels
  * owned by the handle and synchronises `stream`).  enc_sparse / enc_dense point at 2 layers, mlp at 3, head at 1.
  * `device` must be the calling thread's current CUDA device (the library never switches devices).
- * fp32 FMA arithmetic like the reference's (TF32 off); accumulation order differs from cuBLAS, parity gate 2e-5 absolute.
- * rvb_policy_forward: obs f32 [N, obs_ld] (obs_ld >= p+S+D) -> out f32 [N, out_ld] columns 0..head-1; one kernel, reads obs
- * once, asynchronous on `stream`; the handle is immutable => usable from any stream.
+ * fp32-grade arithmetic like the reference's (TF32 off); accumulation order differs from cuBLAS, parity gate 2e-5 absolute.
+ * rvb_policy_forward: obs f32 [N, obs_ld] (obs_ld >= p+S+D) -> out f32 [N, out_ld] columns 0..head-1, asynchronous on `stream`;
+ * the handle is immutable => usable from any stream.  Two kernels on the tensor cores (tcgen05, tf32 hi + lo operands,
+ * accumulators in TMEM): the first encoder layers, then the rest of the network as a programmatic dependent launch.  Shapes that
+ * path refuses (p != 4, odd S, D or obs_ld, obs not 8-byte aligned) run one fp32 FFMA2 kernel instead, which computes the same
+ * layers in another summation order.
  * ---------------------------------------------------------------------------------------------- */
 typedef struct rvb_policy rvb_policy;
 typedef struct rvb_linear {
@@ -321,9 +306,10 @@ int rvb_policy_destroy(rvb_policy* policy);
 int64_t rvb_policy_bytes(const rvb_policy* policy);
 int rvb_policy_forward(const rvb_policy* policy, const float* obs, int64_t obs_ld, int64_t N, float* out, int64_t out_ld,
                        void* stream);
-/* Inner-loop variant of the policy kernel, process-wide: 1 = packed FFMA2 (two fp32 FMAs per issue slot; default),
- * 0 = scalar FFMA.  Both are IEEE fma per element => bit-identical results; exists for A/B measurement.  Returns the previous
- * value; any other argument only queries. */
+/* Policy dispatch, process-wide: 2 = default (tensor-core path where the shape allows it, FFMA2 kernel otherwise), 1 = the FFMA2
+ * kernel for every shape.  The hook bench.py (`ffma2_kernel_ms`) and the tests use to force the FFMA path.  1 or 2 sets the
+ * dispatch and returns the previous value; a negative argument only queries it; anything else (0 and 3 selected kernels that are
+ * gone) returns RVB_ERR_INVALID and leaves the setting unchanged. */
 int rvb_policy_variant(int variant);
 /* Two networks on the same observations in ONE launch (grid.y = network): what a PPO step asks for -- policy.compute and
  * value.compute on the same states.  Twice the CTAs for the same obs tile (second read served by L2). */

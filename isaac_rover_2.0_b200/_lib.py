@@ -13,7 +13,7 @@ _lib = None
 
 SEM_TORCH_CUDA = 0
 SEM_TORCH_CPU = 1
-LAYER_INDEX_ONLY = 1          # rvb_terrain_create2 flag
+LAYER_INDEX_ONLY = 1          # RVB_LAYER_INDEX_ONLY, a `flags` bit of rvb_terrain_create
 N_STATS = 16
 
 p = C.c_void_p
@@ -49,20 +49,17 @@ class StepIO(C.Structure):
 _SIGNATURES = {
     "rvb_abi_version": (C.c_int, []),
     "rvb_last_error": (C.c_char_p, []),
-    "rvb_terrain_create": (C.c_int, [C.POINTER(p), p, i64, i64, i64, i64, i64, i64, p, i64, p, i64, f32, f32, f32, C.c_int, p]),
+    "rvb_terrain_create": (C.c_int, [C.POINTER(p), p, i64, i64, i64, i64, i64, i64, p, i64, p, i64, f32, f32, f32, C.c_int, C.c_int, p]),
     "rvb_terrain_destroy": (C.c_int, [p]),
-    "rvb_terrain_create2": (C.c_int, [C.POINTER(p), p, i64, i64, i64, i64, i64, i64, p, i64, p, i64, f32, f32, f32, C.c_int, C.c_int, p]),
     "rvb_terrain_bytes": (i64, [p]),
     "rvb_terrain_release_index": (C.c_int, [p]),
     "rvb_terrain_has_index": (C.c_int, [p]),
     "rvb_terrain_unbounded_triangles": (i64, [p]),
-    "rvb_heightmap_raycast": (C.c_int, [p, p, p, p, p, i64, i64, p, p, p, p, p, p, i64, p, p, C.c_int, p]),
-    "rvb_heightmap_raycast2": (C.c_int, [p, p, p, p, p, i64, i64, p, p, p, p, p, p, i64, p, i64, C.c_int, p, p, C.c_int, p]),
-    "rvb_cast_rays": (C.c_int, [p, p, p, i64, p, p, p, p, C.c_int, p]),
+    "rvb_heightmap_raycast": (C.c_int, [p, p, p, p, p, i64, i64, p, p, p, p, p, p, i64, p, i64, C.c_int, p, p, C.c_int, p]),
+    "rvb_cast_rays": (C.c_int, [p, p, p, i64, p, p, p, p, p]),
     "rvb_ray_distance": (C.c_int, [p, p, p, i64, p, p, p]),
-    "rvb_rock_collision": (C.c_int, [p, p, p, p, p, i64, p, p, p, p, p, C.c_int, p]),
-    "rvb_rock_collision2": (C.c_int, [p, p, p, p, p, p, i64, p, p, p, p, p, C.c_int, p]),
-    "rvb_check_collision": (C.c_int, [p, p, i64, p, C.c_int, p]),
+    "rvb_rock_collision": (C.c_int, [p, p, p, p, p, p, i64, p, p, p, p, p, p]),
+    "rvb_check_collision": (C.c_int, [p, p, i64, p, p]),
     "rvb_quat_to_euler": (C.c_int, [p, i64, p, p]),
     "rvb_ackermann": (C.c_int, [p, i64, p, i64, i64, p, p, p, p, C.c_int, p]),
     "rvb_history_push": (C.c_int, [p, i64, i64, p, i64, p]),
@@ -98,8 +95,8 @@ def lib_path():
 
 
 # kernels launched per entry point (for bench.py's `gpu_launches` claim)
-KERNELS_PER_CALL = {"rvb_terrain_create": 2, "rvb_terrain_create2": 2, "rvb_heightmap_raycast": 4, "rvb_heightmap_raycast2": 4, "rvb_cast_rays": 2, "rvb_ray_distance": 1,
-                    "rvb_rock_collision": 1, "rvb_rock_collision2": 1, "rvb_check_collision": 1, "rvb_quat_to_euler": 1, "rvb_ackermann": 1,
+KERNELS_PER_CALL = {"rvb_terrain_create": 2, "rvb_heightmap_raycast": 4, "rvb_cast_rays": 2, "rvb_ray_distance": 1,
+                    "rvb_rock_collision": 1, "rvb_check_collision": 1, "rvb_quat_to_euler": 1, "rvb_ackermann": 1,
                     "rvb_history_push": 1, "rvb_obs_proprio": 1, "rvb_obs_gather": 1, "rvb_reward_reset": 2, "rvb_env_step": 8,
     "rvb_stone_validate": 1, "rvb_spawn_validate": 1, "rvb_height_lookup": 1, "rvb_build_knn_index": 6, "rvb_reset_targets": 1,
                     "rvb_policy_create": 7, "rvb_policy_forward": 1, "rvb_policy_forward_pair": 1,
@@ -147,7 +144,7 @@ def load():
         fn.restype = res
         fn.argtypes = args
         setattr(lib, name, _Counted(fn, KERNELS_PER_CALL[name]) if name in KERNELS_PER_CALL else fn)
-    if lib.rvb_abi_version() != 3:
+    if lib.rvb_abi_version() != 4:
         raise RuntimeError("librover_b200.so ABI version mismatch")
     _lib = lib
     return lib

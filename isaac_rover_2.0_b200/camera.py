@@ -68,7 +68,7 @@ class Camera():
             _lib.check(lib.rvb_heightmap_raycast(
                 self.layer.handle, _lib.ptr(pos), _lib.ptr(rot), _lib.ptr(trig), _lib.ptr(self.heightmap_distribution), P, N,
                 _lib.ptr(dist), _lib.ptr(slot), _lib.ptr(tri), _lib.ptr(pt), _lib.ptr(src),
-                _lib.ptr(obs), 0 if obs is None else obs.stride(0), _lib.ptr(self._col_a if obs is not None else None),
+                _lib.ptr(obs), 0 if obs is None else obs.stride(0), None, 0, 0, _lib.ptr(self._col_a if obs is not None else None),
                 _lib.ptr(self._col_b if obs is not None else None), self.variant, _lib.stream_of(pos)))
         # variant 0 launches four kernels (classify, tiled kernel on the steep list, shadow, tiled kernel on the hand-back list),
         # variant 1 two (set-up + cast), variants 2/3 one
@@ -97,5 +97,5 @@ def cast_rays(layer, sources, directions, want_hits=False):
     tri = torch.empty((R,), dtype=torch.int32, device=s.device) if want_hits else None
     with torch.cuda.device(s.device):
         _lib.check(lib.rvb_cast_rays(layer.handle, _lib.ptr(s), _lib.ptr(d), R, _lib.ptr(dist), _lib.ptr(slot), _lib.ptr(tri),
-                                     _lib.ptr(pt), 0, _lib.stream_of(s)))
+                                     _lib.ptr(pt), _lib.stream_of(s)))
     return (dist, pt, slot, tri) if want_hits else (dist, pt)

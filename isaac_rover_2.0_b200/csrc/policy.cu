@@ -7,11 +7,13 @@
 //   x  = Linear(124,256)+act, Linear(256,160)+act, Linear(160,128)+act, Linear(128,A) [+ Tanh for the actor] (model.py:169-177,190-191)
 // with the layer widths the reference hard-wires (train.py:95, cfg/trainSKRL/RoverPPOSKRL.yaml:4-9).
 //
-// Arithmetic: the reference runs torch fp32 nn.Linear (TF32 is off by default for matmuls), so this kernel is an fp32
-// FMA chain -- no tensor cores: a bf16/TF32 contraction would change the answer by 1e-3, and the whole net is
-// 0.27 MFMA per env (2.2 GFLOP per 4096-env step), i.e. tens of microseconds of fp32 pipe.  Sums are accumulated in
-// k order per output with fmaf (cuBLAS's order is unspecified; the parity gate is 2e-5 absolute against an fp64 oracle).
+// Arithmetic: the reference runs torch fp32 nn.Linear (TF32 is off by default for matmuls), and a single-pass bf16/TF32
+// contraction would change the answer by 1e-3.  The default path (policy_l1_tc_kernel + policy_tail_tc_kernel, below) runs the
+// network on tcgen05 with every operand split into tf32 hi + lo parts, which is fp32-grade.  policy_forward_kernel, an fp32 FFMA2
+// chain, is the fall-back for the shapes the tensor-core path refuses (tc_usable) and what rvb_policy_variant(1) forces.  Both
+// differ from cuBLAS in the summation order (unspecified there); the parity gate is 2e-5 absolute against an fp64 oracle.
 //
+// policy_forward_kernel: sums are accumulated in k order per output with packed fp32 FMAs (ffma2, IEEE fma per element).
 // One CTA of 256 threads per tile of TM = 32 envs; every activation of the tile stays in shared memory from the
 // observation row to the action (k-major [k][env], row stride 36 floats), so obs is read exactly once from HBM/L2 and
 // nothing but the A outputs is written.  Weights are re-packed once per handle into k-major, 32-column-padded panels
@@ -110,7 +112,7 @@ __global__ void pl_pack_kernel(const float* __restrict__ w, const float* __restr
 // One dense layer of the tile.  Input activations: shared memory `act_in` [K][PL_LDA] (GLOBAL_IN = false) or columns
 // [col0, col0 + K) of the tile's observation rows in global memory, staged transposed through `xs` (GLOBAL_IN = true).
 // Output: act(in . Wt + bias) into shared memory `act_out` [n][PL_LDA], rows n < OUT only.
-template <int CN, bool GLOBAL_IN, bool F2>
+template <int CN, bool GLOBAL_IN>
 __device__ __forceinline__ void pl_dense(const float* __restrict__ act_in, const float* __restrict__ obs, int64_t obs_ld, int64_t m0,
                                          int64_t N, int col0, int K, const PackedLinear& L, float* __restrict__ xs,
                                          float* __restrict__ ws, float* __restrict__ act_out, int act_kind) {
@@ -159,40 +161,23 @@ __device__ __forceinline__ void pl_dense(const float* __restrict__ act_in, const
         __syncthreads();
         if (k0 + KC < K) fetch(k0 + KC);
         const float* a_base = GLOBAL_IN ? xs : act_in + (int64_t)k0 * PL_LDA;
-        if (F2) {
-            auto step = [&](int kk) {
-                const float4 a = *reinterpret_cast<const float4*>(a_base + kk * PL_LDA + mg * 4);
-                float w[CN];
+        auto step = [&](int kk) {
+            const float4 a = *reinterpret_cast<const float4*>(a_base + kk * PL_LDA + mg * 4);
+            float w[CN];
 #pragma unroll
-                for (int j = 0; j < CN; ++j) w[j] = ws[kk * OUTP + ng + 32 * j];
+            for (int j = 0; j < CN; ++j) w[j] = ws[kk * OUTP + ng + 32 * j];
 #pragma unroll
-                for (int j = 0; j < CN; ++j) {
-                    ffma2(acc[0][j], acc[1][j], a.x, a.y, w[j]);
-                    ffma2(acc[2][j], acc[3][j], a.z, a.w, w[j]);
-                }
-            };
-            if (kc == KC) {                                // full chunks: no loop overhead
-#pragma unroll
-                for (int kk = 0; kk < KC; ++kk) step(kk);
-            } else {
-#pragma unroll 4
-                for (int kk = 0; kk < kc; ++kk) step(kk);
+            for (int j = 0; j < CN; ++j) {
+                ffma2(acc[0][j], acc[1][j], a.x, a.y, w[j]);
+                ffma2(acc[2][j], acc[3][j], a.z, a.w, w[j]);
             }
+        };
+        if (kc == KC) {                                    // full chunks: no loop overhead
+#pragma unroll
+            for (int kk = 0; kk < KC; ++kk) step(kk);
         } else {
 #pragma unroll 4
-            for (int kk = 0; kk < kc; ++kk) {
-                const float4 a = *reinterpret_cast<const float4*>(a_base + kk * PL_LDA + mg * 4);
-                float w[CN];
-#pragma unroll
-                for (int j = 0; j < CN; ++j) w[j] = ws[kk * OUTP + ng + 32 * j];
-#pragma unroll
-                for (int j = 0; j < CN; ++j) {
-                    acc[0][j] = fmaf(a.x, w[j], acc[0][j]);
-                    acc[1][j] = fmaf(a.y, w[j], acc[1][j]);
-                    acc[2][j] = fmaf(a.z, w[j], acc[2][j]);
-                    acc[3][j] = fmaf(a.w, w[j], acc[3][j]);
-                }
-            }
+            for (int kk = 0; kk < kc; ++kk) step(kk);
         }
     }
 #pragma unroll
@@ -219,7 +204,6 @@ __device__ __forceinline__ void pl_dense(const float* __restrict__ act_in, const
 #define PL_SM_FLOATS (PL_SM_WS + PL_WS_FLOATS)
 #define PL_SMEM_BYTES (PL_SM_FLOATS * 4)
 
-template <bool F2>
 __global__ void __launch_bounds__(PL_THREADS, 2)
 policy_forward_kernel(const PolicyDev* __restrict__ p0, const PolicyDev* __restrict__ p1, const float* __restrict__ obs,
                       int64_t obs_ld, int64_t N, float* __restrict__ out0, int64_t out0_ld, float* __restrict__ out1,
@@ -244,15 +228,15 @@ policy_forward_kernel(const PolicyDev* __restrict__ p0, const PolicyDev* __restr
         A[k * PL_LDA + m] = (m0 + m < N) ? __ldg(obs + (m0 + m) * obs_ld + k) : 0.f;
     }
     // sparse encoder (model.py:186) -> concat rows p .. p+59
-    pl_dense<3, true, F2>(nullptr, obs, obs_ld, m0, N, p, P.n_sparse, P.es1, xs, ws, Cb, P.act);
-    pl_dense<2, false, F2>(Cb, nullptr, 0, 0, 0, 0, PL_E1, P.es2, xs, ws, A + p * PL_LDA, P.act);
+    pl_dense<3, true>(nullptr, obs, obs_ld, m0, N, p, P.n_sparse, P.es1, xs, ws, Cb, P.act);
+    pl_dense<2, false>(Cb, nullptr, 0, 0, 0, 0, PL_E1, P.es2, xs, ws, A + p * PL_LDA, P.act);
     // dense encoder (model.py:187) -> concat rows p+60 .. p+119
-    pl_dense<3, true, F2>(nullptr, obs, obs_ld, m0, N, p + P.n_sparse, P.n_dense, P.ed1, xs, ws, Cb, P.act);
-    pl_dense<2, false, F2>(Cb, nullptr, 0, 0, 0, 0, PL_E1, P.ed2, xs, ws, A + (p + PL_E2) * PL_LDA, P.act);
+    pl_dense<3, true>(nullptr, obs, obs_ld, m0, N, p + P.n_sparse, P.n_dense, P.ed1, xs, ws, Cb, P.act);
+    pl_dense<2, false>(Cb, nullptr, 0, 0, 0, 0, PL_E1, P.ed2, xs, ws, A + (p + PL_E2) * PL_LDA, P.act);
     // MLP (model.py:190-191)
-    pl_dense<8, false, F2>(A, nullptr, 0, 0, 0, 0, p + 2 * PL_E2, P.m1, xs, ws, B, P.act);
-    pl_dense<5, false, F2>(B, nullptr, 0, 0, 0, 0, PL_M1, P.m2, xs, ws, Cb, P.act);
-    pl_dense<4, false, F2>(Cb, nullptr, 0, 0, 0, 0, PL_M2, P.m3, xs, ws, A, P.act);
+    pl_dense<8, false>(A, nullptr, 0, 0, 0, 0, p + 2 * PL_E2, P.m1, xs, ws, B, P.act);
+    pl_dense<5, false>(B, nullptr, 0, 0, 0, 0, PL_M1, P.m2, xs, ws, Cb, P.act);
+    pl_dense<4, false>(Cb, nullptr, 0, 0, 0, 0, PL_M2, P.m3, xs, ws, A, P.act);
     __syncthreads();
     // head: Linear(128, A) [+ Tanh] -- warp o computes output o for the tile's 32 envs
     const int m = tid & 31, o = tid >> 5;
@@ -900,8 +884,7 @@ extern "C" int rvb_policy_create(rvb_policy** out, int32_t n_proprio, int32_t n_
     if (e == cudaSuccess)       // the descriptor the kernel reads (P outlives the copy: the stream is synchronised below)
         e = cudaMemcpyAsync(P->storage, static_cast<const PolicyDev*>(P), sizeof(PolicyDev), cudaMemcpyHostToDevice, st);
     if (e == cudaSuccess) e = cudaGetLastError();
-    if (e == cudaSuccess) e = cudaFuncSetAttribute(policy_forward_kernel<false>, cudaFuncAttributeMaxDynamicSharedMemorySize, PL_SMEM_BYTES);
-    if (e == cudaSuccess) e = cudaFuncSetAttribute(policy_forward_kernel<true>, cudaFuncAttributeMaxDynamicSharedMemorySize, PL_SMEM_BYTES);
+    if (e == cudaSuccess) e = cudaFuncSetAttribute(policy_forward_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, PL_SMEM_BYTES);
     if (e == cudaSuccess) e = cudaFuncSetAttribute(policy_l1_tc_kernel<1>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)tc_smem_bytes(1));
     if (e == cudaSuccess) e = cudaFuncSetAttribute(policy_l1_tc_kernel<2>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)tc_smem_bytes(2));
     if (e == cudaSuccess) e = cudaFuncSetAttribute(policy_tail_tc_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)tt_smem_bytes());
@@ -925,19 +908,21 @@ extern "C" int rvb_policy_destroy(rvb_policy* P) {
 extern "C" int64_t rvb_policy_bytes(const rvb_policy* P) { return P ? P->storage_floats * (int64_t)sizeof(float) : 0; }
 
 // 2 (default) = the whole network on tcgen05 (policy_l1_tc_kernel + policy_tail_tc_kernel: faster than the FFMA path from a single
-// 128-env tile upwards); 3 = the same (kept for the tests that force the path); 1 = packed FFMA2 throughout (round 1's kernel);
-// 0 = scalar FFMA throughout.  1 and 0 are bit-identical; 2 / 3 differ from them in the summation order (all within 2e-5 of the
-// fp64 oracle, the gate of the tests).
+// 128-env tile upwards) where tc_usable allows it, policy_forward_kernel otherwise; 1 = policy_forward_kernel for every shape (what
+// bench.py's ffma2_kernel_ms and the tests force).  The two sum in different orders, both within 2e-5 of the fp64 oracle (the gate
+// of the tests).
 static int g_policy_variant = 2;
 extern "C" int rvb_policy_variant(int v) {
+    if (v < 0) return g_policy_variant;
+    RVB_REQUIRE(v == 1 || v == 2, "rvb_policy_variant: 1 (FFMA2 kernel) or 2 (default dispatch); variants 0 (scalar FFMA) and 3 are removed");
     const int prev = g_policy_variant;
-    if (v >= 0 && v <= 3) g_policy_variant = v;
+    g_policy_variant = v;
     return prev;
 }
 
 // the tensor-core path reads the observation rows with 8-byte loads
-static bool tc_usable(const PolicyDev* P, const float* obs, int64_t obs_ld, int64_t /*N*/) {
-    return (g_policy_variant == 3 || g_policy_variant == 2) && (obs_ld % 2 == 0) && (P->n_proprio == 4) && (P->n_sparse % 2 == 0) && (P->n_dense % 2 == 0) && (((uintptr_t)obs & 7u) == 0);
+static bool tc_usable(const PolicyDev* P, const float* obs, int64_t obs_ld) {
+    return g_policy_variant == 2 && (obs_ld % 2 == 0) && (P->n_proprio == 4) && (P->n_sparse % 2 == 0) && (P->n_dense % 2 == 0) && (((uintptr_t)obs & 7u) == 0);
 }
 
 static int check_forward(const rvb_policy* P, const float* obs, int64_t obs_ld, const float* out, int64_t out_ld) {
@@ -966,29 +951,38 @@ static cudaError_t launch_tail_tc(dim3 grid, cudaStream_t st, const PolicyDev* a
     return cudaLaunchKernelEx(&cfg, policy_tail_tc_kernel, a, b, obs, obs_ld, N, h1, nets, out0, out0_ld, out1, out1_ld);
 }
 
+// One network (B == nullptr) or two on the same observations (grid.y = network; the pair's first layers share the observation tiles).
+static int policy_launch(const char* name, const rvb_policy* A, const rvb_policy* B, const float* obs, int64_t obs_ld, int64_t N,
+                         float* out_a, int64_t out_a_ld, float* out_b, int64_t out_b_ld, cudaStream_t st) {
+    RVB_REQUIRE(N <= (int64_t)PL_TM * 0x7fffffff, "rvb_policy_forward: too many envs");
+    const int nets = B ? 2 : 1;
+    const PolicyDev* db = B ? B->dev : nullptr;
+    float* h1 = nullptr;
+    cudaError_t le = cudaSuccess;
+    if (tc_usable(A, obs, obs_ld)) {
+        RVB_CUDA(rvb_scratch_alloc((void**)&h1, sizeof(float) * (size_t)N * nets * 2 * PL_E1, st));
+        const dim3 grid((unsigned)ceil_div(N, TC_M), 2);
+        if (B) policy_l1_tc_kernel<2><<<grid, TC_THREADS, tc_smem_bytes(2), st>>>(A->dev, db, obs, obs_ld, N, h1);
+        else policy_l1_tc_kernel<1><<<grid, TC_THREADS, tc_smem_bytes(1), st>>>(A->dev, db, obs, obs_ld, N, h1);
+        le = launch_tail_tc(dim3((unsigned)ceil_div(N, TC_M), nets), st, A->dev, db, obs, obs_ld, N, h1, nets, out_a, out_a_ld, out_b, out_b_ld);
+    } else {
+        policy_forward_kernel<<<dim3((unsigned)ceil_div(N, PL_TM), nets), PL_THREADS, PL_SMEM_BYTES, st>>>(A->dev, db, obs, obs_ld, N, out_a,
+                                                                                                       out_a_ld, out_b, out_b_ld);
+    }
+    const cudaError_t last = cudaGetLastError();          // also clears the error state of a failed launch
+    if (le == cudaSuccess) le = last;
+    if (h1) cudaFreeAsync(h1, st);
+    if (le != cudaSuccess) return rvb_set_error(RVB_ERR_CUDA, name, cudaGetErrorString(le));
+    return RVB_OK;
+}
+
 extern "C" int rvb_policy_forward(const rvb_policy* P, const float* obs, int64_t obs_ld, int64_t N, float* out, int64_t out_ld,
                                   void* stream) {
     RVB_REQUIRE(P, "rvb_policy_forward: null handle");
     if (N <= 0) return RVB_OK;
     int rc;
     if ((rc = check_forward(P, obs, obs_ld, out, out_ld))) return rc;
-    RVB_REQUIRE(N <= (int64_t)PL_TM * 0x7fffffff, "rvb_policy_forward: too many envs");
-    auto kern = g_policy_variant ? policy_forward_kernel<true> : policy_forward_kernel<false>;
-    cudaStream_t st = as_stream(stream);
-    float* h1 = nullptr;
-    cudaError_t le = cudaSuccess;
-    if (tc_usable(P, obs, obs_ld, N)) {
-        RVB_CUDA(rvb_scratch_alloc((void**)&h1, sizeof(float) * (size_t)N * 2 * PL_E1, st));
-        policy_l1_tc_kernel<1><<<dim3((unsigned)ceil_div(N, TC_M), 2), TC_THREADS, tc_smem_bytes(1), st>>>(P->dev, nullptr, obs, obs_ld, N, h1);
-        le = launch_tail_tc(dim3((unsigned)ceil_div(N, TC_M), 1), st, P->dev, nullptr, obs, obs_ld, N, h1, 1, out, out_ld, nullptr, 0);
-    } else {
-        kern<<<dim3((unsigned)ceil_div(N, PL_TM), 1), PL_THREADS, PL_SMEM_BYTES, st>>>(P->dev, nullptr, obs, obs_ld, N, out, out_ld, nullptr, 0);
-    }
-    const cudaError_t last = cudaGetLastError();          // also clears the error state of a failed launch
-    if (le == cudaSuccess) le = last;
-    if (h1) cudaFreeAsync(h1, st);
-    if (le != cudaSuccess) return rvb_set_error(RVB_ERR_CUDA, "rvb_policy_forward", cudaGetErrorString(le));
-    return RVB_OK;
+    return policy_launch("rvb_policy_forward", P, nullptr, obs, obs_ld, N, out, out_ld, nullptr, 0, as_stream(stream));
 }
 
 extern "C" int rvb_policy_forward_pair(const rvb_policy* A, const rvb_policy* B, const float* obs, int64_t obs_ld, int64_t N,
@@ -999,24 +993,8 @@ extern "C" int rvb_policy_forward_pair(const rvb_policy* A, const rvb_policy* B,
     if ((rc = check_forward(A, obs, obs_ld, out_a, out_a_ld))) return rc;
     if ((rc = check_forward(B, obs, obs_ld, out_b, out_b_ld))) return rc;
     RVB_REQUIRE(A->device == B->device, "rvb_policy_forward_pair: the two networks live on different devices");
-    RVB_REQUIRE(N <= (int64_t)PL_TM * 0x7fffffff, "rvb_policy_forward: too many envs");
     RVB_REQUIRE(A->n_proprio == B->n_proprio && A->n_sparse == B->n_sparse && A->n_dense == B->n_dense,
                 "rvb_policy_forward_pair: the two networks read different observation splits");
     RVB_REQUIRE(A->act == B->act, "rvb_policy_forward_pair: the two networks use different activations");
-    auto kern = g_policy_variant ? policy_forward_kernel<true> : policy_forward_kernel<false>;
-    cudaStream_t st = as_stream(stream);
-    float* h1 = nullptr;
-    cudaError_t le = cudaSuccess;
-    if (tc_usable(A, obs, obs_ld, N)) {          // both networks' first layers in one launch: they share the observation tiles
-        RVB_CUDA(rvb_scratch_alloc((void**)&h1, sizeof(float) * (size_t)N * 4 * PL_E1, st));
-        policy_l1_tc_kernel<2><<<dim3((unsigned)ceil_div(N, TC_M), 2), TC_THREADS, tc_smem_bytes(2), st>>>(A->dev, B->dev, obs, obs_ld, N, h1);
-        le = launch_tail_tc(dim3((unsigned)ceil_div(N, TC_M), 2), st, A->dev, B->dev, obs, obs_ld, N, h1, 2, out_a, out_a_ld, out_b, out_b_ld);
-    } else {
-        kern<<<dim3((unsigned)ceil_div(N, PL_TM), 2), PL_THREADS, PL_SMEM_BYTES, st>>>(A->dev, B->dev, obs, obs_ld, N, out_a, out_a_ld, out_b, out_b_ld);
-    }
-    const cudaError_t last = cudaGetLastError();          // also clears the error state of a failed launch
-    if (le == cudaSuccess) le = last;
-    if (h1) cudaFreeAsync(h1, st);
-    if (le != cudaSuccess) return rvb_set_error(RVB_ERR_CUDA, "rvb_policy_forward_pair", cudaGetErrorString(le));
-    return RVB_OK;
+    return policy_launch("rvb_policy_forward_pair", A, B, obs, obs_ld, N, out_a, out_a_ld, out_b, out_b_ld, as_stream(stream));
 }

@@ -3,7 +3,7 @@
 //
 // variant 1 ("simple"): one warp per ray, lanes stride over the K candidates of the ray's cell, every
 // (ray, candidate) pair evaluated with the literal op sequence of ray_casting.py.  Kept as the on-device
-// cross-check for the production kernel (raycast_tiled.cu).
+// cross-check for the production kernel (raycast_shadow.cu) and its tiled fall-back (raycast_tiled.cu).
 #include "raycast_common.cuh"
 
 int launch_heightmap_tiled(const rvb_terrain* t, const float* pos, const float* euler, const float* trig,
@@ -141,23 +141,15 @@ static int launch_cast_simple(const rvb_terrain* t, const __half* src16, const _
 extern "C" int rvb_heightmap_raycast(const rvb_terrain* t, const float* pos, const float* euler, const float* trig,
                                      const double* pattern, int64_t P, int64_t N, uint16_t* dist, int32_t* hit_slot,
                                      int32_t* hit_tri, uint16_t* pt, uint16_t* sources, float* obs, int64_t obs_ld,
-                                     const int32_t* col_a, const int32_t* col_b, int variant, void* stream) {
-    return rvb_heightmap_raycast2(t, pos, euler, trig, pattern, P, N, dist, hit_slot, hit_tri, pt, sources, obs, obs_ld, nullptr, 0,
-                                  0, col_a, col_b, variant, stream);
-}
-
-extern "C" int rvb_heightmap_raycast2(const rvb_terrain* t, const float* pos, const float* euler, const float* trig,
-                                      const double* pattern, int64_t P, int64_t N, uint16_t* dist, int32_t* hit_slot,
-                                      int32_t* hit_tri, uint16_t* pt, uint16_t* sources, float* obs, int64_t obs_ld,
-                                      uint16_t* obs_h16, int64_t obs_h16_ld, int obs_h16_col0, const int32_t* col_a,
-                                      const int32_t* col_b, int variant, void* stream) {
+                                     uint16_t* obs_h16, int64_t obs_h16_ld, int obs_h16_col0, const int32_t* col_a,
+                                     const int32_t* col_b, int variant, void* stream) {
     RVB_REQUIRE(N >= 0 && P > 0 && P <= 65535, "rvb_heightmap_raycast: need N >= 0, 0 < P <= 65535");
     if (N == 0) return RVB_OK;
     RVB_REQUIRE(t && pos && euler && pattern && dist, "rvb_heightmap_raycast: null pointer");
     RVB_REQUIRE(!obs || (col_a && col_b && obs_ld > 0), "rvb_heightmap_raycast: obs needs col_a, col_b, obs_ld");
-    RVB_REQUIRE(!obs_h16 || (col_a && col_b && obs_h16_ld > 0 && obs_h16_col0 >= 0), "rvb_heightmap_raycast2: obs_h16 needs col_a, col_b, obs_h16_ld");
+    RVB_REQUIRE(!obs_h16 || (col_a && col_b && obs_h16_ld > 0 && obs_h16_col0 >= 0), "rvb_heightmap_raycast: obs_h16 needs col_a, col_b, obs_h16_ld");
     RVB_REQUIRE(variant >= 0 && variant <= 3, "rvb_heightmap_raycast: variant must be 0, 1, 2 or 3");
-    RVB_REQUIRE(!obs_h16 || variant != 1, "rvb_heightmap_raycast2: the per-pair cross-check kernel (variant 1) has no packed output");
+    RVB_REQUIRE(!obs_h16 || variant != 1, "rvb_heightmap_raycast: the per-pair cross-check kernel (variant 1) has no packed output");
     RVB_REQUIRE(variant != 2 || t->index != nullptr, "rvb_heightmap_raycast: variant 2 reads the index the layer released (rvb_terrain_release_index)");
     const RvbObs16 o16v = {obs_h16, obs_h16_ld, obs_h16_col0};
     const RvbObs16* o16 = obs_h16 ? &o16v : nullptr;
@@ -192,13 +184,11 @@ extern "C" int rvb_heightmap_raycast2(const rvb_terrain* t, const float* pos, co
 }
 
 extern "C" int rvb_cast_rays(const rvb_terrain* t, const uint16_t* sources, const uint16_t* directions, int64_t R,
-                             uint16_t* dist, int32_t* hit_slot, int32_t* hit_tri, uint16_t* pt, int variant,
-                             void* stream) {
+                             uint16_t* dist, int32_t* hit_slot, int32_t* hit_tri, uint16_t* pt, void* stream) {
     RVB_REQUIRE(R >= 0, "rvb_cast_rays: R < 0");
     if (R == 0) return RVB_OK;
     RVB_REQUIRE(t && sources && directions && dist, "rvb_cast_rays: null pointer");
     RVB_REQUIRE(t->index != nullptr, "rvb_cast_rays: the layer released its index (rvb_terrain_release_index)");
-    (void)variant;
     cudaStream_t st = as_stream(stream);
     __half* dneg = nullptr;
     RVB_CUDA(rvb_scratch_alloc((void**)&dneg, sizeof(__half) * 3 * (size_t)R, st));

@@ -74,8 +74,8 @@ extern "C" int rvb_env_step(const rvb_terrain* terrain, const rvb_terrain* rocks
         RVB_CUDA(rvb_side_stream(0, &side));
         RVB_CUDA(cudaEventRecord(side->fork, st));
         RVB_CUDA(cudaStreamWaitEvent(side->s, side->fork, 0));
-        const int rc = rvb_rock_collision(rocks, io.pos, io.euler, nullptr, io.joints, N, io.wheel_dist, io.body_dist, nullptr,
-                                          io.rock_collision, nullptr, 0, side->s);
+        const int rc = rvb_rock_collision(rocks, io.pos, io.euler, nullptr, io.joints, nullptr, N, io.wheel_dist, io.body_dist,
+                                          nullptr, io.rock_collision, nullptr, side->s);
         if (rc != RVB_OK) return rc;
         RVB_CUDA(cudaEventRecord(side->join, side->s));
         guard.join = side->join;
@@ -96,8 +96,8 @@ extern "C" int rvb_env_step(const rvb_terrain* terrain, const rvb_terrain* rocks
     }
     // packed observation requested: the heightmap columns go to obs_h16 (fp16, what they are by construction) and the f32
     // columns 4.. of obs are left alone
-    int rc = rvb_heightmap_raycast2(terrain, io.pos, io.euler, nullptr, pattern, P, N, io.dist, nullptr, nullptr, nullptr, nullptr,
-                                    io.obs_h16 ? nullptr : io.obs, io.obs_ld, io.obs_h16, io.obs_h16_ld, 4, col_a, col_b, 0, st);
+    int rc = rvb_heightmap_raycast(terrain, io.pos, io.euler, nullptr, pattern, P, N, io.dist, nullptr, nullptr, nullptr, nullptr,
+                                   io.obs_h16 ? nullptr : io.obs, io.obs_ld, io.obs_h16, io.obs_h16_ld, 4, col_a, col_b, 0, st);
     if (rc != RVB_OK) return rc;
     if (t1) RVB_CUDA(cudaEventRecord(t1, st));
     if (guard.join) {

@@ -465,17 +465,9 @@ static int build_block_lists(rvb_terrain* t, cudaStream_t st) {
 extern "C" int rvb_terrain_create(rvb_terrain** out, const int32_t* map_indices, int64_t G0, int64_t G1, int64_t K,
                                   int64_t stride_g0, int64_t stride_g1, int64_t stride_k, const int32_t* triangles,
                                   int64_t T, const uint16_t* vertices, int64_t V, float res, float shift_x,
-                                  float shift_y, int sem, void* stream) {
-    return rvb_terrain_create2(out, map_indices, G0, G1, K, stride_g0, stride_g1, stride_k, triangles, T, vertices, V, res, shift_x,
-                               shift_y, sem, 0, stream);
-}
-
-extern "C" int rvb_terrain_create2(rvb_terrain** out, const int32_t* map_indices, int64_t G0, int64_t G1, int64_t K,
-                                   int64_t stride_g0, int64_t stride_g1, int64_t stride_k, const int32_t* triangles,
-                                   int64_t T, const uint16_t* vertices, int64_t V, float res, float shift_x,
-                                   float shift_y, int sem, int flags, void* stream) {
+                                  float shift_y, int sem, int flags, void* stream) {
     RVB_REQUIRE(out != nullptr, "rvb_terrain_create: out is null");
-    RVB_REQUIRE((flags & ~RVB_LAYER_INDEX_ONLY) == 0, "rvb_terrain_create2: unknown flag");
+    RVB_REQUIRE((flags & ~RVB_LAYER_INDEX_ONLY) == 0, "rvb_terrain_create: unknown flag");
     *out = nullptr;
     RVB_REQUIRE(map_indices && triangles && vertices, "rvb_terrain_create: null device pointer");
     RVB_REQUIRE(G0 > 0 && G1 > 0 && K > 0 && K <= 4096, "rvb_terrain_create: need G0,G1 > 0 and 0 < K <= 4096");
@@ -509,29 +501,17 @@ extern "C" int rvb_terrain_create2(rvb_terrain** out, const int32_t* map_indices
     hbad = hb2[0];
     t->n_ill = hb2[1];
     if (bad) cudaFree(bad);
+    // failure: the handle was zeroed at allocation, so rvb_terrain_destroy frees exactly what was built (cudaFree(nullptr) is a no-op)
     if (e == cudaSuccess && !hbad && !(flags & RVB_LAYER_INDEX_ONLY)) {
         const int rc = build_block_lists(t, st);
         if (rc == RVB_OK) e = cudaStreamSynchronize(st);
         if (rc != RVB_OK || e != cudaSuccess) {
-            cudaFree(t->index);
-            cudaFree(t->recs);
-            cudaFree(t->s1recs);
-            cudaFree(t->blk_off);
-            cudaFree(t->blk_ids);
-            cudaFree(t->blk_slots);
-            cudaFree(t->sb_off);
-            cudaFree(t->sb_ids);
-            cudaFree(t->sb_slot9);
-            cudaFree(t->sb_chunk);
-            delete t;
+            rvb_terrain_destroy(t);
             return rc != RVB_OK ? rc : rvb_set_error(RVB_ERR_CUDA, "rvb_terrain_create (block lists)", cudaGetErrorString(e));
         }
     }
     if (e != cudaSuccess || hbad) {
-        cudaFree(t->index);
-        cudaFree(t->recs);
-            cudaFree(t->s1recs);
-        delete t;
+        rvb_terrain_destroy(t);
         if (e != cudaSuccess) return rvb_set_error(RVB_ERR_CUDA, "rvb_terrain_create", cudaGetErrorString(e));
         return rvb_set_error(RVB_ERR_INVALID, "rvb_terrain_create",
                              hbad == 1 ? "map_indices holds a triangle id outside [0,T)"
@@ -545,7 +525,7 @@ extern "C" int rvb_terrain_destroy(rvb_terrain* t) {
     if (!t) return RVB_OK;
     cudaFree(t->index);
     cudaFree(t->recs);
-            cudaFree(t->s1recs);
+    cudaFree(t->s1recs);
     cudaFree(t->blk_off);
     cudaFree(t->blk_ids);
     cudaFree(t->blk_slots);

@@ -51,8 +51,8 @@ class Rock_Detection():
             if tuple(joint_trig.shape) != (N, 18):
                 raise ValueError("joint_trig must be [N,18]")
         with torch.cuda.device(dev):
-            _lib.check(lib.rvb_rock_collision2(self.layer.handle, _lib.ptr(pos), _lib.ptr(rot), _lib.ptr(trig), _lib.ptr(jnt),
-                                               _lib.ptr(joint_trig), N, _lib.ptr(wheel), _lib.ptr(body), _lib.ptr(tri), _lib.ptr(col),
-                                               _lib.ptr(rays), 0, _lib.stream_of(pos)))
+            _lib.check(lib.rvb_rock_collision(self.layer.handle, _lib.ptr(pos), _lib.ptr(rot), _lib.ptr(trig), _lib.ptr(jnt),
+                                              _lib.ptr(joint_trig), N, _lib.ptr(wheel), _lib.ptr(body), _lib.ptr(tri), _lib.ptr(col),
+                                              _lib.ptr(rays), _lib.stream_of(pos)))
         self.last_hit_tri, self.last_collision, self.last_rays = tri, col, rays
         return wheel, body

@@ -317,8 +317,7 @@ class RoverTask():
         b = body_dists.to(torch.float16).contiguous()
         out = torch.empty(w.shape[0], dtype=torch.long, device=w.device)
         with torch.cuda.device(w.device):
-            _lib.check(self._lib.rvb_check_collision(_lib.ptr(w), _lib.ptr(b), w.shape[0], _lib.ptr(out), self.sem,
-                                                     self._stream()))
+            _lib.check(self._lib.rvb_check_collision(_lib.ptr(w), _lib.ptr(b), w.shape[0], _lib.ptr(out), self._stream()))
         self.rock_collison = out
         return out
 

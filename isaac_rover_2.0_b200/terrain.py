@@ -34,11 +34,11 @@ class TerrainLayer:
         self.sem = sem
         h = C.c_void_p()
         with torch.cuda.device(self.device):
-            _lib.check(lib.rvb_terrain_create2(C.byref(h), _lib.ptr(view), self.G0, self.G1, self.K,
-                                               view.stride(0), view.stride(1), view.stride(2),
-                                               _lib.ptr(tri), self.T, _lib.ptr(ver), self.V,
-                                               self.res, float(shift[0]), float(shift[1]), sem,
-                                               _lib.LAYER_INDEX_ONLY if index_only else 0, _lib.stream_of(idx)))
+            _lib.check(lib.rvb_terrain_create(C.byref(h), _lib.ptr(view), self.G0, self.G1, self.K,
+                                              view.stride(0), view.stride(1), view.stride(2),
+                                              _lib.ptr(tri), self.T, _lib.ptr(ver), self.V,
+                                              self.res, float(shift[0]), float(shift[1]), sem,
+                                              _lib.LAYER_INDEX_ONLY if index_only else 0, _lib.stream_of(idx)))
         self._h = h
         self._lib = lib
 

@@ -24,7 +24,9 @@ def test_header_symbols_exported():
     for n in names:
         assert hasattr(raw, n), "missing export " + n
     assert set(names) == set(_lib.EXPORTS), set(names) ^ set(_lib.EXPORTS)
-    assert lib.rvb_abi_version() == 3
+    for n in ("rvb_terrain_create", "rvb_heightmap_raycast", "rvb_rock_collision"):        # their "2" forms were merged into them
+        assert not hasattr(raw, n + "2"), "removed entry point still exported: " + n + "2"
+    assert lib.rvb_abi_version() == 4
 
 
 def test_argument_validation_without_gpu():
@@ -37,8 +39,23 @@ def test_argument_validation_without_gpu():
     rc = lib.rvb_ackermann(None, 1, None, 1, 4, None, None, None, None, 0, None)
     assert rc == -1
     h = ctypes.c_void_p()
-    rc = lib.rvb_terrain_create(ctypes.byref(h), None, 10, 10, 8, 1, 1, 1, None, 4, None, 4, 0.1, 0.0, 0.0, 0, None)
+    rc = lib.rvb_terrain_create(ctypes.byref(h), None, 10, 10, 8, 1, 1, 1, None, 4, None, 4, 0.1, 0.0, 0.0, 0, 0, None)
     assert rc == -1 and h.value is None
+    rc = lib.rvb_terrain_create(ctypes.byref(h), None, 10, 10, 8, 1, 1, 1, None, 4, None, 4, 0.1, 0.0, 0.0, 0, 2, None)
+    assert rc == -1 and h.value is None and b"rvb_terrain_create: unknown flag" in lib.rvb_last_error()
+    assert lib.rvb_heightmap_raycast(None, None, None, None, None, 4, 1, None, None, None, None, None,
+                                     None, 0, None, 0, 0, None, None, 0, None) == -1
+    assert lib.rvb_cast_rays(None, None, None, 4, None, None, None, None, None) == -1
+    assert lib.rvb_rock_collision(None, None, None, None, None, None, 4, None, None, None, None, None, None) == -1
+    assert lib.rvb_check_collision(None, None, 4, None, None) == -1
+    # policy dispatch: 2 = default, 1 = FFMA2 kernel for every shape; the removed variants 0 and 3 are refused
+    assert lib.rvb_policy_variant(-1) == 2
+    for v in (0, 3):
+        assert lib.rvb_policy_variant(v) == -1 and b"removed" in lib.rvb_last_error()
+        assert lib.rvb_policy_variant(-1) == 2
+    assert lib.rvb_policy_variant(1) == 2
+    assert lib.rvb_policy_variant(2) == 1
+    assert lib.rvb_policy_variant(-1) == 2
     assert lib.rvb_stats_scratch_len(1000) == 4 * 16
     # policy epilogue / hooks (SURVEY 8f-3, 8f-4)
     h = ctypes.c_void_p()

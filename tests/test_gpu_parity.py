@@ -135,7 +135,7 @@ def test_golden_rock_cast_given_reference_rays(R, golden, grock):
     task_col = torch.empty(refw.shape[0], dtype=torch.long, device="cuda")
     lib = R._lib.load()
     w, b = dist.reshape(refw.shape)[:, :24].contiguous(), dist.reshape(refw.shape)[:, 24:].contiguous()
-    R._lib.check(lib.rvb_check_collision(R._lib.ptr(w), R._lib.ptr(b), w.shape[0], R._lib.ptr(task_col), R.SEM_TORCH_CPU, None))
+    R._lib.check(lib.rvb_check_collision(R._lib.ptr(w), R._lib.ptr(b), w.shape[0], R._lib.ptr(task_col), None))
     torch.cuda.synchronize()
     assert torch.equal(task_col.cpu(), golden["ref_rock_collision"])
 
@@ -462,6 +462,26 @@ def test_compact_layer_matches_full_layer(R, O, world20):
     assert rl.bytes() == 4 * rl.G0 * rl.G1 * ((rl.K + 1) // 2 * 2) + 64 * rl.T
 
 
+@pytest.mark.parametrize("index_only", [False, True])
+def test_terrain_create_rejects_out_of_range_ids(R, world20, index_only):
+    """rvb_terrain_create checks the ids on the device: a triangle id T in map_indices or a vertex id V in triangles fails the call
+    with RVB_ERR_INVALID once the build kernels have run; the half-built layer is freed and the next valid layer builds."""
+    w = world20
+    T, V = w.triangles.shape[0], w.vertices.shape[0]
+    bad_index = w.map_indices.clone()
+    bad_index[-1, 3, 5] = T
+    bad_tris = w.triangles.clone()
+    bad_tris[T // 2, 1] = V
+    shift = torch.tensor([0, 0, 0.0])
+    with pytest.raises(RuntimeError, match=r"rvb_terrain_create \(map_indices holds a triangle id outside \[0,T\)\) \[status -1\]"):
+        R.TerrainLayer(bad_index, w.triangles, w.vertices, shift, index_only=index_only)
+    with pytest.raises(RuntimeError, match=r"rvb_terrain_create \(triangles holds a vertex id outside \[0,V\)\) \[status -1\]"):
+        R.TerrainLayer(w.map_indices, bad_tris, w.vertices, shift, index_only=index_only)
+    layer = R.TerrainLayer(w.map_indices, w.triangles, w.vertices, shift, index_only=index_only)
+    assert layer.has_index and layer.bytes() > 0
+    layer.close()
+
+
 @pytest.mark.parametrize("patch,route", [(2.0, "tiles"), (4.6, "layer")])
 def test_degenerate_triangles_take_the_exact_paths(R, patch, route, monkeypatch):
     """A mesh with edge-on triangles (all vertices of a patch moved onto one vertical plane: fp16 determinant 0 for a vertical ray,
@@ -596,7 +616,7 @@ def test_far_hits_and_spread_rays(R, O, world20):
     for variant in (0, 1, 2, 3):
         R._lib.check(lib.rvb_heightmap_raycast(cam.layer.handle, R._lib.ptr(d_pos), R._lib.ptr(d_eul), R._lib.ptr(d_trig),
                                                R._lib.ptr(d_pat), 4096, 2, R._lib.ptr(dist), R._lib.ptr(slot), None, None, None,
-                                               None, 0, None, None, variant, None))
+                                               None, 0, None, 0, 0, None, None, variant, None))
         torch.cuda.synchronize()
         assert_bits_equal(dist, ref2["dist"], "wide pattern dist v%d" % variant)
         assert_bits_equal(slot, ref2["slot"].to(torch.int32), "wide pattern slot v%d" % variant)
