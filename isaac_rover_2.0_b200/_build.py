@@ -10,7 +10,8 @@ SOURCES = ["terrain.cu", "raycast.cu", "raycast_tiled.cu", "raycast_shadow.cu", 
 NVCC_FLAGS = ["-gencode", "arch=compute_100a,code=sm_100a", "-lineinfo", "-O3", "-std=c++17",
               "-fmad=false",                 # bit-exact parity: never contract mul+add
               "--threads", "0",              # one compilation per source file in parallel (74 s -> 12 s); same object code
-              "-Xcompiler", "-fPIC", "-shared"]
+              "-Xcompiler", "-fPIC", "-shared",
+              "-Xlinker", "--no-undefined"]   # a declaration that no source defines fails the link, not the library's load
 
 
 def _nvcc():

@@ -47,14 +47,6 @@ struct RvbJoinGuard {
     }
 };
 
-// Optional packed fp16 observation output of a heightmap ray-cast (rvb_heightmap_raycast2, rvb_step_io.obs_h16):
-// obs16[n * ld + (column - col0)] = fp16(dist / 2) for the columns col_a / col_b name.
-struct RvbObs16 {
-    uint16_t* p;
-    int64_t ld;
-    int col0;
-};
-
 // ---------------------------------------------------------------- terrain handle
 // One pre-resolved record per triangle, 32 B = one L2 sector, two 16-byte loads.
 // halves: a.xyz | b.xyz | c.xyz | n.xyz (n = b x c) | 4 x pad      (ray_casting.py:34-40)

@@ -6,16 +6,6 @@
 // cross-check for the production kernel (raycast_shadow.cu) and its tiled fall-back (raycast_tiled.cu).
 #include "raycast_common.cuh"
 
-int launch_heightmap_tiled(const rvb_terrain* t, const float* pos, const float* euler, const float* trig,
-                           const double* pattern, int64_t P, int64_t N, uint16_t* dist, int32_t* hit_slot,
-                           int32_t* hit_tri, uint16_t* pt, uint16_t* sources, float* obs, int64_t obs_ld,
-                           const int32_t* col_a, const int32_t* col_b, bool per_cell, const RvbObs16* o16, cudaStream_t st);
-int launch_heightmap_shadow(const rvb_terrain* t, const float* pos, const float* euler, const float* trig,
-                           const double* pattern, int64_t P, int64_t N, uint16_t* dist, int32_t* hit_slot,
-                           int32_t* hit_tri, uint16_t* pt, uint16_t* sources, float* obs, int64_t obs_ld,
-                           const int32_t* col_a, const int32_t* col_b, const RaycastKnobs& knobs, const RvbObs16* o16,
-                           cudaStream_t st);
-
 // ------------------------------------------------------------------------------------------------
 // setup: sources (fp64 transform -> fp16), per-env direction, per-ray cell
 // ------------------------------------------------------------------------------------------------
@@ -44,11 +34,7 @@ __global__ void hm_setup_kernel(const float* __restrict__ pos, const float* __re
         o[2] = h_from_double(zo);
     }
     if (blockIdx.x == 0 && threadIdx.x == 0) {
-        // the appended point (0,0,-1) minus the translation (camera.py:179-181,202-207)
-        double xo, yo, zo;
-        body_transform<double>(0.0, 0.0, -1.0, t, tx, ty, tz, xo, yo, zo);
-        H3 dir = {h_from_double(__dsub_rn(xo, tx)), h_from_double(__dsub_rn(yo, ty)), h_from_double(__dsub_rn(zo, tz))};
-        H3 d = neg_normalize(dir);
+        const H3 d = rc::env_dir16(t, tx, ty, tz);
         dneg16[n * 3 + 0] = d.x;
         dneg16[n * 3 + 1] = d.y;
         dneg16[n * 3 + 2] = d.z;
@@ -80,10 +66,8 @@ cast_simple_kernel(const int32_t* __restrict__ index, const TriRec* __restrict__
     const H3 s = {src16[ray * 3], src16[ray * 3 + 1], src16[ray * 3 + 2]};
     const int64_t di = ray / rays_per_dir;
     const H3 d = {dneg16[di * 3], dneg16[di * 3 + 1], dneg16[di * 3 + 2]};
-    int cx = cell_coord(s.x, shift_x, res, inv_res, G0 - 1, sem);
-    int cy = cell_coord(s.y, shift_y, res, inv_res, G0 - 1, sem);     // both axes clamp to size(0)-1 (camera.py:243)
-    cy = min(cy, G1 - 1);
-    const int32_t* row = index + ((int64_t)cx * G1 + cy) * Ks;
+    const int2 cell = rc::ray_cell(s.x, s.y, shift_x, shift_y, res, inv_res, G0, G1, sem);
+    const int32_t* row = index + ((int64_t)cell.x * G1 + cell.y) * Ks;
     uint32_t best = 0xffffffffu;
     unsigned short best_bits = RVB_H_MISS;
     for (int j = lane; j < K; j += 32) {
@@ -151,20 +135,20 @@ extern "C" int rvb_heightmap_raycast(const rvb_terrain* t, const float* pos, con
     RVB_REQUIRE(variant >= 0 && variant <= 3, "rvb_heightmap_raycast: variant must be 0, 1, 2 or 3");
     RVB_REQUIRE(!obs_h16 || variant != 1, "rvb_heightmap_raycast: the per-pair cross-check kernel (variant 1) has no packed output");
     RVB_REQUIRE(variant != 2 || t->index != nullptr, "rvb_heightmap_raycast: variant 2 reads the index the layer released (rvb_terrain_release_index)");
-    const RvbObs16 o16v = {obs_h16, obs_h16_ld, obs_h16_col0};
-    const RvbObs16* o16 = obs_h16 ? &o16v : nullptr;
     RaycastKnobs knobs;
     const int krc = read_raycast_knobs(knobs);
     if (krc != RVB_OK) return krc;
     cudaStream_t st = as_stream(stream);
-    // a layer with more than 2 % of triangles the shadow kernel has no bound for (terrain.cu: n_ill): the tiled kernel is the faster one
-    const bool shadow_ok = knobs.force >= 0 ? knobs.force == 1 : t->n_ill * 50 <= t->T;
-    if (variant == 0 && t->sb_ids != nullptr && shadow_ok)
-        return launch_heightmap_shadow(t, pos, euler, trig, pattern, P, N, dist, hit_slot, hit_tri, pt, sources, obs,
-                                       obs_ld, col_a, col_b, knobs, o16, st);
-    if (variant != 1)
-        return launch_heightmap_tiled(t, pos, euler, trig, pattern, P, N, dist, hit_slot, hit_tri, pt, sources, obs,
-                                      obs_ld, col_a, col_b, variant == 2, o16, st);
+    if (variant != 1) {
+        rc::TiledParams q;
+        const int frc = fill_tiled_params(t, pos, euler, trig, pattern, P, N, dist, hit_slot, hit_tri, pt, sources, obs, obs_ld,
+                                          obs_h16, obs_h16_ld, obs_h16_col0, col_a, col_b, q);
+        if (frc != RVB_OK) return frc;
+        // a layer with more than 2 % of triangles the shadow kernel has no bound for (terrain.cu: n_ill): the tiled kernel is the faster one
+        const bool shadow_ok = knobs.force >= 0 ? knobs.force == 1 : t->n_ill * 50 <= t->T;
+        if (variant == 0 && t->sb_ids != nullptr && shadow_ok) return launch_shadow(q, N, knobs, st);
+        return launch_tiled(q, t->blk_ids != nullptr && variant != 2, N * q.tiles, st);
+    }
     RVB_REQUIRE(t->index != nullptr, "rvb_heightmap_raycast: variant 1 reads the index the layer released (rvb_terrain_release_index)");
     RVB_REQUIRE(N <= 65535, "rvb_heightmap_raycast: variant 1 handles at most 65535 envs per call");
     __half* src16 = (__half*)sources;

@@ -1,5 +1,8 @@
-// Pieces shared by the heightmap ray-cast kernels (raycast_tiled.cu, raycast_shadow.cu).
+// Pieces shared by the heightmap ray-cast kernels (raycast.cu, raycast_tiled.cu, raycast_shadow.cu) and the rock layer's
+// cast (rock.cu), and the host functions of rvb_heightmap_raycast that one of those files calls in another.
 #pragma once
+#include <initializer_list>
+
 #include "common.cuh"
 
 // Tuning knobs of the heightmap ray-cast: parameters of the shipped design that tools/ sweep (DESIGN.md 6, "Tuning knobs").
@@ -14,6 +17,35 @@ struct RaycastKnobs {
     bool dbg;             // RVB_SHADOW_DBG: per-stage counters of each launch on stderr
 };
 int read_raycast_knobs(RaycastKnobs& k);
+
+namespace rc { struct TiledParams; }
+// rvb_heightmap_raycast (raycast.cu) fills one parameter block from its arguments and hands it to a launcher.
+// fill_tiled_params (raycast_tiled.cu): the layer's lists and grid, the call's inputs and outputs, the tiling of the P rays.
+int fill_tiled_params(const rvb_terrain* t, const float* pos, const float* euler, const float* trig, const double* pattern,
+                      int64_t P, int64_t N, uint16_t* dist, int32_t* hit_slot, int32_t* hit_tri, uint16_t* pt,
+                      uint16_t* sources, float* obs, int64_t obs_ld, uint16_t* obs_h16, int64_t obs_h16_ld, int obs_h16_col0,
+                      const int32_t* col_a, const int32_t* col_b, rc::TiledParams& q);
+// launch_tiled (raycast_tiled.cu): q.work_list / q.work_count set: `grid` CTAs loop over the list; otherwise one CTA per
+// (env, tile).  `blocks`: the 3x3-cell block lists instead of the K-contiguous index.
+int launch_tiled(const rc::TiledParams& q, bool blocks, int64_t grid, cudaStream_t st);
+// launch_shadow (raycast_shadow.cu): the shadow kernel over N envs, with the tiled kernel for the envs and tiles it leaves.
+int launch_shadow(rc::TiledParams q, int64_t N, const RaycastKnobs& knobs, cudaStream_t st);
+
+// Raises each kernel's dynamic shared-memory limit to its size, once per (thread, device): the attribute belongs to the
+// current device.  `configured_device` is the caller's thread_local record of the device it was last set on.
+struct SmemLimit {
+    const void* kernel;
+    size_t bytes;
+};
+inline int set_smem_limits(int& configured_device, std::initializer_list<SmemLimit> kernels) {
+    int dev = 0;
+    RVB_CUDA(cudaGetDevice(&dev));
+    if (configured_device == dev) return RVB_OK;
+    for (const SmemLimit& k : kernels)
+        RVB_CUDA(cudaFuncSetAttribute(k.kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)k.bytes));
+    configured_device = dev;
+    return RVB_OK;
+}
 
 namespace rc {
 
@@ -61,16 +93,32 @@ struct TiledParams {
     const int* work_count;
     const int32_t* work_list;
     int work_slices;
-    // shadow kernel: env order (envs with tilted rays first: they are the slow CTAs, so they must not start last) and the
-    // pre-sorted steep envs (cast by the tiled kernel on a second stream, concurrently); both written by hm_classify_kernel
-    const int32_t* order;     // [N] or NULL
-    int presorted;            // steep envs are already on a work list: the shadow kernel just skips them
-    int min_sh;               // bins are 2^sh x 2^sh cells, sh >= min_sh (0 = one cell; tuning knob)
+    // shadow kernel: env order (envs with tilted rays first: they are the slow CTAs, so they must not start last), written by
+    // hm_classify_kernel with the list of steep envs (cast by the tiled kernel on a second stream, concurrently)
+    const int32_t* order;     // [N]
+    int min_sh;              // bins are 2^sh x 2^sh cells, sh >= min_sh (0 = one cell; tuning knob)
     int task_rays;            // shadow kernel: rays per task of stage 3L (1..32: one mask bit each; tuning knob)
     int64_t split_from;       // shadow kernel: order positions >= split_from are cast by two CTAs (half the rays each); -1 = none
     int split_at;             // first ray of the second half
     unsigned long long* dbg;  // optional [24] work counters / cycle counts of the shadow kernel (RVB_SHADOW_DBG=1)
 };
+
+// Cell (cx, cy) of an fp16 source: the x and y look-ups of camera.py:241-253.  Both axes clamp to size(0) - 1 (camera.py:243),
+// then y also to G1 - 1.  The scalars are references so that, inlined, each is read where its axis needs it: with copies made
+// before the call, ptxas schedules hm_tiled_kernel<3> differently (12952 instead of 12960 SASS instructions, nvcc 12.9).
+__device__ __forceinline__ int2 ray_cell(__half x, __half y, const float& shift_x, const float& shift_y, const float& res,
+                                         const float& inv_res, const int& G0, const int& G1, const int& sem) {
+    return make_int2(cell_coord(x, shift_x, res, inv_res, G0 - 1, sem),
+                     min(cell_coord(y, shift_y, res, inv_res, G0 - 1, sem), G1 - 1));
+}
+
+// The env's ray direction d = -normalize(dir) in fp16: dir is the body transform of the appended point (0, 0, -1) minus the
+// translation, cast to fp16 (camera.py:179-181,202-207; ray_casting.py:31).
+__device__ __forceinline__ H3 env_dir16(const Trig& tr, double tx, double ty, double tz) {
+    double xo, yo, zo;
+    body_transform<double>(0.0, 0.0, -1.0, tr, tx, ty, tz, xo, yo, zo);
+    return neg_normalize({h_from_double(__dsub_rn(xo, tx)), h_from_double(__dsub_rn(yo, ty)), h_from_double(__dsub_rn(zo, tz))});
+}
 
 // two candidates of one cell, component-wise packed: .x = candidate j, .y = candidate j+1
 struct Tri2 {
@@ -264,14 +312,13 @@ __device__ __forceinline__ void epilogue(const TiledParams& q, int64_t n, int p0
             double xo, yo, zo;
             body_transform<double>(pp[0], pp[1], pp[2], tr, tx, ty, tz, xo, yo, zo);
             const H3 s = {h_from_double(xo), h_from_double(yo), h_from_double(zo)};
-            const int cx = cell_coord(s.x, q.shift_x, q.res, q.inv_res, q.G0 - 1, q.sem);
-            const int cy = min(cell_coord(s.y, q.shift_y, q.res, q.inv_res, q.G0 - 1, q.sem), q.G1 - 1);
+            const int2 c = ray_cell(s.x, s.y, q.shift_x, q.shift_y, q.res, q.inv_res, q.G0, q.G1, q.sem);
             if (q.index) {
-                key = literal_ray(q.index + ((int64_t)cx * q.G1 + cy) * q.Ks, q.K, q.recs, s, dlit);
+                key = literal_ray(q.index + ((int64_t)c.x * q.G1 + c.y) * q.Ks, q.K, q.recs, s, dlit);
             } else {
-                const uint32_t bi = (uint32_t)(cx / RVB_BLK) * (uint32_t)q.nBy + (uint32_t)(cy / RVB_BLK);
+                const uint32_t bi = (uint32_t)(c.x / RVB_BLK) * (uint32_t)q.nBy + (uint32_t)(c.y / RVB_BLK);
                 const uint32_t o0 = __ldg(q.blk_off + bi), o1 = __ldg(q.blk_off + bi + 1);
-                key = literal_ray_blk(q.blk_ids + o0, q.blk_slots + o0, (int)(o1 - o0), (cx % RVB_BLK) * RVB_BLK + cy % RVB_BLK, q.recs, s, dlit);
+                key = literal_ray_blk(q.blk_ids + o0, q.blk_slots + o0, (int)(o1 - o0), (c.x % RVB_BLK) * RVB_BLK + c.y % RVB_BLK, q.recs, s, dlit);
             }
         }
         const unsigned short kb = key_bits(key);
@@ -286,14 +333,13 @@ __device__ __forceinline__ void epilogue(const TiledParams& q, int64_t n, int p0
             const __half hx = h_from_double(xo), hy = h_from_double(yo), hz = h_from_double(zo);
             if (q.sources) { q.sources[o * 3 + 0] = hx; q.sources[o * 3 + 1] = hy; q.sources[o * 3 + 2] = hz; }
             if (q.hit_tri) {
-                const int cx = cell_coord(hx, q.shift_x, q.res, q.inv_res, q.G0 - 1, q.sem);
-                const int cy = min(cell_coord(hy, q.shift_y, q.res, q.inv_res, q.G0 - 1, q.sem), q.G1 - 1);
+                const int2 c = ray_cell(hx, hy, q.shift_x, q.shift_y, q.res, q.inv_res, q.G0, q.G1, q.sem);
                 if (q.index) {
-                    q.hit_tri[o] = __ldg(q.index + ((int64_t)cx * q.G1 + cy) * q.Ks + slot);
+                    q.hit_tri[o] = __ldg(q.index + ((int64_t)c.x * q.G1 + c.y) * q.Ks + slot);
                 } else {
-                    const uint32_t bi = (uint32_t)(cx / RVB_BLK) * (uint32_t)q.nBy + (uint32_t)(cy / RVB_BLK);
+                    const uint32_t bi = (uint32_t)(c.x / RVB_BLK) * (uint32_t)q.nBy + (uint32_t)(c.y / RVB_BLK);
                     const uint32_t o0 = __ldg(q.blk_off + bi), o1 = __ldg(q.blk_off + bi + 1);
-                    q.hit_tri[o] = tri_of_slot_blk(q.blk_ids + o0, q.blk_slots + o0, (int)(o1 - o0), (cx % RVB_BLK) * RVB_BLK + cy % RVB_BLK, slot);
+                    q.hit_tri[o] = tri_of_slot_blk(q.blk_ids + o0, q.blk_slots + o0, (int)(o1 - o0), (c.x % RVB_BLK) * RVB_BLK + c.y % RVB_BLK, slot);
                 }
             }
             if (q.pt) {

@@ -42,12 +42,6 @@
 #include "raycast_common.cuh"
 #include "shadow_bounds.cuh"
 
-int fill_tiled_params(const rvb_terrain* t, const float* pos, const float* euler, const float* trig, const double* pattern,
-                      int64_t P, int64_t N, uint16_t* dist, int32_t* hit_slot, int32_t* hit_tri, uint16_t* pt,
-                      uint16_t* sources, float* obs, int64_t obs_ld, const int32_t* col_a, const int32_t* col_b,
-                      const RvbObs16* o16, rc::TiledParams& q);
-int launch_tiled(const rc::TiledParams& q, bool blocks, int64_t grid, cudaStream_t st);
-
 namespace {
 
 using namespace rc;
@@ -182,10 +176,7 @@ __global__ void hm_classify_kernel(const TiledParams q, int64_t N, int32_t* __re
     const int64_t n = blockIdx.x * (int64_t)blockDim.x + threadIdx.x;
     if (n >= N) return;
     const Trig tr = make_trig(q.euler, q.trig, n);
-    const double tx = (double)q.pos[n * 3 + 0], ty = (double)q.pos[n * 3 + 1], tz = (double)q.pos[n * 3 + 2];
-    double xo, yo, zo;
-    body_transform<double>(0.0, 0.0, -1.0, tr, tx, ty, tz, xo, yo, zo);
-    const H3 d16 = neg_normalize({h_from_double(__dsub_rn(xo, tx)), h_from_double(__dsub_rn(yo, ty)), h_from_double(__dsub_rn(zo, tz))});
+    const H3 d16 = env_dir16(tr, (double)q.pos[n * 3 + 0], (double)q.pos[n * 3 + 1], (double)q.pos[n * 3 + 2]);
     const bool steep = is_steep(d16, q.cos_steep);
     if (steep) {
         const int at = atomicAdd(counters + 0, q.tiles);
@@ -219,7 +210,7 @@ __global__ void __launch_bounds__(TT, RTC <= RT_SMALL ? 4 : 3) hm_shadow_kernel(
         p0_ = (k & 1) ? q.split_at : 0;
         np_ = (k & 1) ? q.P - q.split_at : q.split_at;
     }
-    const int64_t n = q.order ? (int64_t)__ldg(q.order + opos) : opos;
+    const int64_t n = __ldg(q.order + opos);
     const int32_t work_id = (int32_t)(n * q.tiles + tile);
     const int p0 = p0_;
     const int np = np_;
@@ -254,16 +245,10 @@ __global__ void __launch_bounds__(TT, RTC <= RT_SMALL ? 4 : 3) hm_shadow_kernel(
     }
     const Trig tr = make_trig(q.euler, q.trig, n);
     const double tx = (double)q.pos[n * 3 + 0], ty = (double)q.pos[n * 3 + 1], tz = (double)q.pos[n * 3 + 2];
-    __half2 dx2, dy2, dz2;
-    H3 d16;
-    {
-        double xo, yo, zo;
-        body_transform<double>(0.0, 0.0, -1.0, tr, tx, ty, tz, xo, yo, zo);
-        d16 = neg_normalize({h_from_double(__dsub_rn(xo, tx)), h_from_double(__dsub_rn(yo, ty)), h_from_double(__dsub_rn(zo, tz))});
-        dx2 = __half2half2(d16.x); dy2 = __half2half2(d16.y); dz2 = __half2half2(d16.z);
-    }
+    const H3 d16 = env_dir16(tr, tx, ty, tz);
+    const __half2 dx2 = __half2half2(d16.x), dy2 = __half2half2(d16.y), dz2 = __half2half2(d16.z);
     // rays nearly horizontal in the WORLD (steep env): hm_classify_kernel put this env on the tiled kernel's list already
-    if (q.presorted && is_steep(d16, q.cos_steep)) return;
+    if (is_steep(d16, q.cos_steep)) return;
     __syncthreads();
 
     // ---- phase 1: sources, cells, ranges
@@ -285,12 +270,11 @@ __global__ void __launch_bounds__(TT, RTC <= RT_SMALL ? 4 : 3) hm_shadow_kernel(
             body_transform<double>(px, py, pz, tr, tx, ty, tz, xo, yo, zo);
             const __half hx = h_from_double(xo), hy = h_from_double(yo), hz = h_from_double(zo);
             r_sxy[i] = (uint32_t)h_bits(hx) | ((uint32_t)h_bits(hy) << 16);
-            int cx = cell_coord(hx, q.shift_x, q.res, q.inv_res, q.G0 - 1, q.sem);
-            int cy = min(cell_coord(hy, q.shift_y, q.res, q.inv_res, q.G0 - 1, q.sem), q.G1 - 1);   // camera.py:243
+            const int2 c = ray_cell(hx, hy, q.shift_x, q.shift_y, q.res, q.inv_res, q.G0, q.G1, q.sem);
             // (the 5 spare bits next to p: the cell's y within its superblock, half of the slot-table index of stage 3b)
-            r_sz[i] = (uint32_t)h_bits(hz) | (((uint32_t)p | ((uint32_t)(cy % SBC) << 11)) << 16);
-            r_cell[i] = (cx << 16) | cy;
-            mnx = min(mnx, cx); mxx = max(mxx, cx); mny = min(mny, cy); mxy = max(mxy, cy);
+            r_sz[i] = (uint32_t)h_bits(hz) | (((uint32_t)p | ((uint32_t)(c.y % SBC) << 11)) << 16);
+            r_cell[i] = (c.x << 16) | c.y;
+            mnx = min(mnx, c.x); mxx = max(mxx, c.x); mny = min(mny, c.y); mxy = max(mxy, c.y);
             const float fx = __half2float(hx), fy = __half2float(hy), fz = __half2float(hz);
             lo_x = fminf(lo_x, fx); hi_x = fmaxf(hi_x, fx); lo_y = fminf(lo_y, fy); hi_y = fmaxf(hi_y, fy);
             amax_s = fmaxf(amax_s, fmaxf(fmaxf(fabsf(fx), fabsf(fy)), fabsf(fz)));
@@ -942,17 +926,17 @@ int read_raycast_knobs(RaycastKnobs& k) {
     return RVB_OK;
 }
 
-int launch_heightmap_shadow(const rvb_terrain* t, const float* pos, const float* euler, const float* trig,
-                            const double* pattern, int64_t P, int64_t N, uint16_t* dist, int32_t* hit_slot,
-                            int32_t* hit_tri, uint16_t* pt, uint16_t* sources, float* obs, int64_t obs_ld,
-                            const int32_t* col_a, const int32_t* col_b, const RaycastKnobs& knobs, const RvbObs16* o16,
-                            cudaStream_t st) {
-    RVB_REQUIRE(t->sb_ids != nullptr && t->sb_slot9 != nullptr && t->sb_chunk != nullptr && t->blk_ids != nullptr && t->s1recs != nullptr,
+// The tiled kernel over the (env, tile) items of a work list on the device; each item is cut into 8 slices, one CTA each.
+static int launch_tiled_list(rc::TiledParams q, const int* count, const int32_t* list, int64_t grid, cudaStream_t st) {
+    q.work_count = count;
+    q.work_list = list;
+    q.work_slices = 8;
+    return launch_tiled(q, true, grid, st);
+}
+
+int launch_shadow(rc::TiledParams q, int64_t N, const RaycastKnobs& knobs, cudaStream_t st) {
+    RVB_REQUIRE(q.sb_ids != nullptr && q.sb_slot9 != nullptr && q.sb_chunk != nullptr && q.blk_ids != nullptr && q.s1 != nullptr,
                 "heightmap ray-cast (shadow): layer has no block lists");
-    rc::TiledParams q;
-    int rc_ = fill_tiled_params(t, pos, euler, trig, pattern, P, N, dist, hit_slot, hit_tri, pt, sources, obs, obs_ld, col_a,
-                                col_b, o16, q);
-    if (rc_ != RVB_OK) return rc_;
     RVB_REQUIRE(q.tile_size <= 2048, "heightmap ray-cast (shadow): tile larger than 2048 rays");
     int64_t nblocks = N * q.tiles;
     // the last nsplit envs of the order are cast by two CTAs of half the rays each
@@ -967,55 +951,42 @@ int launch_heightmap_shadow(const rvb_terrain* t, const float* pos, const float*
             nblocks = N + nsplit;
         }
     }
-    // scratch: [0] steep count, [1] tilted envs placed, [2] other envs placed, [3] handed-back count, then the steep list
-    // [nblocks], the hand-back list [nblocks] and the env order [N]
+    // scratch: with RVB_SHADOW_DBG=1 the kernel's 24 counters (8 bytes each) first; then [0] steep count, [1] tilted envs placed,
+    // [2] other envs placed, [3] handed-back count, the steep list [nblocks], the hand-back list [nblocks] and the env order [N]
+    const int64_t ndbg = knobs.dbg ? 2 * 24 : 0;          // in ints
     int* scratch = nullptr;
     RvbJoinGuard guard(st);
-    RVB_CUDA(rvb_scratch_alloc((void**)&scratch, sizeof(int) * (size_t)(4 + 2 * nblocks + N), st));
+    RVB_CUDA(rvb_scratch_alloc((void**)&scratch, sizeof(int) * (size_t)(ndbg + 4 + 2 * nblocks + N), st));
     guard.scratch = scratch;
-    RVB_CUDA(cudaMemsetAsync(scratch, 0, sizeof(int) * 4, st));
-    int32_t* steep_list = scratch + 4;
-    q.fb_count = scratch + 3;
-    q.fb_list = scratch + 4 + nblocks;
-    int32_t* order = scratch + 4 + 2 * nblocks;
-    q.cos_steep = knobs.cos_steep;
+    RVB_CUDA(cudaMemsetAsync(scratch, 0, sizeof(int) * (size_t)(ndbg + 4), st));
+    int* const counts = scratch + ndbg;
+    int32_t* steep_list = counts + 4;
+    q.fb_count = counts + 3;
+    q.fb_list = counts + 4 + nblocks;
+    int32_t* order = counts + 4 + 2 * nblocks;
     q.order = order;
-    q.presorted = 1;
+    q.cos_steep = knobs.cos_steep;
     q.min_sh = knobs.min_sh;
     q.task_rays = knobs.task_rays;
-    RvbSide* side_p = nullptr;
-    RVB_CUDA(rvb_side_stream(1, &side_p));
-    RvbSide& side = *side_p;
     static thread_local int configured_device = -1;
-    int dev = 0;
-    RVB_CUDA(cudaGetDevice(&dev));
-    hm_classify_kernel<<<(unsigned)ceil_div(N, 256), 256, 0, st>>>(q, N, order, scratch, steep_list);
+    const int lrc = set_smem_limits(configured_device, {{(const void*)hm_shadow_kernel<false, RT_MAX>, shadow_smem_bytes(RT_MAX)},
+                                                        {(const void*)hm_shadow_kernel<true, RT_MAX>, shadow_smem_bytes(RT_MAX)},
+                                                        {(const void*)hm_shadow_kernel<false, RT_SMALL>, shadow_smem_bytes(RT_SMALL)},
+                                                        {(const void*)hm_shadow_kernel<true, RT_SMALL>, shadow_smem_bytes(RT_SMALL)}});
+    if (lrc != RVB_OK) return lrc;
+    RvbSide* side = nullptr;
+    RVB_CUDA(rvb_side_stream(1, &side));
+    hm_classify_kernel<<<(unsigned)ceil_div(N, 256), 256, 0, st>>>(q, N, order, counts, steep_list);
     // steep envs: the tiled kernel on the second stream, concurrently with the shadow kernel
     const int64_t tgrid = nblocks < 148 * 3 ? nblocks : 148 * 3;
-    {
-        rc::TiledParams qs = q;
-        qs.work_count = scratch;
-        qs.work_list = steep_list;
-        qs.work_slices = 8;
-        RVB_CUDA(cudaEventRecord(side.fork, st));
-        RVB_CUDA(cudaStreamWaitEvent(side.s, side.fork, 0));
-        const int rcs = launch_tiled(qs, true, tgrid, side.s);
-        if (rcs != RVB_OK) return rcs;
-        RVB_CUDA(cudaEventRecord(side.join, side.s));
-        guard.join = side.join;
-    }
-    if (configured_device != dev) {
-        RVB_CUDA(cudaFuncSetAttribute(hm_shadow_kernel<false, RT_MAX>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)shadow_smem_bytes(RT_MAX)));
-        RVB_CUDA(cudaFuncSetAttribute(hm_shadow_kernel<true, RT_MAX>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)shadow_smem_bytes(RT_MAX)));
-        RVB_CUDA(cudaFuncSetAttribute(hm_shadow_kernel<false, RT_SMALL>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)shadow_smem_bytes(RT_SMALL)));
-        RVB_CUDA(cudaFuncSetAttribute(hm_shadow_kernel<true, RT_SMALL>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)shadow_smem_bytes(RT_SMALL)));
-        configured_device = dev;
-    }
+    RVB_CUDA(cudaEventRecord(side->fork, st));
+    RVB_CUDA(cudaStreamWaitEvent(side->s, side->fork, 0));
+    const int rcs = launch_tiled_list(q, counts, steep_list, tgrid, side->s);
+    if (rcs != RVB_OK) return rcs;
+    RVB_CUDA(cudaEventRecord(side->join, side->s));
+    guard.join = side->join;
     const bool dbg = knobs.dbg;
-    if (dbg) {
-        cudaMalloc(&q.dbg, 24 * sizeof(unsigned long long));
-        cudaMemset(q.dbg, 0, 24 * sizeof(unsigned long long));
-    }
+    if (dbg) q.dbg = reinterpret_cast<unsigned long long*>(scratch);
     const unsigned grid = (unsigned)nblocks;
     if (q.tile_size <= RT_SMALL) {
         if (dbg) hm_shadow_kernel<true, RT_SMALL><<<grid, TT, shadow_smem_bytes(RT_SMALL), st>>>(q);
@@ -1024,14 +995,13 @@ int launch_heightmap_shadow(const rvb_terrain* t, const float* pos, const float*
         if (dbg) hm_shadow_kernel<true, RT_MAX><<<grid, TT, shadow_smem_bytes(RT_MAX), st>>>(q);
         else hm_shadow_kernel<false, RT_MAX><<<grid, TT, shadow_smem_bytes(RT_MAX), st>>>(q);
     }
+    if (cudaGetLastError() != cudaSuccess) return rvb_set_error(RVB_ERR_CUDA, "hm_shadow_kernel", "launch failed");
     if (dbg) {
         unsigned long long h[24];
         int fb = 0;
-        cudaStreamSynchronize(st);
-        cudaMemcpy(h, q.dbg, sizeof(h), cudaMemcpyDeviceToHost);
-        cudaMemcpy(&fb, q.fb_count, sizeof(int), cudaMemcpyDeviceToHost);
-        cudaFree(q.dbg);
-        q.dbg = nullptr;
+        RVB_CUDA(cudaStreamSynchronize(st));
+        RVB_CUDA(cudaMemcpy(h, q.dbg, sizeof(h), cudaMemcpyDeviceToHost));
+        RVB_CUDA(cudaMemcpy(&fb, q.fb_count, sizeof(int), cudaMemcpyDeviceToHost));
         const double ne = (double)(nblocks - fb);
         fprintf(stderr, "[shadow dbg] tiles %lld, handed back %d; per tile: chunks %.1f, stage-1 keeps %.1f, stage-2 triangles %.1f (no bound: %.2f), "
                         "tasks %.1f (emit iterations %.1f), prism loop iterations %.1f, rays tested %.1f, inside the prism %.1f, "
@@ -1043,14 +1013,7 @@ int launch_heightmap_shadow(const rvb_terrain* t, const float* pos, const float*
             fprintf(stderr, "[shadow dbg] phase 3 per warp (cycles): pulling chunks %.0f, draining the queues %.0f, waiting at the final barrier %.0f\n",
                     (double)h[16] / h[19], (double)h[17] / h[19], (double)h[18] / h[19]);
     }
-    rc_ = RVB_OK;
-    if (cudaGetLastError() != cudaSuccess) rc_ = rvb_set_error(RVB_ERR_CUDA, "hm_shadow_kernel", "launch failed");
-    if (rc_ == RVB_OK) {
-        // (env, tile) items the shadow kernel handed back: the tiled kernel loops over the list (usually empty)
-        q.work_count = q.fb_count;
-        q.work_list = q.fb_list;
-        q.work_slices = 8;
-        rc_ = launch_tiled(q, true, tgrid, st);
-    }
-    return rc_;          // guard: st waits for the steep list's kernel, scratch goes back to the pool
+    // (env, tile) items the shadow kernel handed back: the tiled kernel loops over the list (usually empty).  On return the guard
+    // makes st wait for the steep list's kernel and gives the scratch back to the pool.
+    return launch_tiled_list(q, q.fb_count, q.fb_list, tgrid, st);
 }

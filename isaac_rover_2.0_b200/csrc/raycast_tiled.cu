@@ -109,14 +109,8 @@ __device__ __forceinline__ void hm_tiled_body(const TiledParams& q, const int wo
     }
     const Trig tr = make_trig(q.euler, q.trig, n);
     const double tx = (double)q.pos[n * 3 + 0], ty = (double)q.pos[n * 3 + 1], tz = (double)q.pos[n * 3 + 2];
-    __half2 dx2, dy2, dz2;
-    {
-        // the appended point (0,0,-1) minus the translation, normalised and negated (camera.py:179-181,202-207; ray_casting.py:31)
-        double xo, yo, zo;
-        body_transform<double>(0.0, 0.0, -1.0, tr, tx, ty, tz, xo, yo, zo);
-        const H3 d = neg_normalize({h_from_double(__dsub_rn(xo, tx)), h_from_double(__dsub_rn(yo, ty)), h_from_double(__dsub_rn(zo, tz))});
-        dx2 = __half2half2(d.x); dy2 = __half2half2(d.y); dz2 = __half2half2(d.z);
-    }
+    const H3 d = env_dir16(tr, tx, ty, tz);
+    const __half2 dx2 = __half2half2(d.x), dy2 = __half2half2(d.y), dz2 = __half2half2(d.z);
     __syncthreads();
 
     // ---- phase 1: sources + cells of this thread's rays (kept in registers across the sort)
@@ -133,8 +127,8 @@ __device__ __forceinline__ void hm_tiled_body(const TiledParams& q, const int wo
             body_transform<double>(pp[0], pp[1], pp[2], tr, tx, ty, tz, xo, yo, zo);
             const __half hx = h_from_double(xo), hy = h_from_double(yo), hz = h_from_double(zo);
             r_sxy[i] = (uint32_t)h_bits(hx) | ((uint32_t)h_bits(hy) << 16);
-            int cx = cell_coord(hx, q.shift_x, q.res, q.inv_res, q.G0 - 1, q.sem);
-            int cy = min(cell_coord(hy, q.shift_y, q.res, q.inv_res, q.G0 - 1, q.sem), q.G1 - 1);   // camera.py:243
+            const int2 c = ray_cell(hx, hy, q.shift_x, q.shift_y, q.res, q.inv_res, q.G0, q.G1, q.sem);
+            int cx = c.x, cy = c.y;
             uint32_t sub = 0;
             if (B > 1) {
                 const int bx = cx / B, by = cy / B;
@@ -363,22 +357,10 @@ size_t tiled_smem_bytes(int RT) {
 
 }  // namespace
 
-static int configure_tiled() {
-    static thread_local int configured_device = -1;
-    int dev = 0;
-    RVB_CUDA(cudaGetDevice(&dev));
-    if (configured_device != dev) {
-        RVB_CUDA(cudaFuncSetAttribute(hm_tiled_kernel<1>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)tiled_smem_bytes(RT_MAX)));
-        RVB_CUDA(cudaFuncSetAttribute(hm_tiled_kernel<RVB_BLK>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)tiled_smem_bytes(RT_MAX)));
-        configured_device = dev;
-    }
-    return RVB_OK;
-}
-
 int fill_tiled_params(const rvb_terrain* t, const float* pos, const float* euler, const float* trig, const double* pattern,
                       int64_t P, int64_t N, uint16_t* dist, int32_t* hit_slot, int32_t* hit_tri, uint16_t* pt,
-                      uint16_t* sources, float* obs, int64_t obs_ld, const int32_t* col_a, const int32_t* col_b,
-                      const RvbObs16* o16, rc::TiledParams& q) {
+                      uint16_t* sources, float* obs, int64_t obs_ld, uint16_t* obs_h16, int64_t obs_h16_ld, int obs_h16_col0,
+                      const int32_t* col_a, const int32_t* col_b, rc::TiledParams& q) {
     RVB_REQUIRE(t->G0 <= 32767 && t->G1 <= 65535, "heightmap ray-cast: grid larger than 32767 x 65535 cells");
     RVB_REQUIRE(t->K <= 16383, "heightmap ray-cast: K > 16383");
     RVB_REQUIRE(t->G0 * t->G1 < ((int64_t)1 << 32), "heightmap ray-cast: more than 2^32 cells");
@@ -394,31 +376,21 @@ int fill_tiled_params(const rvb_terrain* t, const float* pos, const float* euler
     q.tile_size = (int)ceil_div(P, q.tiles);
     q.dist = (__half*)dist; q.hit_slot = hit_slot; q.hit_tri = hit_tri; q.pt = (__half*)pt; q.sources = (__half*)sources;
     q.obs = obs; q.obs_ld = obs_ld; q.col_a = col_a; q.col_b = col_b;
-    if (o16 && o16->p) {
-        q.obs16 = (__half*)o16->p; q.obs16_ld = o16->ld; q.obs16_col0 = o16->col0;
+    if (obs_h16) {
+        q.obs16 = (__half*)obs_h16; q.obs16_ld = obs_h16_ld; q.obs16_col0 = obs_h16_col0;
     }
     RVB_REQUIRE(N * q.tiles < ((int64_t)1 << 31), "heightmap ray-cast: too many (env, tile) blocks for one launch");
     return RVB_OK;
 }
 
-// q.work_list / q.work_count set: `grid` CTAs loop over the list; otherwise one CTA per (env, tile).
 int launch_tiled(const rc::TiledParams& q, bool blocks, int64_t grid, cudaStream_t st) {
-    const int rc_ = configure_tiled();
+    static thread_local int configured_device = -1;
+    const int rc_ = set_smem_limits(configured_device, {{(const void*)hm_tiled_kernel<1>, tiled_smem_bytes(RT_MAX)},
+                                                        {(const void*)hm_tiled_kernel<RVB_BLK>, tiled_smem_bytes(RT_MAX)}});
     if (rc_ != RVB_OK) return rc_;
     const size_t smem = tiled_smem_bytes(q.tile_size);
     if (blocks) hm_tiled_kernel<RVB_BLK><<<(unsigned)grid, TT, smem, st>>>(q);
     else hm_tiled_kernel<1><<<(unsigned)grid, TT, smem, st>>>(q);
     RVB_LAUNCH_CHECK();
     return RVB_OK;
-}
-
-int launch_heightmap_tiled(const rvb_terrain* t, const float* pos, const float* euler, const float* trig,
-                           const double* pattern, int64_t P, int64_t N, uint16_t* dist, int32_t* hit_slot,
-                           int32_t* hit_tri, uint16_t* pt, uint16_t* sources, float* obs, int64_t obs_ld,
-                           const int32_t* col_a, const int32_t* col_b, bool per_cell, const RvbObs16* o16, cudaStream_t st) {
-    rc::TiledParams q;
-    const int rc_ = fill_tiled_params(t, pos, euler, trig, pattern, P, N, dist, hit_slot, hit_tri, pt, sources, obs, obs_ld,
-                                      col_a, col_b, o16, q);
-    if (rc_ != RVB_OK) return rc_;
-    return launch_tiled(q, t->blk_ids != nullptr && !per_cell, N * q.tiles, st);
 }

@@ -30,13 +30,6 @@ __global__ void step_pre_kernel(rvb_step_io io, int64_t N, int H, int sem) {
                     io.obs + n * io.obs_ld, io.heading + n);
 }
 
-int launch_reward_reset(const rvb_reward_params* p, const float* pos, const float* target, const float* heading,
-                        const float* rover_rot, const float* lin, const float* lin_prev, const float* ang,
-                        const float* ang_prev, int64_t hs, const float* joints, const int64_t* progress,
-                        const int64_t* rock_collision, int64_t N, float* rew, int64_t* reset, float* ex_pos_reward,
-                        int64_t* ex_collision, float* ex_uprightness, float* ex_heading, float* ex_motion,
-                        float* ex_goal_angle, double* stats, double* stats_scratch, cudaStream_t st);
-
 #include <vector>
 
 namespace {

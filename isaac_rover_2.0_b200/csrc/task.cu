@@ -199,7 +199,6 @@ __global__ void stats_final_kernel(const double* __restrict__ partial, int64_t n
     }
 }
 
-// hs: element stride between consecutive envs in lin / lin_prev / ang / ang_prev (1 for packed columns, H for [N,H] histories)
 int launch_reward_reset(const rvb_reward_params* p, const float* pos, const float* target, const float* heading,
                         const float* rover_rot, const float* lin, const float* lin_prev, const float* ang,
                         const float* ang_prev, int64_t hs, const float* joints, const int64_t* progress,

@@ -4,6 +4,15 @@
 
 #include "common.cuh"
 
+// calculate_metrics + is_done with the episode statistics (task.cu; rvb_reward_reset and the end of rvb_env_step).
+// hs: element stride between consecutive envs in lin / lin_prev / ang / ang_prev (1 for packed columns, H for [N,H] histories)
+int launch_reward_reset(const rvb_reward_params* p, const float* pos, const float* target, const float* heading,
+                        const float* rover_rot, const float* lin, const float* lin_prev, const float* ang,
+                        const float* ang_prev, int64_t hs, const float* joints, const int64_t* progress,
+                        const int64_t* rock_collision, int64_t N, float* rew, int64_t* reset, float* ex_pos_reward,
+                        int64_t* ex_collision, float* ex_uprightness, float* ex_heading, float* ex_motion,
+                        float* ex_goal_angle, double* stats, double* stats_scratch, cudaStream_t st);
+
 #define PI_F32 3.1415927410125732f   // tensor_quat_to_euler.py:4
 
 using F = Ops<float>;
