@@ -10,10 +10,15 @@
 // ---------------------------------------------------------------- errors (thread-local, never thrown)
 int rvb_set_error(int code, const char* what, const char* detail);
 
+// A failed call also sets the runtime's last error (a failed cudaMalloc does).  Once reported it is cleared: otherwise the next
+// launch check -- this library's or the caller's own -- would report it again.  A device fault stays: it is sticky.
 #define RVB_CUDA(expr)                                                                   \
     do {                                                                                 \
         cudaError_t e_ = (expr);                                                         \
-        if (e_ != cudaSuccess) return rvb_set_error(RVB_ERR_CUDA, #expr, cudaGetErrorString(e_)); \
+        if (e_ != cudaSuccess) {                                                         \
+            cudaGetLastError();                                                          \
+            return rvb_set_error(RVB_ERR_CUDA, #expr, cudaGetErrorString(e_));           \
+        }                                                                                \
     } while (0)
 #define RVB_REQUIRE(cond, msg)                                                           \
     do {                                                                                 \
@@ -34,16 +39,38 @@ struct RvbSide {
 };
 cudaError_t rvb_side_stream(int slot, RvbSide** out);
 
-// Runs on EVERY exit path of a launcher that forked work onto a side stream and / or holds stream-ordered scratch: the caller's
-// stream waits for the side stream's join event (once it has been recorded) and the scratch goes back to the pool.
+// Runs on EVERY exit path of a launcher that forked work onto a side stream: the caller's stream waits for the side stream's join
+// event (once it has been recorded).
 struct RvbJoinGuard {
     cudaStream_t st;
     cudaEvent_t join = nullptr;      // set after cudaEventRecord(join, side)
-    void* scratch = nullptr;
     explicit RvbJoinGuard(cudaStream_t s) : st(s) {}
     ~RvbJoinGuard() {
         if (join) cudaStreamWaitEvent(st, join, 0);
-        if (scratch) cudaFreeAsync(scratch, st);
+    }
+};
+
+// A temporary device array of n T, freed on EVERY exit path of its scope.  alloc_pool: stream-ordered scratch from the library's
+// pool, given back on its stream.  alloc: a plain cudaMalloc buffer, for the layer build's temporaries -- the pool keeps what it
+// is given, so gigabytes of sort keys would stay reserved for the life of the process.
+template <typename T>
+struct RvbTemp {
+    T* p = nullptr;
+    cudaStream_t st = nullptr;
+    bool pooled = false;
+    RvbTemp() = default;
+    RvbTemp(const RvbTemp&) = delete;
+    RvbTemp& operator=(const RvbTemp&) = delete;
+    cudaError_t alloc(size_t n) { return cudaMalloc((void**)&p, sizeof(T) * n); }
+    cudaError_t alloc_pool(size_t n, cudaStream_t s) {
+        pooled = true;
+        st = s;
+        return rvb_scratch_alloc((void**)&p, sizeof(T) * n, s);
+    }
+    ~RvbTemp() {
+        if (!p) return;
+        if (pooled) cudaFreeAsync(p, st);
+        else cudaFree(p);
     }
 };
 

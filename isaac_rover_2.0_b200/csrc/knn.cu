@@ -190,55 +190,46 @@ extern "C" int rvb_build_knn_index(const int32_t* triangles, int64_t T, const ui
     RVB_REQUIRE(G0 > 0 && G1 > 0 && G0 * G1 < ((int64_t)1 << 31), "rvb_build_knn_index: bad grid");
     RVB_REQUIRE(K > 0 && K <= 1024 && K <= T, "rvb_build_knn_index: need 0 < K <= min(T, 1024)");
     cudaStream_t st = as_stream(stream);
-    __half2* cen = nullptr;
-    unsigned* bbox = nullptr;
-    int *bad = nullptr, *counts = nullptr, *offsets = nullptr, *items = nullptr;
-    void* tmp = nullptr;
-    int rc = RVB_OK;
-    auto fail = [&](const char* what, cudaError_t e) { rc = rvb_set_error(RVB_ERR_CUDA, what, cudaGetErrorString(e)); };
-    cudaError_t e;
-    do {
-        if ((e = rvb_scratch_alloc((void**)&cen, sizeof(__half2) * T, st)) != cudaSuccess) { fail("alloc centroids", e); break; }
-        if ((e = rvb_scratch_alloc((void**)&bbox, sizeof(unsigned) * 4 + sizeof(int), st)) != cudaSuccess) { fail("alloc bbox", e); break; }
-        bad = reinterpret_cast<int*>(bbox + 4);
-        const unsigned init[5] = {0xffffffffu, 0u, 0xffffffffu, 0u, 0u};
-        cudaMemcpyAsync(bbox, init, sizeof(init), cudaMemcpyHostToDevice, st);
-        centroid_kernel<<<(unsigned)ceil_div(T, 256), 256, 0, st>>>(triangles, T, (const __half*)vertices, V, cen, bbox, bad);
-        unsigned hb[5];
-        if ((e = cudaMemcpyAsync(hb, bbox, sizeof(hb), cudaMemcpyDeviceToHost, st)) != cudaSuccess) { fail("bbox copy", e); break; }
-        if ((e = cudaStreamSynchronize(st)) != cudaSuccess) { fail("centroid_kernel", e); break; }
-        if (hb[4]) { rc = rvb_set_error(RVB_ERR_INVALID, "rvb_build_knn_index", "triangles holds a vertex id outside [0,V)"); break; }
-        const float x0 = dec_f(hb[0]), x1 = dec_f(hb[1]), y0 = dec_f(hb[2]), y1 = dec_f(hb[3]);
-        const float w = fmaxf(x1 - x0, 1e-3f), h = fmaxf(y1 - y0, 1e-3f);
-        // ~12 triangles per bucket on average, at most ~4M buckets
-        float b = sqrtf(12.0f * w * h / (float)T);
-        b = fmaxf(b, fmaxf(w, h) / 2000.0f);
-        BucketGrid g;
-        g.x0 = x0; g.y0 = y0; g.b = b; g.inv_b = 1.0f / b;
-        g.nx = (int)floorf(w / b) + 1; g.ny = (int)floorf(h / b) + 1;
-        const int64_t NB = (int64_t)g.nx * g.ny;
-        if ((e = rvb_scratch_alloc((void**)&counts, sizeof(int) * (NB + 1) * 2, st)) != cudaSuccess) { fail("alloc buckets", e); break; }
-        offsets = counts + NB + 1;
-        if ((e = rvb_scratch_alloc((void**)&items, sizeof(int) * T, st)) != cudaSuccess) { fail("alloc items", e); break; }
-        cudaMemsetAsync(counts, 0, sizeof(int) * (NB + 1), st);
-        bucket_count_kernel<<<(unsigned)ceil_div(T, 256), 256, 0, st>>>(cen, T, g, counts);
-        size_t tmp_bytes = 0;
-        cub::DeviceScan::ExclusiveSum(nullptr, tmp_bytes, counts, offsets, (int)(NB + 1), st);
-        if ((e = rvb_scratch_alloc((void**)&tmp, tmp_bytes, st)) != cudaSuccess) { fail("alloc scan", e); break; }
-        cub::DeviceScan::ExclusiveSum(tmp, tmp_bytes, counts, offsets, (int)(NB + 1), st);
-        cudaMemsetAsync(counts, 0, sizeof(int) * (NB + 1), st);
-        bucket_fill_kernel<<<(unsigned)ceil_div(T, 256), 256, 0, st>>>(cen, T, g, offsets, counts, items);
-        // initial window radius: a disc holding K triangles at average density, in buckets
-        const float dens = (float)T / (w * h);
-        const int r0 = (int)ceilf(sqrtf((float)K / (3.14159f * dens)) / b) + 1;
-        knn_cells_kernel<<<(unsigned)(G0 * G1), KNN_THREADS, 0, st>>>(cen, g, offsets, items, (const __half*)cell_x,
-                                                                     (const __half*)cell_y, (int)G0, (int)G1, (int)K, r0, out);
-        if ((e = cudaGetLastError()) != cudaSuccess) { fail("knn_cells_kernel", e); break; }
-    } while (0);
-    if (tmp) cudaFreeAsync(tmp, st);
-    if (items) cudaFreeAsync(items, st);
-    if (counts) cudaFreeAsync(counts, st);
-    if (bbox) cudaFreeAsync(bbox, st);
-    if (cen) cudaFreeAsync(cen, st);
-    return rc;
+    RvbTemp<__half2> cen;
+    RvbTemp<unsigned> bbox;          // 4 encoded bounds, then the bad-vertex flag
+    RvbTemp<int> counts, items;
+    RvbTemp<unsigned char> tmp;
+    RVB_CUDA(cen.alloc_pool(T, st));
+    RVB_CUDA(bbox.alloc_pool(5, st));
+    int* bad = reinterpret_cast<int*>(bbox.p + 4);
+    const unsigned init[5] = {0xffffffffu, 0u, 0xffffffffu, 0u, 0u};
+    RVB_CUDA(cudaMemcpyAsync(bbox.p, init, sizeof(init), cudaMemcpyHostToDevice, st));
+    centroid_kernel<<<(unsigned)ceil_div(T, 256), 256, 0, st>>>(triangles, T, (const __half*)vertices, V, cen.p, bbox.p, bad);
+    RVB_LAUNCH_CHECK();
+    unsigned hb[5];
+    RVB_CUDA(cudaMemcpyAsync(hb, bbox.p, sizeof(hb), cudaMemcpyDeviceToHost, st));
+    RVB_CUDA(cudaStreamSynchronize(st));
+    if (hb[4]) return rvb_set_error(RVB_ERR_INVALID, "rvb_build_knn_index", "triangles holds a vertex id outside [0,V)");
+    const float x0 = dec_f(hb[0]), x1 = dec_f(hb[1]), y0 = dec_f(hb[2]), y1 = dec_f(hb[3]);
+    const float w = fmaxf(x1 - x0, 1e-3f), h = fmaxf(y1 - y0, 1e-3f);
+    // ~12 triangles per bucket on average, at most ~4M buckets
+    float b = sqrtf(12.0f * w * h / (float)T);
+    b = fmaxf(b, fmaxf(w, h) / 2000.0f);
+    BucketGrid g;
+    g.x0 = x0; g.y0 = y0; g.b = b; g.inv_b = 1.0f / b;
+    g.nx = (int)floorf(w / b) + 1; g.ny = (int)floorf(h / b) + 1;
+    const int64_t NB = (int64_t)g.nx * g.ny;
+    RVB_CUDA(counts.alloc_pool((NB + 1) * 2, st));
+    int* offsets = counts.p + NB + 1;
+    RVB_CUDA(items.alloc_pool(T, st));
+    RVB_CUDA(cudaMemsetAsync(counts.p, 0, sizeof(int) * (NB + 1), st));
+    bucket_count_kernel<<<(unsigned)ceil_div(T, 256), 256, 0, st>>>(cen.p, T, g, counts.p);
+    size_t tmp_bytes = 0;
+    RVB_CUDA(cub::DeviceScan::ExclusiveSum(nullptr, tmp_bytes, counts.p, offsets, (int)(NB + 1), st));
+    RVB_CUDA(tmp.alloc_pool(tmp_bytes, st));
+    RVB_CUDA(cub::DeviceScan::ExclusiveSum(tmp.p, tmp_bytes, counts.p, offsets, (int)(NB + 1), st));
+    RVB_CUDA(cudaMemsetAsync(counts.p, 0, sizeof(int) * (NB + 1), st));
+    bucket_fill_kernel<<<(unsigned)ceil_div(T, 256), 256, 0, st>>>(cen.p, T, g, offsets, counts.p, items.p);
+    // initial window radius: a disc holding K triangles at average density, in buckets
+    const float dens = (float)T / (w * h);
+    const int r0 = (int)ceilf(sqrtf((float)K / (3.14159f * dens)) / b) + 1;
+    knn_cells_kernel<<<(unsigned)(G0 * G1), KNN_THREADS, 0, st>>>(cen.p, g, offsets, items.p, (const __half*)cell_x,
+                                                                 (const __half*)cell_y, (int)G0, (int)G1, (int)K, r0, out);
+    RVB_LAUNCH_CHECK();
+    return RVB_OK;
 }

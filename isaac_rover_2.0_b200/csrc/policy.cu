@@ -20,6 +20,7 @@
 // (Wt[k][OUTP]) that every CTA streams from L2 through a 16 KB staging buffer.  Thread (mg = warp, ng = lane) owns
 // 4 envs x CN columns {ng + 32 j}: per k one broadcast 128-bit activation load + CN conflict-free weight loads feed
 // 4 CN FMAs.  99 KB shared memory -> 2 CTAs per SM.
+#include <memory>
 #include <new>
 #include <stdlib.h>
 
@@ -826,7 +827,8 @@ extern "C" int rvb_policy_create(rvb_policy** out, int32_t n_proprio, int32_t n_
     int cur_dev = -1;                  // like every other entry point: the caller's current device, never changed here
     RVB_CUDA(cudaGetDevice(&cur_dev));
     RVB_REQUIRE(device == cur_dev, "rvb_policy_create: `device` is not the calling thread's current CUDA device");
-    rvb_policy* P = new (std::nothrow) rvb_policy();
+    // value-initialised (storage null), so on a failure rvb_policy_destroy frees exactly what was built
+    std::unique_ptr<rvb_policy, int (*)(rvb_policy*)> P(new (std::nothrow) rvb_policy(), rvb_policy_destroy);
     if (!P) return rvb_set_error(RVB_ERR_NOMEM, "rvb_policy_create", "host allocation failed");
     P->n_proprio = n_proprio; P->n_sparse = n_sparse; P->n_dense = n_dense; P->n_head = head->out_features;
     P->act = activation; P->head_tanh = head_tanh ? 1 : 0; P->device = device;
@@ -846,8 +848,11 @@ extern "C" int rvb_policy_create(rvb_policy** out, int32_t n_proprio, int32_t n_
     total = (total + 63) / 64 * 64;
     const int64_t img_at = total;
     total += img_s + img_d + TT_FLOATS;
-    cudaError_t e = cudaMalloc((void**)&P->storage, sizeof(float) * total);
-    if (e != cudaSuccess) { delete P; return rvb_set_error(RVB_ERR_NOMEM, "rvb_policy_create: cudaMalloc", cudaGetErrorString(e)); }
+    const cudaError_t e = cudaMalloc((void**)&P->storage, sizeof(float) * total);
+    if (e != cudaSuccess) {
+        cudaGetLastError();          // reported here, not again by the next launch check (common.cuh: RVB_CUDA)
+        return rvb_set_error(RVB_ERR_NOMEM, "rvb_policy_create: cudaMalloc", cudaGetErrorString(e));
+    }
     P->storage_floats = total;
     cudaStream_t st = as_stream(stream);
     P->dev = reinterpret_cast<const PolicyDev*>(P->storage);
@@ -879,22 +884,17 @@ extern "C" int rvb_policy_create(rvb_policy** out, int32_t n_proprio, int32_t n_
         for (int i = 0; i < 8; ++i) block(mlp[1], 0, PL_M2, i, (int64_t)TT_OFF_M2 + (int64_t)i * 2 * PL_M2 * TC_KC);
         for (int i = 0; i < 5; ++i) block(mlp[2], 0, 128, i, (int64_t)TT_OFF_M3 + (int64_t)i * 2 * 128 * TC_KC);
     }
-    e = cudaMemcpyAsync(P->head_w, head->weight, sizeof(float) * P->n_head * PL_M3, cudaMemcpyDeviceToDevice, st);
-    if (e == cudaSuccess) e = cudaMemcpyAsync(P->head_b, head->bias, sizeof(float) * P->n_head, cudaMemcpyDeviceToDevice, st);
-    if (e == cudaSuccess)       // the descriptor the kernel reads (P outlives the copy: the stream is synchronised below)
-        e = cudaMemcpyAsync(P->storage, static_cast<const PolicyDev*>(P), sizeof(PolicyDev), cudaMemcpyHostToDevice, st);
-    if (e == cudaSuccess) e = cudaGetLastError();
-    if (e == cudaSuccess) e = cudaFuncSetAttribute(policy_forward_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, PL_SMEM_BYTES);
-    if (e == cudaSuccess) e = cudaFuncSetAttribute(policy_l1_tc_kernel<1>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)tc_smem_bytes(1));
-    if (e == cudaSuccess) e = cudaFuncSetAttribute(policy_l1_tc_kernel<2>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)tc_smem_bytes(2));
-    if (e == cudaSuccess) e = cudaFuncSetAttribute(policy_tail_tc_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)tt_smem_bytes());
-    if (e == cudaSuccess) e = cudaStreamSynchronize(st);   // the caller may free its weight tensors on return
-    if (e != cudaSuccess) {
-        cudaFree(P->storage);
-        delete P;
-        return rvb_set_error(RVB_ERR_CUDA, "rvb_policy_create", cudaGetErrorString(e));
-    }
-    *out = P;
+    RVB_CUDA(cudaMemcpyAsync(P->head_w, head->weight, sizeof(float) * P->n_head * PL_M3, cudaMemcpyDeviceToDevice, st));
+    RVB_CUDA(cudaMemcpyAsync(P->head_b, head->bias, sizeof(float) * P->n_head, cudaMemcpyDeviceToDevice, st));
+    // the descriptor the kernel reads (P outlives the copy: the stream is synchronised below)
+    RVB_CUDA(cudaMemcpyAsync(P->storage, static_cast<const PolicyDev*>(P.get()), sizeof(PolicyDev), cudaMemcpyHostToDevice, st));
+    RVB_LAUNCH_CHECK();
+    RVB_CUDA(cudaFuncSetAttribute(policy_forward_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, PL_SMEM_BYTES));
+    RVB_CUDA(cudaFuncSetAttribute(policy_l1_tc_kernel<1>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)tc_smem_bytes(1)));
+    RVB_CUDA(cudaFuncSetAttribute(policy_l1_tc_kernel<2>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)tc_smem_bytes(2)));
+    RVB_CUDA(cudaFuncSetAttribute(policy_tail_tc_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)tt_smem_bytes()));
+    RVB_CUDA(cudaStreamSynchronize(st));   // the caller may free its weight tensors on return
+    *out = P.release();
     return RVB_OK;
 }
 
@@ -952,27 +952,23 @@ static cudaError_t launch_tail_tc(dim3 grid, cudaStream_t st, const PolicyDev* a
 }
 
 // One network (B == nullptr) or two on the same observations (grid.y = network; the pair's first layers share the observation tiles).
-static int policy_launch(const char* name, const rvb_policy* A, const rvb_policy* B, const float* obs, int64_t obs_ld, int64_t N,
+static int policy_launch(const rvb_policy* A, const rvb_policy* B, const float* obs, int64_t obs_ld, int64_t N,
                          float* out_a, int64_t out_a_ld, float* out_b, int64_t out_b_ld, cudaStream_t st) {
     RVB_REQUIRE(N <= (int64_t)PL_TM * 0x7fffffff, "rvb_policy_forward: too many envs");
     const int nets = B ? 2 : 1;
     const PolicyDev* db = B ? B->dev : nullptr;
-    float* h1 = nullptr;
-    cudaError_t le = cudaSuccess;
+    RvbTemp<float> h1;
     if (tc_usable(A, obs, obs_ld)) {
-        RVB_CUDA(rvb_scratch_alloc((void**)&h1, sizeof(float) * (size_t)N * nets * 2 * PL_E1, st));
+        RVB_CUDA(h1.alloc_pool((size_t)N * nets * 2 * PL_E1, st));
         const dim3 grid((unsigned)ceil_div(N, TC_M), 2);
-        if (B) policy_l1_tc_kernel<2><<<grid, TC_THREADS, tc_smem_bytes(2), st>>>(A->dev, db, obs, obs_ld, N, h1);
-        else policy_l1_tc_kernel<1><<<grid, TC_THREADS, tc_smem_bytes(1), st>>>(A->dev, db, obs, obs_ld, N, h1);
-        le = launch_tail_tc(dim3((unsigned)ceil_div(N, TC_M), nets), st, A->dev, db, obs, obs_ld, N, h1, nets, out_a, out_a_ld, out_b, out_b_ld);
+        if (B) policy_l1_tc_kernel<2><<<grid, TC_THREADS, tc_smem_bytes(2), st>>>(A->dev, db, obs, obs_ld, N, h1.p);
+        else policy_l1_tc_kernel<1><<<grid, TC_THREADS, tc_smem_bytes(1), st>>>(A->dev, db, obs, obs_ld, N, h1.p);
+        RVB_CUDA(launch_tail_tc(dim3((unsigned)ceil_div(N, TC_M), nets), st, A->dev, db, obs, obs_ld, N, h1.p, nets, out_a, out_a_ld, out_b, out_b_ld));
     } else {
         policy_forward_kernel<<<dim3((unsigned)ceil_div(N, PL_TM), nets), PL_THREADS, PL_SMEM_BYTES, st>>>(A->dev, db, obs, obs_ld, N, out_a,
                                                                                                        out_a_ld, out_b, out_b_ld);
     }
-    const cudaError_t last = cudaGetLastError();          // also clears the error state of a failed launch
-    if (le == cudaSuccess) le = last;
-    if (h1) cudaFreeAsync(h1, st);
-    if (le != cudaSuccess) return rvb_set_error(RVB_ERR_CUDA, name, cudaGetErrorString(le));
+    RVB_LAUNCH_CHECK();
     return RVB_OK;
 }
 
@@ -982,7 +978,7 @@ extern "C" int rvb_policy_forward(const rvb_policy* P, const float* obs, int64_t
     if (N <= 0) return RVB_OK;
     int rc;
     if ((rc = check_forward(P, obs, obs_ld, out, out_ld))) return rc;
-    return policy_launch("rvb_policy_forward", P, nullptr, obs, obs_ld, N, out, out_ld, nullptr, 0, as_stream(stream));
+    return policy_launch(P, nullptr, obs, obs_ld, N, out, out_ld, nullptr, 0, as_stream(stream));
 }
 
 extern "C" int rvb_policy_forward_pair(const rvb_policy* A, const rvb_policy* B, const float* obs, int64_t obs_ld, int64_t N,
@@ -996,5 +992,5 @@ extern "C" int rvb_policy_forward_pair(const rvb_policy* A, const rvb_policy* B,
     RVB_REQUIRE(A->n_proprio == B->n_proprio && A->n_sparse == B->n_sparse && A->n_dense == B->n_dense,
                 "rvb_policy_forward_pair: the two networks read different observation splits");
     RVB_REQUIRE(A->act == B->act, "rvb_policy_forward_pair: the two networks use different activations");
-    return policy_launch("rvb_policy_forward_pair", A, B, obs, obs_ld, N, out_a, out_a_ld, out_b, out_b_ld, as_stream(stream));
+    return policy_launch(A, B, obs, obs_ld, N, out_a, out_a_ld, out_b, out_b_ld, as_stream(stream));
 }

@@ -152,19 +152,14 @@ extern "C" int rvb_heightmap_raycast(const rvb_terrain* t, const float* pos, con
     RVB_REQUIRE(t->index != nullptr, "rvb_heightmap_raycast: variant 1 reads the index the layer released (rvb_terrain_release_index)");
     RVB_REQUIRE(N <= 65535, "rvb_heightmap_raycast: variant 1 handles at most 65535 envs per call");
     __half* src16 = (__half*)sources;
-    __half* scratch = nullptr;
-    const size_t src_bytes = sizeof(__half) * 3 * (size_t)N * P, d_bytes = sizeof(__half) * 3 * (size_t)N;
-    RVB_CUDA(rvb_scratch_alloc((void**)&scratch, d_bytes + (sources ? 0 : src_bytes), st));
-    __half* dneg = scratch;
-    if (!sources) src16 = scratch + 3 * N;
+    RvbTemp<__half> scratch;          // the N directions, then (without `sources`) the N * P sources
+    RVB_CUDA(scratch.alloc_pool(3 * (size_t)N + (sources ? 0 : 3 * (size_t)N * P), st));
+    __half* dneg = scratch.p;
+    if (!sources) src16 = scratch.p + 3 * N;
     dim3 grid((unsigned)ceil_div(P, 256), (unsigned)N);
     hm_setup_kernel<<<grid, 256, 0, st>>>(pos, euler, trig, pattern, (int)P, src16, dneg);
-    int rc = RVB_OK;
-    if (cudaGetLastError() != cudaSuccess) rc = rvb_set_error(RVB_ERR_CUDA, "hm_setup_kernel", "launch failed");
-    if (rc == RVB_OK)
-        rc = launch_cast_simple(t, src16, dneg, N * P, P, dist, hit_slot, hit_tri, pt, obs, obs_ld, col_a, col_b, st);
-    cudaFreeAsync(scratch, st);
-    return rc;
+    RVB_LAUNCH_CHECK();
+    return launch_cast_simple(t, src16, dneg, N * P, P, dist, hit_slot, hit_tri, pt, obs, obs_ld, col_a, col_b, st);
 }
 
 extern "C" int rvb_cast_rays(const rvb_terrain* t, const uint16_t* sources, const uint16_t* directions, int64_t R,
@@ -174,13 +169,10 @@ extern "C" int rvb_cast_rays(const rvb_terrain* t, const uint16_t* sources, cons
     RVB_REQUIRE(t && sources && directions && dist, "rvb_cast_rays: null pointer");
     RVB_REQUIRE(t->index != nullptr, "rvb_cast_rays: the layer released its index (rvb_terrain_release_index)");
     cudaStream_t st = as_stream(stream);
-    __half* dneg = nullptr;
-    RVB_CUDA(rvb_scratch_alloc((void**)&dneg, sizeof(__half) * 3 * (size_t)R, st));
-    normalize_dirs_kernel<<<(unsigned)ceil_div(R, 256), 256, 0, st>>>((const __half*)directions, R, dneg);
-    int rc = launch_cast_simple(t, (const __half*)sources, dneg, R, 1, dist, hit_slot, hit_tri, pt, nullptr, 0, nullptr,
-                                nullptr, st);
-    cudaFreeAsync(dneg, st);
-    return rc;
+    RvbTemp<__half> dneg;
+    RVB_CUDA(dneg.alloc_pool(3 * (size_t)R, st));
+    normalize_dirs_kernel<<<(unsigned)ceil_div(R, 256), 256, 0, st>>>((const __half*)directions, R, dneg.p);
+    return launch_cast_simple(t, (const __half*)sources, dneg.p, R, 1, dist, hit_slot, hit_tri, pt, nullptr, 0, nullptr, nullptr, st);
 }
 
 // ------------------------------------------------------------------------------------------------

@@ -954,12 +954,13 @@ int launch_shadow(rc::TiledParams q, int64_t N, const RaycastKnobs& knobs, cudaS
     // scratch: with RVB_SHADOW_DBG=1 the kernel's 24 counters (8 bytes each) first; then [0] steep count, [1] tilted envs placed,
     // [2] other envs placed, [3] handed-back count, the steep list [nblocks], the hand-back list [nblocks] and the env order [N]
     const int64_t ndbg = knobs.dbg ? 2 * 24 : 0;          // in ints
-    int* scratch = nullptr;
+    // The scratch is declared BEFORE the join guard: destructors run in reverse order, so st first waits for the side stream's
+    // tiled kernel, which reads the steep list and the counters, and only then gives the scratch back to the pool.
+    RvbTemp<int> scratch;
     RvbJoinGuard guard(st);
-    RVB_CUDA(rvb_scratch_alloc((void**)&scratch, sizeof(int) * (size_t)(ndbg + 4 + 2 * nblocks + N), st));
-    guard.scratch = scratch;
-    RVB_CUDA(cudaMemsetAsync(scratch, 0, sizeof(int) * (size_t)(ndbg + 4), st));
-    int* const counts = scratch + ndbg;
+    RVB_CUDA(scratch.alloc_pool((size_t)(ndbg + 4 + 2 * nblocks + N), st));
+    RVB_CUDA(cudaMemsetAsync(scratch.p, 0, sizeof(int) * (size_t)(ndbg + 4), st));
+    int* const counts = scratch.p + ndbg;
     int32_t* steep_list = counts + 4;
     q.fb_count = counts + 3;
     q.fb_list = counts + 4 + nblocks;
@@ -986,7 +987,7 @@ int launch_shadow(rc::TiledParams q, int64_t N, const RaycastKnobs& knobs, cudaS
     RVB_CUDA(cudaEventRecord(side->join, side->s));
     guard.join = side->join;
     const bool dbg = knobs.dbg;
-    if (dbg) q.dbg = reinterpret_cast<unsigned long long*>(scratch);
+    if (dbg) q.dbg = reinterpret_cast<unsigned long long*>(scratch.p);
     const unsigned grid = (unsigned)nblocks;
     if (q.tile_size <= RT_SMALL) {
         if (dbg) hm_shadow_kernel<true, RT_SMALL><<<grid, TT, shadow_smem_bytes(RT_SMALL), st>>>(q);
@@ -995,7 +996,7 @@ int launch_shadow(rc::TiledParams q, int64_t N, const RaycastKnobs& knobs, cudaS
         if (dbg) hm_shadow_kernel<true, RT_MAX><<<grid, TT, shadow_smem_bytes(RT_MAX), st>>>(q);
         else hm_shadow_kernel<false, RT_MAX><<<grid, TT, shadow_smem_bytes(RT_MAX), st>>>(q);
     }
-    if (cudaGetLastError() != cudaSuccess) return rvb_set_error(RVB_ERR_CUDA, "hm_shadow_kernel", "launch failed");
+    RVB_LAUNCH_CHECK();
     if (dbg) {
         unsigned long long h[24];
         int fb = 0;
@@ -1013,7 +1014,6 @@ int launch_shadow(rc::TiledParams q, int64_t N, const RaycastKnobs& knobs, cudaS
             fprintf(stderr, "[shadow dbg] phase 3 per warp (cycles): pulling chunks %.0f, draining the queues %.0f, waiting at the final barrier %.0f\n",
                     (double)h[16] / h[19], (double)h[17] / h[19], (double)h[18] / h[19]);
     }
-    // (env, tile) items the shadow kernel handed back: the tiled kernel loops over the list (usually empty).  On return the guard
-    // makes st wait for the steep list's kernel and gives the scratch back to the pool.
+    // (env, tile) items the shadow kernel handed back: the tiled kernel loops over the list (usually empty).
     return launch_tiled_list(q, q.fb_count, q.fb_list, tgrid, st);
 }

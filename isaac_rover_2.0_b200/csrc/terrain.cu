@@ -1,6 +1,6 @@
 // Terrain-layer handle: K-contiguous index copy + pre-resolved triangle records.
+#include <memory>
 #include <new>
-#include <string.h>
 
 #include <cub/device/device_radix_sort.cuh>
 #include <cub/device/device_scan.cuh>
@@ -265,45 +265,31 @@ __global__ void sb_ids_kernel(const unsigned long long* __restrict__ keys, int64
     if (i < n) ids[i] = (int32_t)(uint32_t)keys[i];
 }
 
-// position of every superblock-list triangle in each of the superblock's block lists (binary search; lists sorted by id)
-__global__ void sb_pos_kernel(const uint32_t* __restrict__ sb_off, const int32_t* __restrict__ sb_ids, const uint32_t* __restrict__ blk_off,
-                              const int32_t* __restrict__ blk_ids, int nBx, int nBy, int nSBy, uint16_t* __restrict__ pos) {
+// The slot bytes per (superblock-list entry, block), gathered once from the block lists: the shadow kernel's literal stage then
+// needs ONE look-up per (ray, triangle) pair instead of two dependent ones (position in the block list, then the slot byte there):
+// 6.23 -> 5.99 ms per 32,768 envs for 576 instead of 128 bytes per entry.  The entry's triangle is found in each of the
+// superblock's block lists by binary search (lists sorted by id; the pad entry of an odd list repeats the last id, so the
+// search lands on the real entry).
+__global__ void sb_slot9_kernel(const uint32_t* __restrict__ sb_off, const int32_t* __restrict__ sb_ids, const uint32_t* __restrict__ blk_off,
+                                const int32_t* __restrict__ blk_ids, const uint4* __restrict__ blk_slots, int nBx, int nBy, int nSBy,
+                                unsigned char* __restrict__ out) {
     const int SX = blockIdx.x / nSBy, SY = blockIdx.x % nSBy;
     const uint32_t e0 = sb_off[blockIdx.x], e1 = sb_off[blockIdx.x + 1];
     const uint32_t total = (e1 - e0) * (RVB_SB * RVB_SB);
     for (uint32_t w = threadIdx.x; w < total; w += blockDim.x) {
         const uint32_t ent = e0 + w / (RVB_SB * RVB_SB), b = w % (RVB_SB * RVB_SB);
         const int I = SX * RVB_SB + (int)(b / RVB_SB), J = SY * RVB_SB + (int)(b % RVB_SB);
-        uint16_t out = 0xffffu;
+        uint4 sl = make_uint4(0xffffffffu, 0xffffffffu, 0xffffffffu, 0xffffffffu);
         if (I < nBx && J < nBy) {
             const int32_t id = sb_ids[ent];
-            const uint32_t o0 = blk_off[(uint32_t)I * nBy + J], o1 = blk_off[(uint32_t)I * nBy + J + 1];
-            uint32_t lo = o0, hi = o1;
+            const uint32_t o1 = blk_off[(uint32_t)I * nBy + J + 1];
+            uint32_t lo = blk_off[(uint32_t)I * nBy + J], hi = o1;
             while (lo < hi) {
                 const uint32_t mid = (lo + hi) >> 1;
                 if (blk_ids[mid] < id) lo = mid + 1; else hi = mid;
             }
-            if (lo < o1 && blk_ids[lo] == id && lo - o0 < 0xffffu) out = (uint16_t)(lo - o0);
+            if (lo < o1 && blk_ids[lo] == id) sl = blk_slots[lo];
         }
-        pos[(size_t)ent * (RVB_SB * RVB_SB) + b] = out;
-    }
-}
-
-// The slot bytes themselves per (superblock-list entry, block), gathered once from the block lists: the shadow kernel's literal
-// stage then needs ONE look-up per (ray, triangle) pair instead of two dependent ones (position in the block list, then the slot
-// byte there): 6.23 -> 5.99 ms per 32,768 envs for 576 instead of 128 bytes per entry (the u16 position table is only a
-// temporary of the build now)
-__global__ void sb_slot9_kernel(const uint32_t* __restrict__ sb_off, const uint16_t* __restrict__ pos, const uint32_t* __restrict__ blk_off,
-                                const uint4* __restrict__ blk_slots, int nBx, int nBy, int nSBy, unsigned char* __restrict__ out) {
-    const int SX = blockIdx.x / nSBy, SY = blockIdx.x % nSBy;
-    const uint32_t e0 = sb_off[blockIdx.x], e1 = sb_off[blockIdx.x + 1];
-    const uint32_t total = (e1 - e0) * (RVB_SB * RVB_SB);
-    for (uint32_t w = threadIdx.x; w < total; w += blockDim.x) {
-        const uint32_t ent = e0 + w / (RVB_SB * RVB_SB), b = w % (RVB_SB * RVB_SB);
-        const int I = SX * RVB_SB + (int)(b / RVB_SB), J = SY * RVB_SB + (int)(b % RVB_SB);
-        const uint16_t p16 = pos[(size_t)ent * (RVB_SB * RVB_SB) + b];
-        uint4 sl = make_uint4(0xffffffffu, 0xffffffffu, 0xffffffffu, 0xffffffffu);
-        if (p16 != 0xffffu && I < nBx && J < nBy) sl = blk_slots[blk_off[(uint32_t)I * nBy + J] + p16];
         // laid out by CELL of the superblock (24 x 24): the kernel indexes it with (cx % 24) * 24 + cy % 24
         const unsigned char* sb = reinterpret_cast<const unsigned char*>(&sl);
         constexpr int SBC = RVB_SB * RVB_BLK;
@@ -360,68 +346,44 @@ static int build_superblock_lists(rvb_terrain* t, cudaStream_t st) {
     t->nSBy = (int32_t)ceil_div(t->nBy, RVB_SB);
     const int64_t nb = (int64_t)t->nBx * t->nBy, nsb = (int64_t)t->nSBx * t->nSBy, n = t->n_ent;
     if (!t->blk_ids || n <= 0 || n >= ((int64_t)1 << 31)) return RVB_OK;
-    unsigned long long *k0 = nullptr, *k1 = nullptr;
-    int64_t* d_num = nullptr;
-    void* tmp = nullptr;
-    uint16_t* sb_pos = nullptr;      // position of every entry's triangle in each block list: temporary of the slot table's build
-    int rc = RVB_OK;
-    cudaError_t e = cudaMalloc(&k0, sizeof(unsigned long long) * n);
-    if (e == cudaSuccess) e = cudaMalloc(&k1, sizeof(unsigned long long) * n);
-    if (e == cudaSuccess) e = cudaMalloc(&d_num, sizeof(int64_t));
+    RvbTemp<unsigned long long> k0, k1;
+    RvbTemp<int64_t> d_num;
+    RvbTemp<unsigned char> tmp;
+    RVB_CUDA(k0.alloc(n));
+    RVB_CUDA(k1.alloc(n));
+    RVB_CUDA(d_num.alloc(1));
+    sb_keys_kernel<<<(unsigned)nb, 128, 0, st>>>(t->blk_off, t->blk_ids, t->recs, t->nBy, t->nSBy, k0.p);
+    RVB_LAUNCH_CHECK();
+    const int sb_bits = 32;          // all 64 key bits: the all-ones key of the dropped triangles has to sort last
+    size_t b0 = 0, b1 = 0;
+    RVB_CUDA(cub::DeviceRadixSort::SortKeys(nullptr, b0, k0.p, k1.p, (int)n, 0, 32 + sb_bits, st));
+    RVB_CUDA(cub::DeviceSelect::Unique(nullptr, b1, k1.p, k0.p, d_num.p, (int)n, st));
+    RVB_CUDA(tmp.alloc(b0 > b1 ? b0 : b1));
+    RVB_CUDA(cub::DeviceRadixSort::SortKeys(tmp.p, b0, k0.p, k1.p, (int)n, 0, 32 + sb_bits, st));
+    RVB_CUDA(cub::DeviceSelect::Unique(tmp.p, b1, k1.p, k0.p, d_num.p, (int)n, st));
     int64_t n_u = 0;
-    if (e == cudaSuccess) {
-        sb_keys_kernel<<<(unsigned)nb, 128, 0, st>>>(t->blk_off, t->blk_ids, t->recs, t->nBy, t->nSBy, k0);
-        const int sb_bits = 32;          // all 64 key bits: the all-ones key of the dropped triangles has to sort last
-        size_t b0 = 0, b1 = 0;
-        cub::DeviceRadixSort::SortKeys(nullptr, b0, k0, k1, (int)n, 0, 32 + sb_bits, st);
-        cub::DeviceSelect::Unique(nullptr, b1, k1, k0, d_num, (int)n, st);
-        e = cudaMalloc(&tmp, b0 > b1 ? b0 : b1);
-        if (e == cudaSuccess) {
-            size_t b = b0;
-            cub::DeviceRadixSort::SortKeys(tmp, b, k0, k1, (int)n, 0, 32 + sb_bits, st);
-            b = b1;
-            cub::DeviceSelect::Unique(tmp, b, k1, k0, d_num, (int)n, st);
-            e = cudaMemcpyAsync(&n_u, d_num, sizeof(int64_t), cudaMemcpyDeviceToHost, st);
-            if (e == cudaSuccess) e = cudaStreamSynchronize(st);
-            unsigned long long last = 0;
-            if (e == cudaSuccess && n_u > 0) e = cudaMemcpy(&last, k0 + n_u - 1, sizeof(last), cudaMemcpyDeviceToHost);
-            if (e == cudaSuccess && n_u > 0 && last == ~0ull) --n_u;          // the dropped triangles' one surviving key
-        }
-    }
-    if (e == cudaSuccess) {
-        t->n_sb_ent = n_u;
-        e = cudaMalloc(&t->sb_off, sizeof(uint32_t) * (nsb + 1));
-        if (e == cudaSuccess) e = cudaMalloc(&t->sb_ids, sizeof(int32_t) * (size_t)(n_u > 0 ? n_u : 1));
-        if (e == cudaSuccess) {
-            sb_offsets_kernel<<<(unsigned)ceil_div(nsb + 1, 256), 256, 0, st>>>(k0, n_u, nsb, t->sb_off);
-            sb_ids_kernel<<<(unsigned)ceil_div(n_u > 0 ? n_u : 1, 256), 256, 0, st>>>(k0, n_u, t->sb_ids);
-            e = cudaGetLastError();
-            if (e == cudaSuccess) e = cudaMalloc(&sb_pos, sizeof(uint16_t) * RVB_SB * RVB_SB * (size_t)(n_u > 0 ? n_u : 1));
-            if (e == cudaSuccess) {
-                sb_pos_kernel<<<(unsigned)nsb, 256, 0, st>>>(t->sb_off, t->sb_ids, t->blk_off, t->blk_ids, t->nBx, t->nBy, t->nSBy, sb_pos);
-                e = cudaGetLastError();
-            }
-            if (e == cudaSuccess) e = cudaMalloc(&t->sb_slot9, (size_t)9 * RVB_SB * RVB_SB * (size_t)(n_u > 0 ? n_u : 1));
-            if (e == cudaSuccess) {
-                sb_slot9_kernel<<<(unsigned)nsb, 256, 0, st>>>(t->sb_off, sb_pos, t->blk_off, t->blk_slots, t->nBx, t->nBy, t->nSBy, t->sb_slot9);
-                e = cudaGetLastError();
-            }
-            const int64_t nwin = ceil_div(n_u > 0 ? n_u : 1, 32);
-            if (e == cudaSuccess) e = cudaMalloc(&t->sb_chunk, sizeof(ChunkRec) * (size_t)nwin);
-            if (e == cudaSuccess) {
-                sb_chunk_kernel<<<(unsigned)ceil_div(nwin * 32, 256), 256, 0, st>>>(t->sb_ids, n_u, t->s1recs, t->sb_chunk);
-                e = cudaGetLastError();
-            }
-            if (e == cudaSuccess) e = cudaStreamSynchronize(st);
-        }
-    }
-    cudaFree(sb_pos);
-    cudaFree(tmp);
-    cudaFree(d_num);
-    cudaFree(k1);
-    cudaFree(k0);
-    if (e != cudaSuccess) rc = rvb_set_error(RVB_ERR_CUDA, "rvb_terrain_create (superblock lists)", cudaGetErrorString(e));
-    return rc;
+    unsigned long long last = 0;          // largest sorted key: all ones exactly when dropped triangles exist
+    RVB_CUDA(cudaMemcpyAsync(&n_u, d_num.p, sizeof(int64_t), cudaMemcpyDeviceToHost, st));
+    RVB_CUDA(cudaMemcpyAsync(&last, k1.p + n - 1, sizeof(last), cudaMemcpyDeviceToHost, st));
+    RVB_CUDA(cudaStreamSynchronize(st));
+    if (n_u > 0 && last == ~0ull) --n_u;          // the dropped triangles' one surviving key
+    t->n_sb_ent = n_u;
+    const size_t n_alloc = n_u > 0 ? n_u : 1;
+    RVB_CUDA(cudaMalloc(&t->sb_off, sizeof(uint32_t) * (nsb + 1)));
+    RVB_CUDA(cudaMalloc(&t->sb_ids, sizeof(int32_t) * n_alloc));
+    sb_offsets_kernel<<<(unsigned)ceil_div(nsb + 1, 256), 256, 0, st>>>(k0.p, n_u, nsb, t->sb_off);
+    sb_ids_kernel<<<(unsigned)ceil_div(n_alloc, 256), 256, 0, st>>>(k0.p, n_u, t->sb_ids);
+    RVB_LAUNCH_CHECK();
+    RVB_CUDA(cudaMalloc(&t->sb_slot9, (size_t)9 * RVB_SB * RVB_SB * n_alloc));
+    sb_slot9_kernel<<<(unsigned)nsb, 256, 0, st>>>(t->sb_off, t->sb_ids, t->blk_off, t->blk_ids, t->blk_slots, t->nBx, t->nBy, t->nSBy,
+                                                   t->sb_slot9);
+    RVB_LAUNCH_CHECK();
+    const int64_t nwin = ceil_div(n_alloc, 32);
+    RVB_CUDA(cudaMalloc(&t->sb_chunk, sizeof(ChunkRec) * (size_t)nwin));
+    sb_chunk_kernel<<<(unsigned)ceil_div(nwin * 32, 256), 256, 0, st>>>(t->sb_ids, n_u, t->s1recs, t->sb_chunk);
+    RVB_LAUNCH_CHECK();
+    RVB_CUDA(cudaStreamSynchronize(st));
+    return RVB_OK;
 }
 
 static int build_block_lists(rvb_terrain* t, cudaStream_t st) {
@@ -429,25 +391,18 @@ static int build_block_lists(rvb_terrain* t, cudaStream_t st) {
     t->nBy = (int32_t)ceil_div(t->G1, RVB_BLK);
     const int64_t nb = (int64_t)t->nBx * t->nBy;
     if (t->K > 255 || nb >= ((int64_t)1 << 31)) return RVB_OK;      // per-cell path only
-    // temporaries of this function: freed on every exit, the early error returns included (the handle's own arrays are freed by
-    // rvb_terrain_create when this function fails)
-    struct Tmp {
-        uint32_t* counts = nullptr;
-        void* scan = nullptr;
-        ~Tmp() { cudaFree(scan); cudaFree(counts); }
-    } tm;
-    uint32_t*& counts = tm.counts;
-    void*& tmp = tm.scan;
+    RvbTemp<uint32_t> counts;
+    RvbTemp<unsigned char> tmp;
     RVB_CUDA(cudaMalloc(&t->blk_off, sizeof(uint32_t) * (nb + 1)));
-    RVB_CUDA(cudaMalloc(&counts, sizeof(uint32_t) * (nb + 1)));
-    RVB_CUDA(cudaMemsetAsync(counts, 0, sizeof(uint32_t) * (nb + 1), st));
+    RVB_CUDA(counts.alloc(nb + 1));
+    RVB_CUDA(cudaMemsetAsync(counts.p, 0, sizeof(uint32_t) * (nb + 1), st));
     build_blocks_kernel<<<(unsigned)nb, BLK_THREADS, 0, st>>>(t->index, (int)t->G0, (int)t->G1, (int)t->K, (int)t->Ks, t->nBy, nullptr,
-                                                             counts, nullptr, nullptr);
+                                                             counts.p, nullptr, nullptr);
     RVB_LAUNCH_CHECK();
     size_t tmp_bytes = 0;
-    cub::DeviceScan::ExclusiveSum(nullptr, tmp_bytes, counts, t->blk_off, (int)(nb + 1), st);
-    RVB_CUDA(cudaMalloc(&tmp, tmp_bytes));
-    cub::DeviceScan::ExclusiveSum(tmp, tmp_bytes, counts, t->blk_off, (int)(nb + 1), st);
+    RVB_CUDA(cub::DeviceScan::ExclusiveSum(nullptr, tmp_bytes, counts.p, t->blk_off, (int)(nb + 1), st));
+    RVB_CUDA(tmp.alloc(tmp_bytes));
+    RVB_CUDA(cub::DeviceScan::ExclusiveSum(tmp.p, tmp_bytes, counts.p, t->blk_off, (int)(nb + 1), st));
     uint32_t total = 0;
     RVB_CUDA(cudaMemcpyAsync(&total, t->blk_off + nb, sizeof(uint32_t), cudaMemcpyDeviceToHost, st));
     RVB_CUDA(cudaStreamSynchronize(st));
@@ -475,49 +430,38 @@ extern "C" int rvb_terrain_create(rvb_terrain** out, const int32_t* map_indices,
     RVB_REQUIRE(res > 0.0f, "rvb_terrain_create: res must be > 0");
     RVB_REQUIRE(sem == RVB_SEM_TORCH_CUDA || sem == RVB_SEM_TORCH_CPU, "rvb_terrain_create: bad sem");
     cudaStream_t st = as_stream(stream);
-    rvb_terrain* t = new (std::nothrow) rvb_terrain();
+    // value-initialised (every array null), so on a failure rvb_terrain_destroy frees exactly what was built
+    std::unique_ptr<rvb_terrain, int (*)(rvb_terrain*)> t(new (std::nothrow) rvb_terrain(), rvb_terrain_destroy);
     if (!t) return rvb_set_error(RVB_ERR_NOMEM, "rvb_terrain_create", "host allocation failed");
-    memset(t, 0, sizeof(*t));
     t->G0 = G0; t->G1 = G1; t->K = K; t->Ks = (K + 1) & ~(int64_t)1; t->T = T; t->V = V;
     t->res = res; t->shift_x = shift_x; t->shift_y = shift_y; t->sem = sem;
-    int* bad = nullptr;
-    int hbad = 0;
-    cudaError_t e = cudaGetDevice(&t->device);
-    if (e == cudaSuccess) e = cudaMalloc(&t->index, sizeof(int32_t) * G0 * G1 * t->Ks);
-    if (e == cudaSuccess) e = cudaMalloc(&t->recs, sizeof(TriRec) * T);
-    if (e == cudaSuccess) e = cudaMalloc(&t->s1recs, sizeof(S1Rec) * T);
-    if (e == cudaSuccess) e = cudaMalloc(&bad, 2 * sizeof(int));
-    if (e == cudaSuccess) e = cudaMemsetAsync(bad, 0, 2 * sizeof(int), st);
-    if (e == cudaSuccess) {
+    RVB_CUDA(cudaGetDevice(&t->device));
+    RVB_CUDA(cudaMalloc(&t->index, sizeof(int32_t) * G0 * G1 * t->Ks));
+    RVB_CUDA(cudaMalloc(&t->recs, sizeof(TriRec) * T));
+    RVB_CUDA(cudaMalloc(&t->s1recs, sizeof(S1Rec) * T));
+    {
+        RvbTemp<int> bad;
+        RVB_CUDA(bad.alloc(2));
+        RVB_CUDA(cudaMemsetAsync(bad.p, 0, 2 * sizeof(int), st));
         repack_index_kernel<<<148 * 8, 256, 0, st>>>(map_indices, G0, G1, K, t->Ks, stride_g0, stride_g1, stride_k, (int32_t)T,
-                                                     t->index, bad);
+                                                     t->index, bad.p);
         build_records_kernel<<<(unsigned)ceil_div(T, 256), 256, 0, st>>>(triangles, T, (const __half*)vertices, V,
-                                                                         t->recs, t->s1recs, bad);
-        e = cudaGetLastError();
+                                                                         t->recs, t->s1recs, bad.p);
+        RVB_LAUNCH_CHECK();
+        int hb[2] = {0, 0};
+        RVB_CUDA(cudaMemcpyAsync(hb, bad.p, sizeof(hb), cudaMemcpyDeviceToHost, st));
+        RVB_CUDA(cudaStreamSynchronize(st));
+        if (hb[0])
+            return rvb_set_error(RVB_ERR_INVALID, "rvb_terrain_create",
+                                 hb[0] == 1 ? "map_indices holds a triangle id outside [0,T)" : "triangles holds a vertex id outside [0,V)");
+        t->n_ill = hb[1];
     }
-    int hb2[2] = {0, 0};
-    if (e == cudaSuccess) e = cudaMemcpyAsync(hb2, bad, 2 * sizeof(int), cudaMemcpyDeviceToHost, st);
-    if (e == cudaSuccess) e = cudaStreamSynchronize(st);
-    hbad = hb2[0];
-    t->n_ill = hb2[1];
-    if (bad) cudaFree(bad);
-    // failure: the handle was zeroed at allocation, so rvb_terrain_destroy frees exactly what was built (cudaFree(nullptr) is a no-op)
-    if (e == cudaSuccess && !hbad && !(flags & RVB_LAYER_INDEX_ONLY)) {
-        const int rc = build_block_lists(t, st);
-        if (rc == RVB_OK) e = cudaStreamSynchronize(st);
-        if (rc != RVB_OK || e != cudaSuccess) {
-            rvb_terrain_destroy(t);
-            return rc != RVB_OK ? rc : rvb_set_error(RVB_ERR_CUDA, "rvb_terrain_create (block lists)", cudaGetErrorString(e));
-        }
+    if (!(flags & RVB_LAYER_INDEX_ONLY)) {
+        const int rc = build_block_lists(t.get(), st);
+        if (rc != RVB_OK) return rc;
+        RVB_CUDA(cudaStreamSynchronize(st));
     }
-    if (e != cudaSuccess || hbad) {
-        rvb_terrain_destroy(t);
-        if (e != cudaSuccess) return rvb_set_error(RVB_ERR_CUDA, "rvb_terrain_create", cudaGetErrorString(e));
-        return rvb_set_error(RVB_ERR_INVALID, "rvb_terrain_create",
-                             hbad == 1 ? "map_indices holds a triangle id outside [0,T)"
-                                       : "triangles holds a vertex id outside [0,V)");
-    }
-    *out = t;
+    *out = t.release();
     return RVB_OK;
 }
 
