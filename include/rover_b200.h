@@ -315,6 +315,16 @@ int rvb_policy_variant(int variant);
  * value.compute on the same states.  Twice the CTAs for the same obs tile (second read served by L2). */
 int rvb_policy_forward_pair(const rvb_policy* a, const rvb_policy* b, const float* obs, int64_t obs_ld, int64_t N,
                             float* out_a, int64_t out_a_ld, float* out_b, int64_t out_b_ld, void* stream);
+/* The same networks on the packed observation of the fused step (rvb_step_io.obs_h16): proprio f32 [N, proprio_ld >= p] (obs[:, 0:p],
+ * e.g. the strided view obs_buf[:, :4]) and heightmap f16 [N, heightmap_ld >= S+D] (the sparse then the dense columns, as raw fp16
+ * bits).  b = NULL runs network a alone (out_b is ignored); otherwise a and b as in rvb_policy_forward_pair.  The result is bit for bit
+ * that of rvb_policy_forward(_pair) on the widened rows cat(proprio, float(heightmap)), on either path: the heightmap's fp16 values
+ * are exact in tf32, so the tensor-core path reads them as they are (half the bytes) and splits nothing.  It takes the tensor-core
+ * path when p == 4, S and D are even, heightmap_ld is even and heightmap is 4-byte aligned (and rvb_policy_variant is 2); the FFMA2
+ * kernel otherwise, for any 2-byte aligned heightmap.  Null pointers, short rows and mismatched networks are refused on the host. */
+int rvb_policy_forward_packed(const rvb_policy* a, const rvb_policy* b, const float* proprio, int64_t proprio_ld,
+                              const uint16_t* heightmap, int64_t heightmap_ld, int64_t N, float* out_a, int64_t out_a_ld,
+                              float* out_b, int64_t out_b_ld, void* stream);
 
 /* ------------------------------------------------------------------------------------------------
  * Observation hooks and the teacher-data recorder (SURVEY.md 8f-4).

@@ -82,6 +82,7 @@ _SIGNATURES = {
     "rvb_policy_bytes": (i64, [p]),
     "rvb_policy_forward": (C.c_int, [p, p, i64, i64, p, i64, p]),
     "rvb_policy_forward_pair": (C.c_int, [p, p, p, i64, i64, p, i64, p, i64, p]),
+    "rvb_policy_forward_packed": (C.c_int, [p, p, p, i64, p, i64, i64, p, i64, p, i64, p]),
     "rvb_policy_variant": (C.c_int, [C.c_int]),
     "rvb_obs_hooks": (C.c_int, [p, i64, i64, i64, i64, f32, f32, f32, p, C.c_uint64, C.c_uint64, i64, p]),
     "rvb_teacher_record": (C.c_int, [p, p, i64, p, i64, i64, i64, p, i64, p]),
@@ -100,6 +101,7 @@ KERNELS_PER_CALL = {"rvb_terrain_create": 2, "rvb_heightmap_raycast": 4, "rvb_ca
                     "rvb_history_push": 1, "rvb_obs_proprio": 1, "rvb_obs_gather": 1, "rvb_reward_reset": 2, "rvb_env_step": 8,
     "rvb_stone_validate": 1, "rvb_spawn_validate": 1, "rvb_height_lookup": 1, "rvb_build_knn_index": 6, "rvb_reset_targets": 1,
                     "rvb_policy_create": 7, "rvb_policy_forward": 1, "rvb_policy_forward_pair": 1,
+                    "rvb_policy_forward_packed": 2,
                     "rvb_obs_hooks": 1, "rvb_teacher_record": 1}
 launch_count = 0
 

@@ -24,6 +24,7 @@
 #include <memory>
 #include <new>
 #include <stdlib.h>
+#include <type_traits>
 
 #include "common.cuh"
 
@@ -111,11 +112,16 @@ __global__ void pl_pack_kernel(const float* __restrict__ w, const float* __restr
     if (i < outp) bias[i] = i < out ? b[i] : 0.f;
 }
 
+// an observation value as f32: the f32 rows as they are, the packed fp16 heightmap widened (exact)
+__device__ __forceinline__ float pl_ldg(const float* p) { return __ldg(p); }
+__device__ __forceinline__ float pl_ldg(const __half* p) { return __half2float(__ldg(p)); }
+
 // One dense layer of the tile.  Input activations: shared memory `act_in` [K][PL_LDA] (GLOBAL_IN = false) or columns
-// [col0, col0 + K) of the tile's observation rows in global memory, staged transposed through `xs` (GLOBAL_IN = true).
-// Output: act(in . Wt + bias) into shared memory `act_out` [n][PL_LDA], rows n < OUT only.
-template <int CN, bool GLOBAL_IN>
-__device__ __forceinline__ void pl_dense(const float* __restrict__ act_in, const float* __restrict__ obs, int64_t obs_ld, int64_t m0,
+// [col0, col0 + K) of the tile's observation rows in global memory (f32 or fp16), staged transposed through `xs` as f32
+// (GLOBAL_IN = true).  Output: act(in . Wt + bias) into shared memory `act_out` [n][PL_LDA], rows n < OUT only.
+template <typename T> struct pl_given { using type = T; };      // T as the caller names it (the layers on shared memory pass nullptr)
+template <int CN, bool GLOBAL_IN, typename T = float>
+__device__ __forceinline__ void pl_dense(const float* __restrict__ act_in, const typename pl_given<T>::type* __restrict__ obs, int64_t obs_ld, int64_t m0,
                                          int64_t N, int col0, int K, const PackedLinear& L, float* __restrict__ xs,
                                          float* __restrict__ ws, float* __restrict__ act_out, int act_kind) {
     constexpr int OUTP = 32 * CN;
@@ -143,7 +149,7 @@ __device__ __forceinline__ void pl_dense(const float* __restrict__ act_in, const
 #pragma unroll
             for (int r = 0; r < PL_TM / 8; ++r) {
                 const int m = mg + 8 * r;
-                xreg[r] = (ng < kc && m0 + m < N) ? __ldg(obs + (m0 + m) * obs_ld + col0 + k0 + ng) : 0.f;
+                xreg[r] = (ng < kc && m0 + m < N) ? pl_ldg(obs + (m0 + m) * obs_ld + col0 + k0 + ng) : 0.f;
             }
         }
     };
@@ -206,10 +212,13 @@ __device__ __forceinline__ void pl_dense(const float* __restrict__ act_in, const
 #define PL_SM_FLOATS (PL_SM_WS + PL_WS_FLOATS)
 #define PL_SMEM_BYTES (PL_SM_FLOATS * 4)
 
-__global__ void __launch_bounds__(PL_THREADS, 2)
-policy_forward_kernel(const PolicyDev* __restrict__ p0, const PolicyDev* __restrict__ p1, const float* __restrict__ obs,
-                      int64_t obs_ld, int64_t N, float* __restrict__ out0, int64_t out0_ld, float* __restrict__ out1,
-                      int64_t out1_ld) {
+// The observation of a row: proprio[0, p) and the heightmap's sparse | dense columns, which start at column p of hm's row
+// (hm_after_proprio: the f32 rows, passed as both sources) or at column 0 (the packed form: obs_buf[:, :p] and the fp16 heightmap).
+template <typename T>
+__device__ __forceinline__ void policy_forward_body(const PolicyDev* __restrict__ p0, const PolicyDev* __restrict__ p1,
+                                                    const float* __restrict__ proprio, int64_t proprio_ld, const T* __restrict__ hm,
+                                                    int64_t hm_ld, bool hm_after_proprio, int64_t N, float* __restrict__ out0,
+                                                    int64_t out0_ld, float* __restrict__ out1, int64_t out1_ld) {
     // blockIdx.y selects the network (actor / critic of one PPO step read the same obs tile, hot in L2)
     const PolicyDev& P = *(blockIdx.y ? p1 : p0);
     float* __restrict__ out = blockIdx.y ? out1 : out0;
@@ -227,13 +236,14 @@ policy_forward_kernel(const PolicyDev* __restrict__ p0, const PolicyDev* __restr
     // proprioceptive columns -> concat rows 0..p-1 (model.py:188)
     if (tid < PL_TM * p) {
         const int m = tid & 31, k = tid >> 5;
-        A[k * PL_LDA + m] = (m0 + m < N) ? __ldg(obs + (m0 + m) * obs_ld + k) : 0.f;
+        A[k * PL_LDA + m] = (m0 + m < N) ? __ldg(proprio + (m0 + m) * proprio_ld + k) : 0.f;
     }
+    const int hm_col0 = hm_after_proprio ? p : 0;
     // sparse encoder (model.py:186) -> concat rows p .. p+59
-    pl_dense<3, true>(nullptr, obs, obs_ld, m0, N, p, P.n_sparse, P.es1, xs, ws, Cb, P.act);
+    pl_dense<3, true, T>(nullptr, hm, hm_ld, m0, N, hm_col0, P.n_sparse, P.es1, xs, ws, Cb, P.act);
     pl_dense<2, false>(Cb, nullptr, 0, 0, 0, 0, PL_E1, P.es2, xs, ws, A + p * PL_LDA, P.act);
     // dense encoder (model.py:187) -> concat rows p+60 .. p+119
-    pl_dense<3, true>(nullptr, obs, obs_ld, m0, N, p + P.n_sparse, P.n_dense, P.ed1, xs, ws, Cb, P.act);
+    pl_dense<3, true, T>(nullptr, hm, hm_ld, m0, N, hm_col0 + P.n_sparse, P.n_dense, P.ed1, xs, ws, Cb, P.act);
     pl_dense<2, false>(Cb, nullptr, 0, 0, 0, 0, PL_E1, P.ed2, xs, ws, A + (p + PL_E2) * PL_LDA, P.act);
     // MLP (model.py:190-191)
     pl_dense<8, false>(A, nullptr, 0, 0, 0, 0, p + 2 * PL_E2, P.m1, xs, ws, B, P.act);
@@ -250,6 +260,21 @@ policy_forward_kernel(const PolicyDev* __restrict__ p0, const PolicyDev* __restr
         acc = __fadd_rn(acc, __ldg(P.head_b + o));
         out[(m0 + m) * out_ld + o] = P.head_tanh ? tanhf(acc) : acc;
     }
+}
+
+__global__ void __launch_bounds__(PL_THREADS, 2)
+policy_forward_kernel(const PolicyDev* __restrict__ p0, const PolicyDev* __restrict__ p1, const float* __restrict__ obs,
+                      int64_t obs_ld, int64_t N, float* __restrict__ out0, int64_t out0_ld, float* __restrict__ out1,
+                      int64_t out1_ld) {
+    policy_forward_body(p0, p1, obs, obs_ld, obs, obs_ld, true, N, out0, out0_ld, out1, out1_ld);
+}
+
+// the packed observation: any 2-byte aligned heightmap, any hm_ld (scalar loads)
+__global__ void __launch_bounds__(PL_THREADS, 2)
+policy_forward_h16_kernel(const PolicyDev* __restrict__ p0, const PolicyDev* __restrict__ p1, const float* __restrict__ proprio,
+                          int64_t proprio_ld, const __half* __restrict__ hm, int64_t hm_ld, int64_t N, float* __restrict__ out0,
+                          int64_t out0_ld, float* __restrict__ out1, int64_t out1_ld) {
+    policy_forward_body(p0, p1, proprio, proprio_ld, hm, hm_ld, false, N, out0, out0_ld, out1, out1_ld);
 }
 
 
@@ -314,10 +339,13 @@ __device__ __forceinline__ void tc_wait(uint64_t* bar, uint32_t parity) {
     __trap();
 }
 
-template <int NETS>
-__global__ void __launch_bounds__(TC_THREADS, 1)
-policy_l1_tc_kernel(const PolicyDev* __restrict__ p0, const PolicyDev* __restrict__ p1, const float* __restrict__ obs, int64_t obs_ld,
-                    int64_t N, float* __restrict__ h1) {
+// T = float: the f32 observation rows (the encoders' columns start at p).  T = __half: the packed heightmap rows (they start at 0),
+// fp16 values, exact in tf32: the loaders widen them and store the hi tile only -- no lo part, no lo flag, so the MMA warp issues
+// the two MMAs per k-step it issues for f32 rows holding the same values.
+template <int NETS, typename T>
+__device__ __forceinline__ void policy_l1_tc_body(const PolicyDev* __restrict__ p0, const PolicyDev* __restrict__ p1,
+                                                  const T* __restrict__ obs, int64_t obs_ld, int64_t N, float* __restrict__ h1) {
+    constexpr bool H16 = std::is_same<T, __half>::value;
     constexpr int NB = PL_E1 * NETS;                      // MMA N: 80 columns per network
     constexpr int A_FLOATS = 2 * TC_M * TC_KC;            // hi + lo, 2 x 16 KB
     constexpr int W_FLOATS = 2 * NB * TC_KC;              // hi + lo, 20 KB per network
@@ -371,24 +399,27 @@ policy_l1_tc_kernel(const PolicyDev* __restrict__ p0, const PolicyDev* __restric
         // part.  (A thread-per-row layout made every load 32 L1 wavefronts; a lane-per-column layout needed two 4-byte stores per
         // element: the loaders, not the tensor core, set the pace -- 2.2 us per chunk.)  Chunk c+1 travels global -> registers
         // while chunk c is split and stored (two register buffers in ping-pong: a copy would wait for the loads it should hide).
+        // The fp16 rows keep the lane map: a chunk row is 64 bytes, eight lanes read 8 bytes each as two 4-byte loads (a dense block
+        // S halves into the row is only 4-byte aligned) and store the lane's 16-byte group of the f32 hi tile with one store.
         const int ri = lane >> 3, c16 = lane & 7;
         const int64_t rbase = m0 + warp * 16 + ri;
-        const float* obase = obs + P0.n_proprio + (dense ? P0.n_sparse : 0) + c16 * 4;
+        const T* obase = obs + (H16 ? 0 : P0.n_proprio) + (dense ? P0.n_sparse : 0) + c16 * 4;
         const int kall = dense ? P0.n_dense : P0.n_sparse;
-        auto fetch = [&](int c, float2* v) {
+        using V = typename std::conditional<H16, __half2, float2>::type;
+        auto fetch = [&](int c, V* v) {
             const int k0 = c * TC_KC;
             const int kmax = kall - k0;                                             // valid columns of this chunk (even)
-            const float* src = obase + k0;
+            const T* src = obase + k0;
 #pragma unroll
             for (int it = 0; it < 4; ++it) {
                 const int64_t row = rbase + 4 * it;
-                const float2* q = reinterpret_cast<const float2*>(src + row * obs_ld);
+                const V* q = reinterpret_cast<const V*>(src + row * obs_ld);
                 const bool ok = row < N;
-                v[2 * it] = (ok && c16 * 4 < kmax) ? __ldg(q) : make_float2(0.f, 0.f);
-                v[2 * it + 1] = (ok && c16 * 4 + 2 < kmax) ? __ldg(q + 1) : make_float2(0.f, 0.f);
+                v[2 * it] = (ok && c16 * 4 < kmax) ? __ldg(q) : V{};
+                v[2 * it + 1] = (ok && c16 * 4 + 2 < kmax) ? __ldg(q + 1) : V{};
             }
         };
-        auto process = [&](int c, const float2* v) {
+        auto process = [&](int c, const V* v) {
             const int s = c % TC_STAGES;
             const uint32_t ph = (uint32_t)(c / TC_STAGES) & 1u;
             tc_wait(&empty[s], ph ^ 1u);
@@ -397,25 +428,35 @@ policy_l1_tc_kernel(const PolicyDev* __restrict__ p0, const PolicyDev* __restric
 #pragma unroll
             for (int it = 0; it < 4; ++it) {
                 const int r = warp * 16 + 4 * it + ri;
-                const float x[4] = {v[2 * it].x, v[2 * it].y, v[2 * it + 1].x, v[2 * it + 1].y};
-                float hi[4], lo[4];
+                if constexpr (H16) {
+                    float* dst = tile + (r >> 3) * 256 + (r & 7) * 32 + ((c16 ^ (r & 7)) << 2);
+                    const float2 a = __half22float2(v[2 * it]), b = __half22float2(v[2 * it + 1]);
+                    float x[4] = {a.x, a.y, b.x, b.y};
+                    // +-inf: the f32 rows' split gives lo = inf - inf = NaN, which turns the row's sums into NaN; so does NaN as hi
 #pragma unroll
-                for (int e = 0; e < 4; ++e) {
-                    uint32_t h, l;
-                    asm("cvt.rna.tf32.f32 %0, %1;" : "=r"(h) : "f"(x[e]));
-                    asm("cvt.rna.tf32.f32 %0, %1;" : "=r"(l) : "f"(__fsub_rn(x[e], __uint_as_float(h))));
-                    hi[e] = __uint_as_float(h); lo[e] = __uint_as_float(l);
-                    any_lo |= (l << 1) != 0u;
+                    for (int e = 0; e < 4; ++e) x[e] = isinf(x[e]) ? __int_as_float(0x7fffffff) : x[e];
+                    *reinterpret_cast<float4*>(dst) = make_float4(x[0], x[1], x[2], x[3]);
+                } else {
+                    const float x[4] = {v[2 * it].x, v[2 * it].y, v[2 * it + 1].x, v[2 * it + 1].y};
+                    float hi[4], lo[4];
+#pragma unroll
+                    for (int e = 0; e < 4; ++e) {
+                        uint32_t h, l;
+                        asm("cvt.rna.tf32.f32 %0, %1;" : "=r"(h) : "f"(x[e]));
+                        asm("cvt.rna.tf32.f32 %0, %1;" : "=r"(l) : "f"(__fsub_rn(x[e], __uint_as_float(h))));
+                        hi[e] = __uint_as_float(h); lo[e] = __uint_as_float(l);
+                        any_lo |= (l << 1) != 0u;
+                    }
+                    float* dst = tile + (r >> 3) * 256 + (r & 7) * 32 + ((c16 ^ (r & 7)) << 2);
+                    *reinterpret_cast<float4*>(dst) = make_float4(hi[0], hi[1], hi[2], hi[3]);
+                    *reinterpret_cast<float4*>(dst + TC_M * TC_KC) = make_float4(lo[0], lo[1], lo[2], lo[3]);
                 }
-                float* dst = tile + (r >> 3) * 256 + (r & 7) * 32 + ((c16 ^ (r & 7)) << 2);
-                *reinterpret_cast<float4*>(dst) = make_float4(hi[0], hi[1], hi[2], hi[3]);
-                *reinterpret_cast<float4*>(dst + TC_M * TC_KC) = make_float4(lo[0], lo[1], lo[2], lo[3]);
             }
-            if (__any_sync(0xffffffffu, any_lo) && lane == 0) atomicOr(&s_lo[c & 63], 1u);
+            if (!H16 && __any_sync(0xffffffffu, any_lo) && lane == 0) atomicOr(&s_lo[c & 63], 1u);
             asm volatile("fence.proxy.async.shared::cta;" ::: "memory");
             asm volatile("mbarrier.arrive.shared::cta.b64 _, [%0];" ::"r"(tc_smem(&full[s])) : "memory");
         };
-        float2 va[8], vb[8];
+        V va[8], vb[8];
         fetch(0, va);
         for (int c = 0; c < nchunks; c += 2) {
             if (c + 1 < nchunks) fetch(c + 1, vb);
@@ -491,7 +532,7 @@ policy_l1_tc_kernel(const PolicyDev* __restrict__ p0, const PolicyDev* __restric
                 const uint64_t da = tc_desc(tc_smem(st)), dal = tc_desc(tc_smem(st + TC_M * TC_KC)), dh = tc_desc(tc_smem(st + A_FLOATS)),
                                dl = tc_desc(tc_smem(st + A_FLOATS + NB * TC_KC));
                 uint32_t acc = c == 0 ? 0u : 1u;
-                const bool with_lo = *reinterpret_cast<volatile uint32_t*>(&s_lo[c & 63]) != 0u;
+                const bool with_lo = !H16 && *reinterpret_cast<volatile uint32_t*>(&s_lo[c & 63]) != 0u;
 #pragma unroll
                 for (int k = 0; k < 4; ++k) {                    // 8 tf32 = 32 bytes = 2 descriptor units per MMA
                     tc_mma(d_tmem, da + 2 * k, dh + 2 * k, idesc, acc);
@@ -507,6 +548,21 @@ policy_l1_tc_kernel(const PolicyDev* __restrict__ p0, const PolicyDev* __restric
     asm volatile("tcgen05.fence::before_thread_sync;" ::: "memory");
     __syncthreads();
     if (warp == 8) asm volatile("tcgen05.dealloc.cta_group::1.sync.aligned.b32 %0, %1;" ::"r"(tmem_base), "r"(TMEM_COLS));
+}
+
+template <int NETS>
+__global__ void __launch_bounds__(TC_THREADS, 1)
+policy_l1_tc_kernel(const PolicyDev* __restrict__ p0, const PolicyDev* __restrict__ p1, const float* __restrict__ obs, int64_t obs_ld,
+                    int64_t N, float* __restrict__ h1) {
+    policy_l1_tc_body<NETS>(p0, p1, obs, obs_ld, N, h1);
+}
+
+// the packed heightmap: hm_ld even and hm 4-byte aligned (tc_usable)
+template <int NETS>
+__global__ void __launch_bounds__(TC_THREADS, 1)
+policy_l1_tc_h16_kernel(const PolicyDev* __restrict__ p0, const PolicyDev* __restrict__ p1, const __half* __restrict__ hm, int64_t hm_ld,
+                        int64_t N, float* __restrict__ h1) {
+    policy_l1_tc_body<NETS>(p0, p1, hm, hm_ld, N, h1);
 }
 
 static size_t tc_smem_bytes(int nets) { return (size_t)TC_STAGES * (2 * TC_M * TC_KC + 2 * PL_E1 * nets * TC_KC) * sizeof(float) + 1024; }
@@ -569,8 +625,8 @@ __global__ void pl_tail_image_kernel(const float* __restrict__ w, int in, int ou
 }
 
 __global__ void __launch_bounds__(TT_THREADS, 1)
-policy_tail_tc_kernel(const PolicyDev* __restrict__ p0, const PolicyDev* __restrict__ p1, const float* __restrict__ obs, int64_t obs_ld,
-                      int64_t N, const float* h1, int h1_nets, float* __restrict__ out0, int64_t out0_ld,
+policy_tail_tc_kernel(const PolicyDev* __restrict__ p0, const PolicyDev* __restrict__ p1, const float* __restrict__ proprio,
+                      int64_t proprio_ld, int64_t N, const float* h1, int h1_nets, float* __restrict__ out0, int64_t out0_ld,
                       float* __restrict__ out1, int64_t out1_ld) {
     const PolicyDev& P = *(blockIdx.y ? p1 : p0);
     float* __restrict__ out = blockIdx.y ? out1 : out0;
@@ -692,7 +748,7 @@ policy_tail_tc_kernel(const PolicyDev* __restrict__ p0, const PolicyDev* __restr
         // P2: x = cat(proprio, x0, x1) (model.py:188-189), 4 + 60 + 60 = 124 features (+ 4 zeros)
         wait_pass();
         {
-            const float* orow = obs + (live ? row : 0) * obs_ld;
+            const float* orow = proprio + (live ? row : 0) * proprio_ld;
             if (half == 0) {
                 const float4 pr = live ? make_float4(__ldg(orow), __ldg(orow + 1), __ldg(orow + 2), __ldg(orow + 3)) : make_float4(0.f, 0.f, 0.f, 0.f);
                 store4(0, pr.x, pr.y, pr.z, pr.w);          // n_proprio == 4 on this path (tc_usable)
@@ -893,6 +949,9 @@ extern "C" int rvb_policy_create(rvb_policy** out, int32_t n_proprio, int32_t n_
     RVB_CUDA(cudaFuncSetAttribute(policy_forward_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, PL_SMEM_BYTES));
     RVB_CUDA(cudaFuncSetAttribute(policy_l1_tc_kernel<1>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)tc_smem_bytes(1)));
     RVB_CUDA(cudaFuncSetAttribute(policy_l1_tc_kernel<2>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)tc_smem_bytes(2)));
+    RVB_CUDA(cudaFuncSetAttribute(policy_forward_h16_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, PL_SMEM_BYTES));
+    RVB_CUDA(cudaFuncSetAttribute(policy_l1_tc_h16_kernel<1>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)tc_smem_bytes(1)));
+    RVB_CUDA(cudaFuncSetAttribute(policy_l1_tc_h16_kernel<2>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)tc_smem_bytes(2)));
     RVB_CUDA(cudaFuncSetAttribute(policy_tail_tc_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)tt_smem_bytes()));
     RVB_CUDA(cudaStreamSynchronize(st));   // the caller may free its weight tensors on return
     *out = P.release();
@@ -921,9 +980,20 @@ extern "C" int rvb_policy_variant(int v) {
     return prev;
 }
 
-// the tensor-core path reads the observation rows with 8-byte loads
-static bool tc_usable(const PolicyDev* P, const float* obs, int64_t obs_ld) {
-    return g_policy_variant == 2 && (obs_ld % 2 == 0) && (P->n_proprio == 4) && (P->n_sparse % 2 == 0) && (P->n_dense % 2 == 0) && (((uintptr_t)obs & 7u) == 0);
+// What the kernels read of a row: the f32 observation (hm16 == nullptr: proprio = obs, the heightmap follows at column p of the same
+// row) or the packed form (proprio f32 [N, proprio_ld], the fp16 heightmap hm16 [N, hm_ld]).
+struct PolicyIn {
+    const float* proprio;
+    int64_t proprio_ld;
+    const __half* hm16;
+    int64_t hm_ld;
+};
+
+// the tensor-core path reads f32 observation rows with 8-byte loads and fp16 heightmap rows with 4-byte loads
+static bool tc_usable(const PolicyDev* P, const PolicyIn& in) {
+    const bool aligned = in.hm16 ? (in.hm_ld % 2 == 0) && (((uintptr_t)in.hm16 & 3u) == 0)
+                                 : (in.proprio_ld % 2 == 0) && (((uintptr_t)in.proprio & 7u) == 0);
+    return g_policy_variant == 2 && aligned && (P->n_proprio == 4) && (P->n_sparse % 2 == 0) && (P->n_dense % 2 == 0);
 }
 
 static int check_forward(const rvb_policy* P, const float* obs, int64_t obs_ld, const float* out, int64_t out_ld) {
@@ -937,8 +1007,9 @@ static int check_forward(const rvb_policy* P, const float* obs, int64_t obs_ld, 
 }
 
 // The tail kernel as a programmatic dependent of the first-layer kernel in front of it on `st`.
-static cudaError_t launch_tail_tc(dim3 grid, cudaStream_t st, const PolicyDev* a, const PolicyDev* b, const float* obs, int64_t obs_ld,
-                                  int64_t N, const float* h1, int nets, float* out0, int64_t out0_ld, float* out1, int64_t out1_ld) {
+static cudaError_t launch_tail_tc(dim3 grid, cudaStream_t st, const PolicyDev* a, const PolicyDev* b, const float* proprio,
+                                  int64_t proprio_ld, int64_t N, const float* h1, int nets, float* out0, int64_t out0_ld, float* out1,
+                                  int64_t out1_ld) {
     cudaLaunchConfig_t cfg = {};
     cfg.gridDim = grid;
     cfg.blockDim = dim3(TT_THREADS);
@@ -949,25 +1020,36 @@ static cudaError_t launch_tail_tc(dim3 grid, cudaStream_t st, const PolicyDev* a
     at[0].val.programmaticStreamSerializationAllowed = 1;
     cfg.attrs = at;
     cfg.numAttrs = 1;
-    return cudaLaunchKernelEx(&cfg, policy_tail_tc_kernel, a, b, obs, obs_ld, N, h1, nets, out0, out0_ld, out1, out1_ld);
+    return cudaLaunchKernelEx(&cfg, policy_tail_tc_kernel, a, b, proprio, proprio_ld, N, h1, nets, out0, out0_ld, out1, out1_ld);
 }
 
 // One network (B == nullptr) or two on the same observations (grid.y = network; the pair's first layers share the observation tiles).
-static int policy_launch(const rvb_policy* A, const rvb_policy* B, const float* obs, int64_t obs_ld, int64_t N,
+static int policy_launch(const rvb_policy* A, const rvb_policy* B, const PolicyIn& in, int64_t N,
                          float* out_a, int64_t out_a_ld, float* out_b, int64_t out_b_ld, cudaStream_t st) {
     RVB_REQUIRE(N <= (int64_t)PL_TM * 0x7fffffff, "rvb_policy_forward: too many envs");
     const int nets = B ? 2 : 1;
     const PolicyDev* db = B ? B->dev : nullptr;
     RvbTemp<float> h1;
-    if (tc_usable(A, obs, obs_ld)) {
+    if (tc_usable(A, in)) {
         RVB_CUDA(h1.alloc_pool((size_t)N * nets * 2 * PL_E1, st));
         const dim3 grid((unsigned)ceil_div(N, TC_M), 2);
-        if (B) policy_l1_tc_kernel<2><<<grid, TC_THREADS, tc_smem_bytes(2), st>>>(A->dev, db, obs, obs_ld, N, h1.p);
-        else policy_l1_tc_kernel<1><<<grid, TC_THREADS, tc_smem_bytes(1), st>>>(A->dev, db, obs, obs_ld, N, h1.p);
-        RVB_CUDA(launch_tail_tc(dim3((unsigned)ceil_div(N, TC_M), nets), st, A->dev, db, obs, obs_ld, N, h1.p, nets, out_a, out_a_ld, out_b, out_b_ld));
+        if (in.hm16) {
+            if (B) policy_l1_tc_h16_kernel<2><<<grid, TC_THREADS, tc_smem_bytes(2), st>>>(A->dev, db, in.hm16, in.hm_ld, N, h1.p);
+            else policy_l1_tc_h16_kernel<1><<<grid, TC_THREADS, tc_smem_bytes(1), st>>>(A->dev, db, in.hm16, in.hm_ld, N, h1.p);
+        } else {
+            if (B) policy_l1_tc_kernel<2><<<grid, TC_THREADS, tc_smem_bytes(2), st>>>(A->dev, db, in.proprio, in.proprio_ld, N, h1.p);
+            else policy_l1_tc_kernel<1><<<grid, TC_THREADS, tc_smem_bytes(1), st>>>(A->dev, db, in.proprio, in.proprio_ld, N, h1.p);
+        }
+        RVB_CUDA(launch_tail_tc(dim3((unsigned)ceil_div(N, TC_M), nets), st, A->dev, db, in.proprio, in.proprio_ld, N, h1.p, nets, out_a,
+                                out_a_ld, out_b, out_b_ld));
     } else {
-        policy_forward_kernel<<<dim3((unsigned)ceil_div(N, PL_TM), nets), PL_THREADS, PL_SMEM_BYTES, st>>>(A->dev, db, obs, obs_ld, N, out_a,
-                                                                                                       out_a_ld, out_b, out_b_ld);
+        const dim3 grid((unsigned)ceil_div(N, PL_TM), nets);
+        if (in.hm16)
+            policy_forward_h16_kernel<<<grid, PL_THREADS, PL_SMEM_BYTES, st>>>(A->dev, db, in.proprio, in.proprio_ld, in.hm16, in.hm_ld, N,
+                                                                               out_a, out_a_ld, out_b, out_b_ld);
+        else
+            policy_forward_kernel<<<grid, PL_THREADS, PL_SMEM_BYTES, st>>>(A->dev, db, in.proprio, in.proprio_ld, N, out_a, out_a_ld,
+                                                                           out_b, out_b_ld);
     }
     RVB_LAUNCH_CHECK();
     return RVB_OK;
@@ -979,7 +1061,7 @@ extern "C" int rvb_policy_forward(const rvb_policy* P, const float* obs, int64_t
     if (N <= 0) return RVB_OK;
     int rc;
     if ((rc = check_forward(P, obs, obs_ld, out, out_ld))) return rc;
-    return policy_launch(P, nullptr, obs, obs_ld, N, out, out_ld, nullptr, 0, as_stream(stream));
+    return policy_launch(P, nullptr, PolicyIn{obs, obs_ld, nullptr, 0}, N, out, out_ld, nullptr, 0, as_stream(stream));
 }
 
 extern "C" int rvb_policy_forward_pair(const rvb_policy* A, const rvb_policy* B, const float* obs, int64_t obs_ld, int64_t N,
@@ -993,5 +1075,36 @@ extern "C" int rvb_policy_forward_pair(const rvb_policy* A, const rvb_policy* B,
     RVB_REQUIRE(A->n_proprio == B->n_proprio && A->n_sparse == B->n_sparse && A->n_dense == B->n_dense,
                 "rvb_policy_forward_pair: the two networks read different observation splits");
     RVB_REQUIRE(A->act == B->act, "rvb_policy_forward_pair: the two networks use different activations");
-    return policy_launch(A, B, obs, obs_ld, N, out_a, out_a_ld, out_b, out_b_ld, as_stream(stream));
+    return policy_launch(A, B, PolicyIn{obs, obs_ld, nullptr, 0}, N, out_a, out_a_ld, out_b, out_b_ld, as_stream(stream));
+}
+
+static int check_packed(const rvb_policy* P, int64_t proprio_ld, int64_t heightmap_ld, int64_t out_ld) {
+    RVB_REQUIRE(proprio_ld >= P->n_proprio, "rvb_policy_forward_packed: proprio rows are shorter than the network's proprioceptive input");
+    RVB_REQUIRE(heightmap_ld >= (int64_t)P->n_sparse + P->n_dense,
+                "rvb_policy_forward_packed: heightmap rows are shorter than the network's sparse + dense input");
+    RVB_REQUIRE(out_ld >= P->n_head, "rvb_policy_forward_packed: out rows are shorter than the head");
+    int cur_dev = -1;
+    RVB_CUDA(cudaGetDevice(&cur_dev));
+    RVB_REQUIRE(P->device == cur_dev, "rvb_policy_forward_packed: the network lives on another device than the calling thread's current one");
+    return RVB_OK;
+}
+
+// The pointers are checked before the handle: every malformed call is refused before the handle is read.
+extern "C" int rvb_policy_forward_packed(const rvb_policy* A, const rvb_policy* B, const float* proprio, int64_t proprio_ld,
+                                         const uint16_t* heightmap, int64_t heightmap_ld, int64_t N, float* out_a, int64_t out_a_ld,
+                                         float* out_b, int64_t out_b_ld, void* stream) {
+    RVB_REQUIRE(N <= 0 || (proprio && heightmap && out_a && (!B || out_b)), "rvb_policy_forward_packed: null pointer");
+    RVB_REQUIRE(A, "rvb_policy_forward_packed: null handle");
+    if (N <= 0) return RVB_OK;
+    int rc;
+    if ((rc = check_packed(A, proprio_ld, heightmap_ld, out_a_ld))) return rc;
+    if (B) {
+        if ((rc = check_packed(B, proprio_ld, heightmap_ld, out_b_ld))) return rc;
+        RVB_REQUIRE(A->device == B->device, "rvb_policy_forward_packed: the two networks live on different devices");
+        RVB_REQUIRE(A->n_proprio == B->n_proprio && A->n_sparse == B->n_sparse && A->n_dense == B->n_dense,
+                    "rvb_policy_forward_packed: the two networks read different observation splits");
+        RVB_REQUIRE(A->act == B->act, "rvb_policy_forward_packed: the two networks use different activations");
+    }
+    return policy_launch(A, B, PolicyIn{proprio, proprio_ld, reinterpret_cast<const __half*>(heightmap), heightmap_ld}, N, out_a, out_a_ld,
+                         out_b, out_b_ld, as_stream(stream));
 }

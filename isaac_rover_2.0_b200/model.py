@@ -5,6 +5,9 @@ Same class names, constructor arguments and `compute()` results as `StochasticAc
 the reference's key names (`encoder0.encoder.0.layer.0.weight`, ..., `network.3.weight`, `log_std_parameter`), so a
 checkpoint of the reference's nn.Modules loads as is.  The forward pass is ONE kernel behind the C ABI
 (`rvb_policy_forward`, csrc/policy.cu); skrl's mixins (sampling, clipping, log-prob) are the learner's and stay outside.
+`states` is the f32 observation [N, >=p+S+D] or, from a step run in packed mode, the 2-tuple (proprio f32 [N, >=p],
+heightmap f16 [N, >=S+D]), e.g. `(task.obs_buf[:, :4], task.obs16_buf)`: same results bit for bit as on the widened rows, read
+without widening (`rvb_policy_forward_packed`).
 Inference only: there is no autograd through the kernel.
 """
 import ctypes as C
@@ -180,43 +183,77 @@ class _HeightmapNet:
 
     # ---- forward
     def _forward(self, states, out=None):
-        _lib.require_cuda(states)
-        if states.dim() != 2 or states.dtype != torch.float32 or states.shape[1] < self.num_observations:
-            raise RuntimeError("states must be float32 [N, >=%d]" % self.num_observations)
+        return _launch(self, None, states, out, None)[0]
+
+
+def _packed(states, nets):
+    """The packed form of `states`, (proprio, heightmap), checked against every network of `nets`; nothing is copied."""
+    p = max(n.num_proprioception for n in nets)
+    e = max(n.num_exteroceptive for n in nets)
+    form = ("packed states must be (proprio float32 [N, >=%d], heightmap float16 [N, >=%d]) on one device, each with unit column "
+            "stride" % (p, e))
+    if len(states) != 2 or not all(isinstance(t, torch.Tensor) for t in states):
+        raise RuntimeError(form)
+    proprio, heightmap = states
+    if (proprio.dim() != 2 or heightmap.dim() != 2 or proprio.dtype != torch.float32 or heightmap.dtype != torch.float16
+            or proprio.shape[0] != heightmap.shape[0] or proprio.shape[1] < p or heightmap.shape[1] < e
+            or proprio.stride(1) != 1 or heightmap.stride(1) != 1 or proprio.device != heightmap.device):
+        raise RuntimeError(form)
+    _lib.require_cuda(proprio, heightmap)
+    return proprio, heightmap
+
+
+def _row_stride(t):
+    return t.stride(0) if t.shape[0] > 1 else t.shape[1]     # a single row's stride is arbitrary in torch
+
+
+def _launch(a, b, states, out_a, out_b):
+    """Network a alone (b None) or the pair a, b on `states`: an f32 tensor [N, >=p+S+D] (rvb_policy_forward / _pair) or the packed
+    2-tuple (proprio f32 [N, >=p], heightmap f16 [N, >=S+D]) (rvb_policy_forward_packed)."""
+    nets = (a,) if b is None else (a, b)
+    packed = isinstance(states, tuple)
+    if packed:
+        proprio, heightmap = _packed(states, nets)
+        ref = proprio
+    else:
+        if isinstance(states, torch.Tensor):
+            _lib.require_cuda(states)
+        for net in nets:
+            if not isinstance(states, torch.Tensor) or states.dim() != 2 or states.dtype != torch.float32 or states.shape[1] < net.num_observations:
+                raise RuntimeError("states must be float32 [N, >=%d] or the packed 2-tuple (proprio float32 [N, >=%d], heightmap "
+                                   "float16 [N, >=%d])" % (net.num_observations, net.num_proprioception, net.num_exteroceptive))
         if states.stride(1) != 1:
             states = states.contiguous()
-        N = states.shape[0]
-        if out is None:
-            out = torch.empty((N, self._head_out), dtype=torch.float32, device=states.device)
-        if self.device.index is not None and states.device.index != self.device.index:
-            raise RuntimeError("states live on %s, the network on %s" % (states.device, self.device))
-        with torch.cuda.device(states.device):
-            _lib.check(self._lib.rvb_policy_forward(self._handle, _lib.ptr(states), states.stride(0), N, _lib.ptr(out), out.stride(0),
-                                                    _lib.stream_of(states)))
-        return out
+        ref = states
+    for net in nets:
+        if net.device.index is not None and ref.device.index != net.device.index:
+            raise RuntimeError("states live on %s, the network on %s" % (ref.device, net.device))
+    N = ref.shape[0]
+    if out_a is None:
+        out_a = torch.empty((N, a._head_out), dtype=torch.float32, device=ref.device)
+    if b is not None and out_b is None:
+        out_b = torch.empty((N, b._head_out), dtype=torch.float32, device=ref.device)
+    lib = a._lib
+    with torch.cuda.device(ref.device):
+        if packed:
+            _lib.check(lib.rvb_policy_forward_packed(a._handle, None if b is None else b._handle, _lib.ptr(proprio), _row_stride(proprio),
+                                                     _lib.ptr(heightmap), _row_stride(heightmap), N, _lib.ptr(out_a), out_a.stride(0),
+                                                     _lib.ptr(out_b), 0 if b is None else out_b.stride(0), _lib.stream_of(ref)))
+        elif b is None:
+            _lib.check(lib.rvb_policy_forward(a._handle, _lib.ptr(states), states.stride(0), N, _lib.ptr(out_a), out_a.stride(0),
+                                              _lib.stream_of(states)))
+        else:
+            _lib.check(lib.rvb_policy_forward_pair(a._handle, b._handle, _lib.ptr(states), states.stride(0), N, _lib.ptr(out_a),
+                                                   out_a.stride(0), _lib.ptr(out_b), out_b.stride(0), _lib.stream_of(states)))
+    return out_a, out_b
 
 
 def compute_pair(policy, value, states, out_policy=None, out_value=None):
     """`policy.compute(states)[0]` and `value.compute(states)` in ONE launch (rvb_policy_forward_pair): the two calls a PPO
-    step makes on the same states (skrl's agent.act + value.act on the reference's models_ppo, train.py:98-99)."""
-    _lib.require_cuda(states)
-    for net in (policy, value):
-        if states.dim() != 2 or states.dtype != torch.float32 or states.shape[1] < net.num_observations:
-            raise RuntimeError("states must be float32 [N, >=%d]" % net.num_observations)
-        if net.device.index is not None and states.device.index != net.device.index:
-            raise RuntimeError("states live on %s, the network on %s" % (states.device, net.device))
-    if states.stride(1) != 1:
-        states = states.contiguous()
-    N = states.shape[0]
-    if out_policy is None:
-        out_policy = torch.empty((N, policy._head_out), dtype=torch.float32, device=states.device)
-    if out_value is None:
-        out_value = torch.empty((N, value._head_out), dtype=torch.float32, device=states.device)
-    with torch.cuda.device(states.device):
-        _lib.check(policy._lib.rvb_policy_forward_pair(policy._handle, value._handle, _lib.ptr(states), states.stride(0), N,
-                                                       _lib.ptr(out_policy), out_policy.stride(0), _lib.ptr(out_value),
-                                                       out_value.stride(0), _lib.stream_of(states)))
-    return out_policy, out_value
+    step makes on the same states (skrl's agent.act + value.act on the reference's models_ppo, train.py:98-99).  `states` is the
+    f32 observation or the step's packed form `(task.obs_buf[:, :4], task.obs16_buf)` (rvb_policy_forward_packed), which gives
+    the same bits as its widened f32 rows without widening them."""
+    return _launch(policy, value, states, out_policy, out_value)
 
 
 class StochasticActorHeightmap(_HeightmapNet):
