@@ -122,11 +122,10 @@ static int launch_cast_simple(const rvb_terrain* t, const __half* src16, const _
     return RVB_OK;
 }
 
-extern "C" int rvb_heightmap_raycast(const rvb_terrain* t, const float* pos, const float* euler, const float* trig,
-                                     const double* pattern, int64_t P, int64_t N, uint16_t* dist, int32_t* hit_slot,
-                                     int32_t* hit_tri, uint16_t* pt, uint16_t* sources, float* obs, int64_t obs_ld,
-                                     uint16_t* obs_h16, int64_t obs_h16_ld, int obs_h16_col0, const int32_t* col_a,
-                                     const int32_t* col_b, int variant, void* stream) {
+int heightmap_raycast(const rvb_terrain* t, const float* pos, const float* euler, const float* trig, const double* pattern,
+                      int64_t P, int64_t N, uint16_t* dist, int32_t* hit_slot, int32_t* hit_tri, uint16_t* pt, uint16_t* sources,
+                      float* obs, int64_t obs_ld, uint16_t* obs_h16, int64_t obs_h16_ld, int obs_h16_col0, const int32_t* col_a,
+                      const int32_t* col_b, int variant, const RaycastKnobs& knobs, const int32_t* order, cudaStream_t st) {
     RVB_REQUIRE(N >= 0 && P > 0 && P <= 65535, "rvb_heightmap_raycast: need N >= 0, 0 < P <= 65535");
     if (N == 0) return RVB_OK;
     RVB_REQUIRE(t && pos && euler && pattern && dist, "rvb_heightmap_raycast: null pointer");
@@ -135,10 +134,6 @@ extern "C" int rvb_heightmap_raycast(const rvb_terrain* t, const float* pos, con
     RVB_REQUIRE(variant >= 0 && variant <= 3, "rvb_heightmap_raycast: variant must be 0, 1, 2 or 3");
     RVB_REQUIRE(!obs_h16 || variant != 1, "rvb_heightmap_raycast: the per-pair cross-check kernel (variant 1) has no packed output");
     RVB_REQUIRE(variant != 2 || t->index != nullptr, "rvb_heightmap_raycast: variant 2 reads the index the layer released (rvb_terrain_release_index)");
-    RaycastKnobs knobs;
-    const int krc = read_raycast_knobs(knobs);
-    if (krc != RVB_OK) return krc;
-    cudaStream_t st = as_stream(stream);
     if (variant != 1) {
         rc::TiledParams q;
         const int frc = fill_tiled_params(t, pos, euler, trig, pattern, P, N, dist, hit_slot, hit_tri, pt, sources, obs, obs_ld,
@@ -146,7 +141,7 @@ extern "C" int rvb_heightmap_raycast(const rvb_terrain* t, const float* pos, con
         if (frc != RVB_OK) return frc;
         // a layer with more than 2 % of triangles the shadow kernel has no bound for (terrain.cu: n_ill): the tiled kernel is the faster one
         const bool shadow_ok = knobs.force >= 0 ? knobs.force == 1 : t->n_ill * 50 <= t->T;
-        if (variant == 0 && t->sb_ids != nullptr && shadow_ok) return launch_shadow(q, N, knobs, st);
+        if (variant == 0 && t->sb_ids != nullptr && shadow_ok) return launch_shadow(q, N, knobs, order, st);
         return launch_tiled(q, t->blk_ids != nullptr && variant != 2, N * q.tiles, st);
     }
     RVB_REQUIRE(t->index != nullptr, "rvb_heightmap_raycast: variant 1 reads the index the layer released (rvb_terrain_release_index)");
@@ -160,6 +155,18 @@ extern "C" int rvb_heightmap_raycast(const rvb_terrain* t, const float* pos, con
     hm_setup_kernel<<<grid, 256, 0, st>>>(pos, euler, trig, pattern, (int)P, src16, dneg);
     RVB_LAUNCH_CHECK();
     return launch_cast_simple(t, src16, dneg, N * P, P, dist, hit_slot, hit_tri, pt, obs, obs_ld, col_a, col_b, st);
+}
+
+extern "C" int rvb_heightmap_raycast(const rvb_terrain* t, const float* pos, const float* euler, const float* trig,
+                                     const double* pattern, int64_t P, int64_t N, uint16_t* dist, int32_t* hit_slot,
+                                     int32_t* hit_tri, uint16_t* pt, uint16_t* sources, float* obs, int64_t obs_ld,
+                                     uint16_t* obs_h16, int64_t obs_h16_ld, int obs_h16_col0, const int32_t* col_a,
+                                     const int32_t* col_b, int variant, void* stream) {
+    RaycastKnobs knobs;
+    const int krc = read_raycast_knobs(knobs);
+    if (krc != RVB_OK) return krc;
+    return heightmap_raycast(t, pos, euler, trig, pattern, P, N, dist, hit_slot, hit_tri, pt, sources, obs, obs_ld, obs_h16,
+                             obs_h16_ld, obs_h16_col0, col_a, col_b, variant, knobs, nullptr, as_stream(stream));
 }
 
 extern "C" int rvb_cast_rays(const rvb_terrain* t, const uint16_t* sources, const uint16_t* directions, int64_t R,

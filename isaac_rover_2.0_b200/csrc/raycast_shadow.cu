@@ -39,6 +39,8 @@
 #include <stdlib.h>
 #include <string.h>
 
+#include <cub/device/device_radix_sort.cuh>
+
 #include "raycast_common.cuh"
 #include "shadow_bounds.cuh"
 
@@ -169,22 +171,40 @@ __device__ __forceinline__ void stage2(const TriF& t, const uint2& q1, const Env
 
 __device__ __forceinline__ bool is_steep(const H3& d16, float cos_steep) { return !(fabsf(__half2float(d16.z)) >= cos_steep); }
 
-// One thread per env: the ray direction as the kernels compute it -> steep envs onto the tiled kernel's work list (every tile),
-// and the env order of the shadow kernel: tilted envs (long shadows = slow CTAs) from the front, the rest from the back.
-__global__ void hm_classify_kernel(const TiledParams q, int64_t N, int32_t* __restrict__ order, int* __restrict__ counters,
-                                   int32_t* __restrict__ steep_list) {
+constexpr int ORDER_SH = 3;          // the env order's map cells: 2^3 x 2^3 index cells (0.8 m at the reference's 0.1 m)
+
+// v's low 16 bits spread to the even bits
+__device__ __forceinline__ uint32_t spread_bits(uint32_t v) {
+    v &= 0xffffu;
+    v = (v | (v << 8)) & 0x00ff00ffu;
+    v = (v | (v << 4)) & 0x0f0f0f0fu;
+    v = (v | (v << 2)) & 0x33333333u;
+    return (v | (v << 1)) & 0x55555555u;
+}
+
+// One thread per env: the ray direction as the kernels compute it -> steep envs onto the tiled kernel's work list (every tile,
+// with `steep_list`), and (with `keys`) the env's key of the order the shadow and rock kernels cast envs in: tilted envs (long
+// shadows = slow CTAs) first, then the rest; within each class the Z-order code of the env's map cell, so that the CTAs resident
+// at one time read the candidate lists, records and slot table of one small patch of the map, from L2.
+__global__ void hm_classify_kernel(const TiledParams q, int64_t N, int zbits, uint32_t* __restrict__ keys, int32_t* __restrict__ ids,
+                                   int* __restrict__ steep_count, int32_t* __restrict__ steep_list) {
     const int64_t n = blockIdx.x * (int64_t)blockDim.x + threadIdx.x;
     if (n >= N) return;
+    const float px = q.pos[n * 3 + 0], py = q.pos[n * 3 + 1];
     const Trig tr = make_trig(q.euler, q.trig, n);
-    const H3 d16 = env_dir16(tr, (double)q.pos[n * 3 + 0], (double)q.pos[n * 3 + 1], (double)q.pos[n * 3 + 2]);
+    const H3 d16 = env_dir16(tr, (double)px, (double)py, (double)q.pos[n * 3 + 2]);
     const bool steep = is_steep(d16, q.cos_steep);
-    if (steep) {
-        const int at = atomicAdd(counters + 0, q.tiles);
+    if (steep && steep_list) {
+        const int at = atomicAdd(steep_count, q.tiles);
         for (int t = 0; t < q.tiles; ++t) steep_list[at + t] = (int32_t)(n * q.tiles + t);
     }
-    const bool tilted = !steep && !(fabsf(__half2float(d16.z)) >= 0.97f);
-    if (tilted) order[atomicAdd(counters + 1, 1)] = (int32_t)n;
-    else order[N - 1 - atomicAdd(counters + 2, 1)] = (int32_t)n;
+    if (keys) {
+        const bool tilted = !steep && !(fabsf(__half2float(d16.z)) >= 0.97f);
+        const uint32_t cx = (uint32_t)cell_coord_f(px, q.shift_x, q.res, q.inv_res, q.G0 - 1, q.sem) >> ORDER_SH;
+        const uint32_t cy = (uint32_t)min(cell_coord_f(py, q.shift_y, q.res, q.inv_res, q.G0 - 1, q.sem), q.G1 - 1) >> ORDER_SH;
+        keys[n] = ((tilted ? 0u : 1u) << (2 * zbits)) | spread_bits(cx) << 1 | spread_bits(cy);
+        ids[n] = (int32_t)n;
+    }
 }
 
 template <bool DBGK, int RTC>
@@ -934,7 +954,42 @@ static int launch_tiled_list(rc::TiledParams q, const int* count, const int32_t*
     return launch_tiled(q, true, grid, st);
 }
 
-int launch_shadow(rc::TiledParams q, int64_t N, const RaycastKnobs& knobs, cudaStream_t st) {
+// The env order of q's N envs into order[N] (hm_classify_kernel's keys, stable radix sort: equal keys keep index order); with
+// steep_list, the same launch also puts the steep envs on it.  q needs the poses, the grid and cos_steep.
+static int sort_envs(const rc::TiledParams& q, int64_t N, int32_t* order, int* steep_count, int32_t* steep_list, cudaStream_t st) {
+    RVB_REQUIRE(N < ((int64_t)1 << 31), "env order: more than 2^31 - 1 envs");
+    int zbits = 0;          // bits per axis of the Z-order code: enough for the layer's grid, no more (fewer radix passes)
+    while ((((int64_t)max(q.G0, q.G1) - 1) >> ORDER_SH) >> zbits) ++zbits;
+    // the class bit and two zbits-bit coordinates in a 32-bit key
+    RVB_REQUIRE(zbits <= 15, "env order: grid wider than 2^18 cells");
+    const int key_bits = 2 * zbits + 1;
+    RvbTemp<uint32_t> keys;           // [2N]  keys, sorted keys
+    RvbTemp<int32_t> ids;
+    RVB_CUDA(keys.alloc_pool(2 * (size_t)N, st));
+    RVB_CUDA(ids.alloc_pool((size_t)N, st));
+    hm_classify_kernel<<<(unsigned)ceil_div(N, 256), 256, 0, st>>>(q, N, zbits, keys.p, ids.p, steep_count, steep_list);
+    RVB_LAUNCH_CHECK();
+    size_t bytes = 0;
+    RVB_CUDA(cub::DeviceRadixSort::SortPairs(nullptr, bytes, keys.p, keys.p + N, ids.p, order, (int)N, 0, key_bits, st));
+    RvbTemp<unsigned char> tmp;
+    RVB_CUDA(tmp.alloc_pool(bytes, st));
+    RVB_CUDA(cub::DeviceRadixSort::SortPairs(tmp.p, bytes, keys.p, keys.p + N, ids.p, order, (int)N, 0, key_bits, st));
+    return RVB_OK;
+}
+
+int build_env_order(const rvb_terrain* t, const float* pos, const float* euler, const float* trig, int64_t N, float cos_steep,
+                    int32_t* order, cudaStream_t st) {
+    RVB_REQUIRE(t && t->G0 >= 1 && t->G1 >= 1 && t->G0 <= (1 << 18) && t->G1 <= (1 << 18), "env order: grid wider than 2^18 cells");
+    rc::TiledParams q;
+    memset(&q, 0, sizeof(q));
+    q.G0 = (int)t->G0; q.G1 = (int)t->G1;
+    q.res = t->res; q.inv_res = 1.0f / t->res; q.shift_x = t->shift_x; q.shift_y = t->shift_y; q.sem = t->sem;
+    q.pos = pos; q.euler = euler; q.trig = trig;
+    q.cos_steep = cos_steep;
+    return sort_envs(q, N, order, nullptr, nullptr, st);
+}
+
+int launch_shadow(rc::TiledParams q, int64_t N, const RaycastKnobs& knobs, const int32_t* order, cudaStream_t st) {
     RVB_REQUIRE(q.sb_ids != nullptr && q.sb_slot9 != nullptr && q.sb_chunk != nullptr && q.blk_ids != nullptr && q.s1 != nullptr,
                 "heightmap ray-cast (shadow): layer has no block lists");
     RVB_REQUIRE(q.tile_size <= 2048, "heightmap ray-cast (shadow): tile larger than 2048 rays");
@@ -951,21 +1006,19 @@ int launch_shadow(rc::TiledParams q, int64_t N, const RaycastKnobs& knobs, cudaS
             nblocks = N + nsplit;
         }
     }
-    // scratch: with RVB_SHADOW_DBG=1 the kernel's 24 counters (8 bytes each) first; then [0] steep count, [1] tilted envs placed,
-    // [2] other envs placed, [3] handed-back count, the steep list [nblocks], the hand-back list [nblocks] and the env order [N]
+    // scratch: with RVB_SHADOW_DBG=1 the kernel's 24 counters (8 bytes each) first; then [0] steep count, [1] handed-back count,
+    // the steep list [nblocks], the hand-back list [nblocks] and, without the caller's, the env order [N]
     const int64_t ndbg = knobs.dbg ? 2 * 24 : 0;          // in ints
     // The scratch is declared BEFORE the join guard: destructors run in reverse order, so st first waits for the side stream's
     // tiled kernel, which reads the steep list and the counters, and only then gives the scratch back to the pool.
     RvbTemp<int> scratch;
     RvbJoinGuard guard(st);
-    RVB_CUDA(scratch.alloc_pool((size_t)(ndbg + 4 + 2 * nblocks + N), st));
-    RVB_CUDA(cudaMemsetAsync(scratch.p, 0, sizeof(int) * (size_t)(ndbg + 4), st));
+    RVB_CUDA(scratch.alloc_pool((size_t)(ndbg + 2 + 2 * nblocks + (order ? 0 : N)), st));
+    RVB_CUDA(cudaMemsetAsync(scratch.p, 0, sizeof(int) * (size_t)(ndbg + 2), st));
     int* const counts = scratch.p + ndbg;
-    int32_t* steep_list = counts + 4;
-    q.fb_count = counts + 3;
-    q.fb_list = counts + 4 + nblocks;
-    int32_t* order = counts + 4 + 2 * nblocks;
-    q.order = order;
+    int32_t* steep_list = counts + 2;
+    q.fb_count = counts + 1;
+    q.fb_list = counts + 2 + nblocks;
     q.cos_steep = knobs.cos_steep;
     q.min_sh = knobs.min_sh;
     q.task_rays = knobs.task_rays;
@@ -977,7 +1030,18 @@ int launch_shadow(rc::TiledParams q, int64_t N, const RaycastKnobs& knobs, cudaS
     if (lrc != RVB_OK) return lrc;
     RvbSide* side = nullptr;
     RVB_CUDA(rvb_side_stream(1, &side));
-    hm_classify_kernel<<<(unsigned)ceil_div(N, 256), 256, 0, st>>>(q, N, order, counts, steep_list);
+    if (order) {
+        // the caller's order (the fused step builds one for the ray-cast and the rock kernel): this launch only makes the steep
+        // list, whose slots depend on this call's tiling (it recomputes every env's ray direction, one thread per env)
+        hm_classify_kernel<<<(unsigned)ceil_div(N, 256), 256, 0, st>>>(q, N, 0, nullptr, nullptr, counts, steep_list);
+        RVB_LAUNCH_CHECK();
+        q.order = order;
+    } else {
+        int32_t* own = counts + 2 + 2 * nblocks;
+        const int orc = sort_envs(q, N, own, counts, steep_list, st);
+        if (orc != RVB_OK) return orc;
+        q.order = own;
+    }
     // steep envs: the tiled kernel on the second stream, concurrently with the shadow kernel
     const int64_t tgrid = nblocks < 148 * 3 ? nblocks : 148 * 3;
     RVB_CUDA(cudaEventRecord(side->fork, st));

@@ -57,22 +57,12 @@ extern "C" int rvb_env_step(const rvb_terrain* terrain, const rvb_terrain* rocks
     RVB_REQUIRE(!io.obs_h16 || io.obs_h16_ld > 0, "rvb_env_step: obs_h16 needs obs_h16_ld");
     RVB_REQUIRE(p->curriculum_level < 2 || (rocks && io.wheel_dist && io.body_dist && io.rock_collision),
                 "rvb_env_step: curriculum_level >= 2 needs the rock layer and its outputs");
+    RaycastKnobs knobs;
+    const int krc = read_raycast_knobs(knobs);
+    if (krc != RVB_OK) return krc;
     cudaStream_t st = as_stream(stream);
     step_pre_kernel<<<(unsigned)ceil_div(N, 256), 256, 0, st>>>(io, N, (int)H, p->sem);
     RVB_LAUNCH_CHECK();
-    const bool with_rocks = rocks && io.wheel_dist && io.body_dist;
-    RvbJoinGuard guard(st);          // on every exit path below: st waits for the rock layer's kernel
-    if (with_rocks) {
-        RvbSide* side = nullptr;
-        RVB_CUDA(rvb_side_stream(0, &side));
-        RVB_CUDA(cudaEventRecord(side->fork, st));
-        RVB_CUDA(cudaStreamWaitEvent(side->s, side->fork, 0));
-        const int rc = rvb_rock_collision(rocks, io.pos, io.euler, nullptr, io.joints, nullptr, N, io.wheel_dist, io.body_dist,
-                                          nullptr, io.rock_collision, nullptr, side->s);
-        if (rc != RVB_OK) return rc;
-        RVB_CUDA(cudaEventRecord(side->join, side->s));
-        guard.join = side->join;
-    }
     cudaEvent_t t0 = nullptr, t1 = nullptr;
     if (g_timing.on) {
         if (g_timing.used + 2 > g_timing.ev.size()) {
@@ -85,12 +75,32 @@ extern "C" int rvb_env_step(const rvb_terrain* terrain, const rvb_terrain* rocks
         t0 = g_timing.ev[g_timing.used];
         t1 = g_timing.ev[g_timing.used + 1];
         g_timing.used += 2;
+        // the timed ray-cast includes its env order, as a standalone rvb_heightmap_raycast (which builds the order inside) does
         RVB_CUDA(cudaEventRecord(t0, st));
+    }
+    // one env order (from this step's euler) for the ray-cast and the rock kernel; declared before the join guard, so that st
+    // waits for the rock kernel before the order goes back to the pool
+    RvbTemp<int32_t> order;
+    RVB_CUDA(order.alloc_pool((size_t)N, st));
+    const int orc = build_env_order(terrain, io.pos, io.euler, nullptr, N, knobs.cos_steep, order.p, st);
+    if (orc != RVB_OK) return orc;
+    const bool with_rocks = rocks && io.wheel_dist && io.body_dist;
+    RvbJoinGuard guard(st);          // on every exit path below: st waits for the rock layer's kernel
+    if (with_rocks) {
+        RvbSide* side = nullptr;
+        RVB_CUDA(rvb_side_stream(0, &side));
+        RVB_CUDA(cudaEventRecord(side->fork, st));
+        RVB_CUDA(cudaStreamWaitEvent(side->s, side->fork, 0));
+        const int rc = rock_collision(rocks, io.pos, io.euler, nullptr, io.joints, nullptr, N, io.wheel_dist, io.body_dist, nullptr,
+                                      io.rock_collision, nullptr, order.p, side->s);
+        if (rc != RVB_OK) return rc;
+        RVB_CUDA(cudaEventRecord(side->join, side->s));
+        guard.join = side->join;
     }
     // packed observation requested: the heightmap columns go to obs_h16 (fp16, what they are by construction) and the f32
     // columns 4.. of obs are left alone
-    int rc = rvb_heightmap_raycast(terrain, io.pos, io.euler, nullptr, pattern, P, N, io.dist, nullptr, nullptr, nullptr, nullptr,
-                                   io.obs_h16 ? nullptr : io.obs, io.obs_ld, io.obs_h16, io.obs_h16_ld, 4, col_a, col_b, 0, st);
+    int rc = heightmap_raycast(terrain, io.pos, io.euler, nullptr, pattern, P, N, io.dist, nullptr, nullptr, nullptr, nullptr,
+                               io.obs_h16 ? nullptr : io.obs, io.obs_ld, io.obs_h16, io.obs_h16_ld, 4, col_a, col_b, 0, knobs, order.p, st);
     if (rc != RVB_OK) return rc;
     if (t1) RVB_CUDA(cudaEventRecord(t1, st));
     if (guard.join) {
