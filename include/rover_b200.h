@@ -218,7 +218,26 @@ int rvb_env_step(const rvb_terrain* terrain, const rvb_terrain* rocks, const rvb
                  const double* pattern, int64_t P, const int32_t* col_a, const int32_t* col_b, int64_t N, int64_t H,
                  void* stream);
 
-/* Device timing of the heightmap ray-cast inside rvb_env_step (CUDA events on the caller's stream, calling thread only):
+/* The same step split at the simulator's boundary, for the loop this library is built into:
+ *   obs_t -> policy -> pre_physics_step(a_t) -> simulator steps -> post_physics_step() -> obs_{t+1}.
+ * rvb_env_pre is the action half of RoverTask.pre_physics_step (rover.py:338-414) on the PRE-physics pose: rover_rot =
+ * tensor_quat_to_eul(quat) (rover.py:343; is_done reads it one post half later, :615-616), Memory.input_state x2 (:379-380,389),
+ * Ackermann + joint targets (:391,400-409).  One launch.  It reads no goal, progress or reset state, so it may run before or
+ * after the reset half of pre_physics_step.
+ *   quat f32 [N,4] (16-byte aligned)  actions f32 [N,2]  lin_hist/ang_hist f32 [N,H] (shifted in place)  rover_rot f32 [N,3]
+ *   steer/vel [N,6], pos_targets [N,4], vel_targets [N,6] optional.
+ * rvb_env_post is RLTask.post_physics_step (rl_task.py:239-259) on the POST-physics poses in io: progress += 1, get_observations
+ * (euler -> io.euler, heading, proprioceptive columns with this step's action read from lin_hist/ang_hist[:, 0], heightmap
+ * ray-cast into obs or obs_h16, rock layer on the forked stream), calculate_metrics + is_done with the rover_rot of rvb_env_pre.
+ * io as rvb_env_step; io.actions, steer, vel, pos_targets and vel_targets are not read and may be NULL.  Same kernels as
+ * rvb_env_step after its first one, so for an unchanged pose the pair gives rvb_env_step's results bit for bit. */
+int rvb_env_pre(const float* quat, const float* actions, int64_t N, int64_t H, float* lin_hist, float* ang_hist,
+                float* rover_rot, float* steer, float* vel, float* pos_targets, float* vel_targets, int sem, void* stream);
+int rvb_env_post(const rvb_terrain* terrain, const rvb_terrain* rocks, const rvb_reward_params* p, const rvb_step_io* io,
+                 const float* rover_rot, const double* pattern, int64_t P, const int32_t* col_a, const int32_t* col_b,
+                 int64_t N, int64_t H, void* stream);
+
+/* Device timing of the heightmap ray-cast inside rvb_env_step and rvb_env_post (CUDA events on the caller's stream, calling thread only):
  * enable, run steps, then read the per-step durations in ms (host array; returns the count or <0; synchronises). */
 int rvb_timing_enable(int on);
 int rvb_timing_read(float* ms_host, int cap);

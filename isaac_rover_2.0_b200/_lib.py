@@ -68,6 +68,8 @@ _SIGNATURES = {
     "rvb_stats_scratch_len": (i64, [i64]),
     "rvb_reward_reset": (C.c_int, [C.POINTER(RewardParams)] + [p] * 11 + [i64] + [p] * 10 + [p]),
     "rvb_env_step": (C.c_int, [p, p, C.POINTER(RewardParams), C.POINTER(StepIO), p, i64, p, p, i64, i64, p]),
+    "rvb_env_pre": (C.c_int, [p, p, i64, i64, p, p, p, p, p, p, p, C.c_int, p]),
+    "rvb_env_post": (C.c_int, [p, p, C.POINTER(RewardParams), C.POINTER(StepIO), p, p, i64, p, p, i64, i64, p]),
     "rvb_timing_enable": (C.c_int, [C.c_int]),
     "rvb_timing_read": (C.c_int, [C.POINTER(f32), C.c_int]),
     "rvb_stone_validate": (C.c_int, [p, i64, i64, p, i64, f32, C.c_int, p, p, p, p]),
@@ -99,6 +101,7 @@ def lib_path():
 KERNELS_PER_CALL = {"rvb_terrain_create": 2, "rvb_heightmap_raycast": 4, "rvb_cast_rays": 2, "rvb_ray_distance": 1,
                     "rvb_rock_collision": 1, "rvb_check_collision": 1, "rvb_quat_to_euler": 1, "rvb_ackermann": 1,
                     "rvb_history_push": 1, "rvb_obs_proprio": 1, "rvb_obs_gather": 1, "rvb_reward_reset": 2, "rvb_env_step": 8,
+                    "rvb_env_pre": 1, "rvb_env_post": 8,
     "rvb_stone_validate": 1, "rvb_spawn_validate": 1, "rvb_height_lookup": 1, "rvb_build_knn_index": 6, "rvb_reset_targets": 1,
                     "rvb_policy_create": 7, "rvb_policy_forward": 1, "rvb_policy_forward_pair": 1,
                     "rvb_policy_forward_packed": 2,

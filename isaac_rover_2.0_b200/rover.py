@@ -30,6 +30,11 @@ STAT_NAMES = ("envs", "reward_sum", "pos_reward_sum", "collisions", "uprightness
               "goals_reached", "collision_resets", "target_dist_sum", "reserved")
 
 
+def _f32(t):
+    """t as a contiguous f32 tensor (itself when it already is one)."""
+    return t if (t.dtype == torch.float32 and t.is_contiguous()) else t.to(torch.float32).contiguous()
+
+
 class Memory():
     """[num_envs, num_states, horizon] shift register, newest at index 0 (rover.py:60-77).  The shift is done
     in place by rvb_history_push instead of cat + slice re-allocation."""
@@ -222,64 +227,141 @@ class RoverTask():
         return self.post_physics_step()
 
     def _hot_step_fused(self, actions):
-        N, dev = self.num_envs, torch.device(self._device)
         pos, quat = self._rover.get_world_poses()
         joints = self._rover.get_joint_positions()
-        f32 = torch.float32
-        pos = pos if (pos.dtype == f32 and pos.is_contiguous()) else pos.to(f32).contiguous()
-        quat = quat if (quat.dtype == f32 and quat.is_contiguous()) else quat.to(f32).contiguous()
-        joints = joints if (joints.dtype == f32 and joints.is_contiguous()) else joints.to(f32).contiguous()
-        act = actions if (actions.dtype == f32 and actions.is_contiguous() and actions.device == dev) else actions.to(dev, f32).contiguous()
+        pos, quat, joints = _f32(pos), _f32(quat), _f32(joints)
+        act = self._actions_f32(actions)
         _lib.require_cuda(pos, quat, joints, act)
-        if self.obs_hooks is not None and self.obs16_buf is not None:
-            raise RuntimeError("hot_step: observation hooks work on obs_buf (f32); they cannot be combined with the packed "
-                               "fp16 observation output (obs16_buf)")
+        self._refuse_hooks_with_obs16("hot_step")
         if self.save_teacher_data:                                  # rover.py:373-375, then :298-317 BEFORE obs_buf is refreshed
             self._teacher_actions = act[:, 0:2]
             if self.teacher_recorder is not None:
                 self.teacher_recorder.record(self.reset_info, self._teacher_actions, self.obs_buf)
+        fb = self._step_buffers()
+        want_rocks = self.curriculum_level >= 2
+        io = self._step_io(pos, quat, joints, act, fb["pos_t"], fb["vel_t"], want_rocks)
+        prm = self._params()
+        cam = self.Camera
+        with torch.cuda.device(torch.device(self._device)):
+            _lib.check(self._lib.rvb_env_step(cam.layer.handle, self.Rock_detector.layer.handle if want_rocks else None,
+                                              C.byref(prm), C.byref(io), _lib.ptr(cam.heightmap_distribution), self.num_exteroceptive,
+                                              _lib.ptr(cam._col_a), _lib.ptr(cam._col_b), self.num_envs, self.linear_velocity.horizon,
+                                              self._stream()))
+        self._after_post(pos, want_rocks)
+        self.rover_rot = fb["euler"]
+        self._hand_targets(fb["pos_t"], fb["vel_t"])
+        return self.obs_buf, self.rew_buf, self.reset_buf, self.extras
+
+    # ------------------------------------------------------------------ the fused step split at the simulator's boundary
+    def pre_physics_step_fused(self, actions, max_attempts=64) -> None:
+        """pre_physics_step_device (rover.py:338-414, reset path on the device) for a loop in which the simulator steps between
+        the halves: the action half is ONE launch (rvb_env_pre) instead of four, rover_rot is the euler of the pose the view holds
+        now.  Same side effects as pre_physics_step_device."""
+        self.global_step += 1
+        self.rover_loc, quat = self._rover.get_world_poses()
+        quat = _f32(quat)
+        act = self._actions_f32(actions)
+        _lib.require_cuda(quat, act)
+        if self.save_teacher_data:                                  # rover.py:373-375
+            self._teacher_actions = act[:, 0:2]
+        fb = self._step_buffers()
+        # The action half is enqueued BEFORE the reset half, so rover_rot is the pose before the simulator's pose reset, as
+        # rover.py:343 takes it before :356.  Moving it ahead changes nothing else: the reset half writes goal targets, progress,
+        # reset flags and reset_info, none of which the action half (histories, steering, wheel velocities) reads or writes.
+        with torch.cuda.device(torch.device(self._device)):
+            _lib.check(self._lib.rvb_env_pre(_lib.ptr(quat), _lib.ptr(act), self.num_envs, self.linear_velocity.horizon,
+                                             _lib.ptr(self.linear_velocity.tracker), _lib.ptr(self.angular_velocity.tracker),
+                                             _lib.ptr(fb["rot"]), None, None, _lib.ptr(fb["pos_t"]), _lib.ptr(fb["vel_t"]), self.sem,
+                                             self._stream()))
+        self.rover_rot = fb["rot"]
+        self._mark_reset_info()
+        if hasattr(self._rover, "reset_idx_masked"):
+            self._rover.reset_idx_masked(self.reset_buf.clone(), self.initial_pos)
+        self.reset_targets_device(max_attempts=max_attempts)
+        self._hand_targets(fb["pos_t"], fb["vel_t"])               # after the resets, as apply_actions does
+
+    def post_physics_step_fused(self):
+        """post_physics_step (rl_task.py:239-259) after pre_physics_step_fused and the simulator's step: ONE library call
+        (rvb_env_post) on the poses and joints the view holds now, is_done on the rover_rot of the pre half.  Honours obs16_buf
+        like hot_step (then obs_buf[:, 4:] is not written)."""
+        if not self._is_playing():                                  # rl_task.py:241 comes before the guard at :250
+            self.progress_buf[:] += 1
+            return self.obs_buf, self.rew_buf, self.reset_buf, self.extras
+        pos, quat = self._rover.get_world_poses()
+        joints = self._rover.get_joint_positions()
+        pos, quat, joints = _f32(pos), _f32(quat), _f32(joints)
+        _lib.require_cuda(pos, quat, joints)
+        self._refuse_hooks_with_obs16("post_physics_step_fused")
+        if self.rover_rot is None:
+            raise RuntimeError("post_physics_step_fused: no rover_rot; the pre-physics half has not run")
+        self._step_buffers()
+        if self.save_teacher_data and self.teacher_recorder is not None:       # rover.py:298-317: BEFORE obs_buf is refreshed
+            self.teacher_recorder.record(self.reset_info, self._teacher_actions, self.obs_buf)
+        want_rocks = self.curriculum_level >= 2
+        io = self._step_io(pos, quat, joints, None, None, None, want_rocks)
+        prm = self._params()
+        cam = self.Camera
+        with torch.cuda.device(torch.device(self._device)):
+            _lib.check(self._lib.rvb_env_post(cam.layer.handle, self.Rock_detector.layer.handle if want_rocks else None,
+                                              C.byref(prm), C.byref(io), _lib.ptr(self.rover_rot), _lib.ptr(cam.heightmap_distribution),
+                                              self.num_exteroceptive, _lib.ptr(cam._col_a), _lib.ptr(cam._col_b), self.num_envs,
+                                              self.linear_velocity.horizon, self._stream()))
+        self._after_post(pos, want_rocks)
+        return self.obs_buf, self.rew_buf, self.reset_buf, self.extras
+
+    def _actions_f32(self, actions):
+        dev = torch.device(self._device)
+        ok = actions.dtype == torch.float32 and actions.is_contiguous() and actions.device == dev
+        return actions if ok else actions.to(dev, torch.float32).contiguous()
+
+    def _refuse_hooks_with_obs16(self, who):
+        if self.obs_hooks is not None and self.obs16_buf is not None:
+            raise RuntimeError("%s: observation hooks work on obs_buf (f32); they cannot be combined with the packed "
+                               "fp16 observation output (obs16_buf)" % who)
+
+    def _step_buffers(self):
+        """Device outputs of the fused step and its halves that have no attribute of the reference's (allocated once)."""
         if self._fused is None:
-            P = self.num_exteroceptive
+            N, P, dev = self.num_envs, self.num_exteroceptive, torch.device(self._device)
             self._fused = dict(
                 euler=torch.empty((N, 3), device=dev), dist=torch.empty((N, P), device=dev, dtype=torch.float16),
                 wheel=torch.empty((N, 24), device=dev, dtype=torch.float16), body=torch.empty((N, 2), device=dev, dtype=torch.float16),
-                pos_t=torch.empty((N, 4), device=dev), vel_t=torch.empty((N, 6), device=dev))
+                pos_t=torch.empty((N, 4), device=dev), vel_t=torch.empty((N, 6), device=dev), rot=torch.empty((N, 3), device=dev))
+        return self._fused
+
+    def _step_io(self, pos, quat, joints, act, pos_t, vel_t, want_rocks):
         fb = self._fused
-        want_rocks = self.curriculum_level >= 2
         e = self._ex
-        io = _lib.StepIO(*[_lib.ptr(t) for t in (pos, quat, joints, act, self.target_positions, self.linear_velocity.tracker,
-                                                  self.angular_velocity.tracker, self.progress_buf, fb["euler"], self.heading_diff,
-                                                  None, None, fb["pos_t"], fb["vel_t"], self.obs_buf)],
-                         self.obs_buf.stride(0),
-                         *[_lib.ptr(t) for t in (fb["dist"], fb["wheel"] if want_rocks else None, fb["body"] if want_rocks else None,
-                                                  self.rock_collison if want_rocks else None, self.rew_buf, self.reset_buf,
-                                                  e["pos_reward"], e["collision_penalty"], e["uprightness_penalty"],
-                                                  e["heading_contraint_penalty"], e["motion_contraint_penalty"],
-                                                  e["goal_angle_penalty"], self.stats, self._stats_scratch, self.obs16_buf)],
-                         0 if self.obs16_buf is None else self.obs16_buf.stride(0))
-        prm = self._params()
-        cam = self.Camera
-        with torch.cuda.device(dev):
-            _lib.check(self._lib.rvb_env_step(cam.layer.handle, self.Rock_detector.layer.handle if want_rocks else None,
-                                              C.byref(prm), C.byref(io), _lib.ptr(cam.heightmap_distribution), self.num_exteroceptive,
-                                              _lib.ptr(cam._col_a), _lib.ptr(cam._col_b), N, self.linear_velocity.horizon,
-                                              self._stream()))
-        if not want_rocks:
+        return _lib.StepIO(*[_lib.ptr(t) for t in (pos, quat, joints, act, self.target_positions, self.linear_velocity.tracker,
+                                                    self.angular_velocity.tracker, self.progress_buf, fb["euler"], self.heading_diff,
+                                                    None, None, pos_t, vel_t, self.obs_buf)],
+                           self.obs_buf.stride(0),
+                           *[_lib.ptr(t) for t in (fb["dist"], fb["wheel"] if want_rocks else None, fb["body"] if want_rocks else None,
+                                                    self.rock_collison if want_rocks else None, self.rew_buf, self.reset_buf,
+                                                    e["pos_reward"], e["collision_penalty"], e["uprightness_penalty"],
+                                                    e["heading_contraint_penalty"], e["motion_contraint_penalty"],
+                                                    e["goal_angle_penalty"], self.stats, self._stats_scratch, self.obs16_buf)],
+                           0 if self.obs16_buf is None else self.obs16_buf.stride(0))
+
+    def _after_post(self, pos, want_rocks):
+        """What follows rvb_env_step / rvb_env_post: observation hooks (rover.py:326-329), attributes, extras."""
+        fb = self._fused
+        if not want_rocks:                                          # no rock kernel was launched
             _lib.launch_count -= 1
-        if self.obs_hooks is not None:                              # rover.py:326-329
+        if self.obs_hooks is not None:
             self.obs_hooks.apply(self.obs_buf, epoch=self.global_step, env_offset=self.env_offset)
-        self.rover_positions, self.rover_rotation, self.rover_rot = pos, fb["euler"], fb["euler"]
+        self.rover_positions, self.rover_rotation = pos, fb["euler"]
         self.rock_wheel_dist, self.rock_body_dist = (fb["wheel"], fb["body"]) if want_rocks else (None, None)
-        self.joint_position_targets, self.joint_velocity_targets = fb["pos_t"], fb["vel_t"]
-        if hasattr(self._rover, "set_joint_position_targets"):
-            self._rover.set_joint_position_targets(fb["pos_t"], indices=None,
-                                                   joint_indices=getattr(self._rover, "actuated_pos_indices", None))
-            self._rover.set_joint_velocity_targets(fb["vel_t"], indices=None,
-                                                   joint_indices=getattr(self._rover, "actuated_vel_indices", None))
         self.extras.update(self._ex)
         self.extras["torque_penalty_driving"] = self.linear_velocity.tracker[:, 0, 0]      # rover.py:530-531
         self.extras["torque_penalty_steering"] = self.angular_velocity.tracker[:, 0, 0]
-        return self.obs_buf, self.rew_buf, self.reset_buf, self.extras
+
+    def _hand_targets(self, pos_t, vel_t):
+        """rover.py:412-414: the joint targets go to the view."""
+        self.joint_position_targets, self.joint_velocity_targets = pos_t, vel_t
+        if hasattr(self._rover, "set_joint_position_targets"):
+            self._rover.set_joint_position_targets(pos_t, indices=None, joint_indices=getattr(self._rover, "actuated_pos_indices", None))
+            self._rover.set_joint_velocity_targets(vel_t, indices=None, joint_indices=getattr(self._rover, "actuated_vel_indices", None))
 
     # ------------------------------------------------------------------ get_observations (rover.py:272-336)
     def get_observations(self) -> dict:
