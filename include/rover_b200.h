@@ -211,7 +211,8 @@ typedef struct rvb_step_io {
     double* stats; double* stats_scratch;
     /* optional packed observation (ABI 2): obs_h16 f16 [N, obs_h16_ld >= sparse+dense] receives the heightmap columns
      * (obs column c -> obs_h16 column c - 4) as the fp16 values they are by construction (fp16(dist / 2), rover.py:324-325);
-     * obs[:, 4:] is then NOT written (obs[:, 0:4] still is).  Halves the bytes a host-side consumer has to read back. */
+     * obs[:, 4:] is then NOT written (obs[:, 0:4] still is).  Halves the bytes a host-side consumer has to read back.  The teacher-data
+     * recorder then reads the observation from obs_h16 and obs[:, 0:4] (rvb_teacher_record_packed), never from obs[:, 4:]. */
     uint16_t* obs_h16; int64_t obs_h16_ld;
 } rvb_step_io;
 int rvb_env_step(const rvb_terrain* terrain, const rvb_terrain* rocks, const rvb_reward_params* p, const rvb_step_io* io,
@@ -363,6 +364,17 @@ int rvb_obs_hooks(float* obs, int64_t obs_ld, int64_t N, int64_t C, int64_t col0
                   float offset, const uint8_t* zero_mask, uint64_t seed, uint64_t epoch, int64_t env_offset, void* stream);
 int rvb_teacher_record(const float* reset_info, const float* actions, int64_t actions_ld, const float* obs, int64_t obs_ld,
                        int64_t N, int64_t C, float* record, int64_t record_ld, void* stream);
+/* rvb_teacher_record on the packed observation of the fused step (rvb_step_io.obs_h16): proprio f32 [N, proprio_ld >= p] = obs[:, 0:p]
+ * (e.g. the strided view obs_buf[:, :4]; may be NULL when p == 0), heightmap f16 [N, heightmap_ld >= E] = obs_h16 (raw fp16 bits).
+ *   rec16 == NULL: rec[n] = [reset_info[n], a0, a1, proprio[n, 0..p), f32(heightmap[n, 0..E))]   rec_ld >= 3 + p + E
+ *                  -- bit for bit what rvb_teacher_record writes for the widened row cat(proprio, heightmap.float()).
+ *   rec16 != NULL: rec[n] = [reset_info[n], a0, a1, proprio[n, 0..p)]   rec_ld >= 3 + p,   rec16[n, 0..E) = heightmap[n, 0..E)
+ *                  (the bits copied: half the bytes of the f32 row; fp16 -> f32 is exact, so widening rec16 later gives the same rows).
+ * Any 2-byte aligned heightmap / rec16 and any row strides, odd ones included; 64-bit row offsets.  p in 0..8, E >= 1; N == 0 is a
+ * no-op.  Null pointers, short rows and misaligned pointers are refused on the host. */
+int rvb_teacher_record_packed(const float* reset_info, const float* actions, int64_t actions_ld, const float* proprio,
+                              int64_t proprio_ld, int64_t p, const uint16_t* heightmap, int64_t heightmap_ld, int64_t E, int64_t N,
+                              float* rec, int64_t rec_ld, uint16_t* rec16, int64_t rec16_ld, void* stream);
 
 #ifdef __cplusplus
 }

@@ -88,6 +88,7 @@ _SIGNATURES = {
     "rvb_policy_variant": (C.c_int, [C.c_int]),
     "rvb_obs_hooks": (C.c_int, [p, i64, i64, i64, i64, f32, f32, f32, p, C.c_uint64, C.c_uint64, i64, p]),
     "rvb_teacher_record": (C.c_int, [p, p, i64, p, i64, i64, i64, p, i64, p]),
+    "rvb_teacher_record_packed": (C.c_int, [p, p, i64, p, i64, i64, p, i64, i64, i64, p, i64, p, i64, p]),
 }
 
 EXPORTS = tuple(_SIGNATURES)
@@ -105,7 +106,7 @@ KERNELS_PER_CALL = {"rvb_terrain_create": 2, "rvb_heightmap_raycast": 4, "rvb_ca
     "rvb_stone_validate": 1, "rvb_spawn_validate": 1, "rvb_height_lookup": 1, "rvb_build_knn_index": 6, "rvb_reset_targets": 1,
                     "rvb_policy_create": 7, "rvb_policy_forward": 1, "rvb_policy_forward_pair": 1,
                     "rvb_policy_forward_packed": 2,
-                    "rvb_obs_hooks": 1, "rvb_teacher_record": 1}
+                    "rvb_obs_hooks": 1, "rvb_teacher_record": 1, "rvb_teacher_record_packed": 1}
 launch_count = 0
 
 

@@ -91,3 +91,115 @@ extern "C" int rvb_teacher_record(const float* reset_info, const float* actions,
     RVB_LAUNCH_CHECK();
     return RVB_OK;
 }
+
+// The recorder on the packed observation of the fused step (rvb_step_io.obs_h16): the row's lead [reset_info, a0, a1, proprio[0..p)]
+// in f32, then the E heightmap columns -- widened with __half2float (what torch's .float() does on the device, so the row is bit for
+// bit teacher_record_kernel's on cat(proprio, heightmap.float())) or copied as fp16 bits into their own block (rec16).
+// HBM-streaming.  One CTA per (row, chunk of TRP_CHUNK columns); the shipped row (1746 columns) is one chunk.  A 1746-half row is
+// only 4-byte aligned and every pointer and row stride may be odd, so the chunk is staged in shared memory: 16-byte loads aligned
+// on the source, then 16-byte streaming stores aligned on the destination, scalar accesses only for the partial lines at either end.
+// Bytes per env-step: 4 (reset) + 8 (actions) + 4p (proprio) + 2E read; 4(3 + p + E) written (f32 block) or 4(3 + p) + 2E (rec16).
+constexpr int TRP_THREADS = 128;
+constexpr int TRP_LINES = 2;                                      // 16-byte source lines per thread
+constexpr int TRP_CHUNK = TRP_LINES * TRP_THREADS * 8 - 8;       // 2040 columns: at any alignment they span <= 256 lines
+
+template <bool WIDEN>
+__global__ void __launch_bounds__(TRP_THREADS)
+teacher_record_packed_kernel(const float* __restrict__ reset_info, const float* __restrict__ actions, int64_t actions_ld,
+                             const float* __restrict__ proprio, int64_t proprio_ld, int p, const uint16_t* __restrict__ hm,
+                             int64_t hm_ld, int E, float* __restrict__ rec, int64_t rec_ld, uint16_t* __restrict__ rec16,
+                             int64_t rec16_ld) {
+    __shared__ __align__(16) uint16_t s[TRP_CHUNK + 8];
+    const int64_t n = blockIdx.y;
+    const int j0 = blockIdx.x * TRP_CHUNK;
+    const int m = min(TRP_CHUNK, E - j0);
+    float* row = rec + n * rec_ld;
+    const int t = threadIdx.x;
+    if (blockIdx.x == 0 && t < 3 + p) {
+        float v;
+        if (t == 0) v = reset_info[n];
+        else if (t < 3) v = actions[n * actions_ld + (t - 1)];
+        else v = proprio[n * proprio_ld + (t - 3)];
+        row[t] = v;
+    }
+    // column j of the chunk goes to s[a + j]: the source's 16-byte lines land on 16-byte lines of s
+    const uint16_t* src = hm + n * hm_ld + j0;
+    const int a = (int)((reinterpret_cast<uintptr_t>(src) >> 1) & 7);
+    uint4 v[TRP_LINES];
+#pragma unroll
+    for (int k = 0; k < TRP_LINES; ++k) {                   // every full line's load is in flight before the first is stored
+        const int lo = (t + k * TRP_THREADS) * 8 - a;
+        if (lo >= 0 && lo + 8 <= m) v[k] = __ldg(reinterpret_cast<const uint4*>(src + lo));
+    }
+#pragma unroll
+    for (int k = 0; k < TRP_LINES; ++k) {
+        const int l = t + k * TRP_THREADS, lo = l * 8 - a;
+        if (lo >= 0 && lo + 8 <= m) *reinterpret_cast<uint4*>(s + l * 8) = v[k];
+        else
+            for (int q = max(lo, 0); q < min(lo + 8, m); ++q) s[a + q] = src[q];
+    }
+    __syncthreads();
+    if (WIDEN) {
+        float* dst = row + 3 + p + j0;
+        const int b = (int)((reinterpret_cast<uintptr_t>(dst) >> 2) & 3);
+        for (int l = t; l < (b + m + 3) >> 2; l += TRP_THREADS) {
+            const int lo = l * 4 - b;
+            if (lo >= 0 && lo + 4 <= m) {
+                const uint16_t* h = s + a + lo;
+                __stcs(reinterpret_cast<float4*>(dst + lo), make_float4(__half2float(__ushort_as_half(h[0])), __half2float(__ushort_as_half(h[1])),
+                                                                        __half2float(__ushort_as_half(h[2])), __half2float(__ushort_as_half(h[3]))));
+            } else {
+                for (int q = max(lo, 0); q < min(lo + 4, m); ++q) dst[q] = __half2float(__ushort_as_half(s[a + q]));
+            }
+        }
+    } else {
+        uint16_t* dst = rec16 + n * rec16_ld + j0;
+        const int b = (int)((reinterpret_cast<uintptr_t>(dst) >> 1) & 7);
+        for (int l = t; l < (b + m + 7) >> 3; l += TRP_THREADS) {
+            const int lo = l * 8 - b;
+            if (lo >= 0 && lo + 8 <= m) {
+                uint4 w;
+                if (a == b) {
+                    w = *reinterpret_cast<const uint4*>(s + l * 8);
+                } else {
+                    const uint16_t* h = s + a + lo;
+                    w = make_uint4(h[0] | (uint32_t)h[1] << 16, h[2] | (uint32_t)h[3] << 16, h[4] | (uint32_t)h[5] << 16,
+                                   h[6] | (uint32_t)h[7] << 16);
+                }
+                __stcs(reinterpret_cast<uint4*>(dst + lo), w);
+            } else {
+                for (int q = max(lo, 0); q < min(lo + 8, m); ++q) dst[q] = s[a + q];
+            }
+        }
+    }
+}
+
+extern "C" int rvb_teacher_record_packed(const float* reset_info, const float* actions, int64_t actions_ld, const float* proprio,
+                                         int64_t proprio_ld, int64_t p, const uint16_t* heightmap, int64_t heightmap_ld, int64_t E,
+                                         int64_t N, float* rec, int64_t rec_ld, uint16_t* rec16, int64_t rec16_ld, void* stream) {
+    if (N == 0) return RVB_OK;
+    RVB_REQUIRE(reset_info && actions && heightmap && rec && (proprio || p == 0), "rvb_teacher_record_packed: null pointer");
+    RVB_REQUIRE(p >= 0 && p <= 8, "rvb_teacher_record_packed: p must be in 0..8");
+    RVB_REQUIRE(N > 0 && E > 0 && E < (1 << 30), "rvb_teacher_record_packed: bad shape");
+    RVB_REQUIRE(actions_ld >= 2 && proprio_ld >= p && heightmap_ld >= E && rec_ld >= 3 + p + (rec16 ? 0 : E) && (!rec16 || rec16_ld >= E),
+                "rvb_teacher_record_packed: short row");
+    RVB_REQUIRE(!((uintptr_t)reset_info & 3) && !((uintptr_t)actions & 3) && !((uintptr_t)proprio & 3) && !((uintptr_t)heightmap & 1) &&
+                    !((uintptr_t)rec & 3) && !((uintptr_t)rec16 & 1),
+                "rvb_teacher_record_packed: misaligned pointer");
+    const unsigned chunks = (unsigned)ceil_div(E, TRP_CHUNK);
+    for (int64_t n0 = 0; n0 < N; n0 += 65535) {             // grid.y = row: up to 65,535 per launch
+        const int64_t nb = (N - n0 < 65535) ? N - n0 : 65535;
+        const dim3 grid(chunks, (unsigned)nb);
+        const float* pr = proprio ? proprio + n0 * proprio_ld : nullptr;
+        if (rec16)
+            teacher_record_packed_kernel<false><<<grid, TRP_THREADS, 0, as_stream(stream)>>>(
+                reset_info + n0, actions + n0 * actions_ld, actions_ld, pr, proprio_ld, (int)p, heightmap + n0 * heightmap_ld,
+                heightmap_ld, (int)E, rec + n0 * rec_ld, rec_ld, rec16 + n0 * rec16_ld, rec16_ld);
+        else
+            teacher_record_packed_kernel<true><<<grid, TRP_THREADS, 0, as_stream(stream)>>>(
+                reset_info + n0, actions + n0 * actions_ld, actions_ld, pr, proprio_ld, (int)p, heightmap + n0 * heightmap_ld,
+                heightmap_ld, (int)E, rec + n0 * rec_ld, rec_ld, nullptr, 0);
+    }
+    RVB_LAUNCH_CHECK();
+    return RVB_OK;
+}

@@ -188,10 +188,17 @@ class _HeightmapNet:
 
 def _packed(states, nets):
     """The packed form of `states`, (proprio, heightmap), checked against every network of `nets`; nothing is copied."""
-    p = max(n.num_proprioception for n in nets)
-    e = max(n.num_exteroceptive for n in nets)
-    form = ("packed states must be (proprio float32 [N, >=%d], heightmap float16 [N, >=%d]) on one device, each with unit column "
-            "stride" % (p, e))
+    proprio, heightmap = packed_obs(states, max(n.num_proprioception for n in nets), max(n.num_exteroceptive for n in nets))
+    _lib.require_cuda(proprio, heightmap)
+    return proprio, heightmap
+
+
+def packed_obs(states, p, e, what="states"):
+    """`states` checked as the fused step's packed observation (proprio f32 [N, >=p], heightmap f16 [N, >=e]), e.g.
+    `(task.obs_buf[:, :4], task.obs16_buf)`; returns the two tensors, nothing is copied (their device is the caller's to check).
+    Shared by the networks and the teacher-data recorder (hooks.TeacherRecorder)."""
+    form = ("packed %s must be (proprio float32 [N, >=%d], heightmap float16 [N, >=%d]) on one device, each with unit column "
+            "stride" % (what, p, e))
     if len(states) != 2 or not all(isinstance(t, torch.Tensor) for t in states):
         raise RuntimeError(form)
     proprio, heightmap = states
@@ -199,7 +206,6 @@ def _packed(states, nets):
             or proprio.shape[0] != heightmap.shape[0] or proprio.shape[1] < p or heightmap.shape[1] < e
             or proprio.stride(1) != 1 or heightmap.stride(1) != 1 or proprio.device != heightmap.device):
         raise RuntimeError(form)
-    _lib.require_cuda(proprio, heightmap)
     return proprio, heightmap
 
 

@@ -236,7 +236,7 @@ class RoverTask():
         if self.save_teacher_data:                                  # rover.py:373-375, then :298-317 BEFORE obs_buf is refreshed
             self._teacher_actions = act[:, 0:2]
             if self.teacher_recorder is not None:
-                self.teacher_recorder.record(self.reset_info, self._teacher_actions, self.obs_buf)
+                self.teacher_recorder.record(self.reset_info, self._teacher_actions, self._teacher_obs())
         fb = self._step_buffers()
         want_rocks = self.curriculum_level >= 2
         io = self._step_io(pos, quat, joints, act, fb["pos_t"], fb["vel_t"], want_rocks)
@@ -283,7 +283,7 @@ class RoverTask():
     def post_physics_step_fused(self):
         """post_physics_step (rl_task.py:239-259) after pre_physics_step_fused and the simulator's step: ONE library call
         (rvb_env_post) on the poses and joints the view holds now, is_done on the rover_rot of the pre half.  Honours obs16_buf
-        like hot_step (then obs_buf[:, 4:] is not written)."""
+        like hot_step (then obs_buf[:, 4:] is not written, and the teacher recorder reads (obs_buf[:, :4], obs16_buf))."""
         if not self._is_playing():                                  # rl_task.py:241 comes before the guard at :250
             self.progress_buf[:] += 1
             return self.obs_buf, self.rew_buf, self.reset_buf, self.extras
@@ -296,7 +296,7 @@ class RoverTask():
             raise RuntimeError("post_physics_step_fused: no rover_rot; the pre-physics half has not run")
         self._step_buffers()
         if self.save_teacher_data and self.teacher_recorder is not None:       # rover.py:298-317: BEFORE obs_buf is refreshed
-            self.teacher_recorder.record(self.reset_info, self._teacher_actions, self.obs_buf)
+            self.teacher_recorder.record(self.reset_info, self._teacher_actions, self._teacher_obs())
         want_rocks = self.curriculum_level >= 2
         io = self._step_io(pos, quat, joints, None, None, None, want_rocks)
         prm = self._params()
@@ -313,6 +313,15 @@ class RoverTask():
         dev = torch.device(self._device)
         ok = actions.dtype == torch.float32 and actions.is_contiguous() and actions.device == dev
         return actions if ok else actions.to(dev, torch.float32).contiguous()
+
+    def _teacher_obs(self):
+        """The observation the fused step's recorder row pairs with this step's actions: obs_buf, or with obs16_buf set the packed
+        pair (obs_buf[:, :4], obs16_buf) -- the fused step then leaves obs_buf[:, 4:] unwritten.  The choice follows obs16_buf as it
+        is now: a task that switches obs16_buf on or off between steps records, for the step after the switch, a buffer the previous
+        step did not write."""
+        if self.obs16_buf is None:
+            return self.obs_buf
+        return self.obs_buf[:, :self._num_proprioceptive], self.obs16_buf
 
     def _refuse_hooks_with_obs16(self, who):
         if self.obs_hooks is not None and self.obs16_buf is not None:
