@@ -29,7 +29,7 @@
 extern "C" {
 #endif
 
-#define RVB_ABI_VERSION 4
+#define RVB_ABI_VERSION 5
 
 typedef enum rvb_status {
     RVB_OK = 0,
@@ -75,7 +75,7 @@ int rvb_terrain_destroy(rvb_terrain* t);
 int64_t rvb_terrain_bytes(const rvb_terrain* t);
 /* Gives back the handle's K-contiguous copy of map_indices (G0*G1*K int32 -- the same size as the reference's tensor,
  * camera.py:154-157; more than half of a layer).  The production heightmap ray-cast (variants 0 and 3 of rvb_heightmap_raycast,
- * rvb_env_step) never reads it; afterwards variants 1 / 2, rvb_cast_rays and rvb_rock_collision on THIS handle return
+ * rvb_env_post) never reads it; afterwards variants 1 / 2, rvb_cast_rays and rvb_rock_collision on THIS handle return
  * RVB_ERR_INVALID.  Needs the block lists (K <= 255).  Synchronises the device.  rvb_terrain_has_index: 1 / 0. */
 int rvb_terrain_release_index(rvb_terrain* t);
 int rvb_terrain_has_index(const rvb_terrain* t);
@@ -96,7 +96,7 @@ int64_t rvb_terrain_unbounded_triangles(const rvb_terrain* t);
  *   obs_h16/obs_h16_ld/obs_h16_col0: optional PACKED form of the same columns -- they are fp16 values by construction
  *        (rover.py:324-325 stores fp16(dist / 2) into the f32 obs_buf), so a consumer that wants half the bytes passes
  *        obs_h16[n*obs_h16_ld + (col - obs_h16_col0)] = fp16(dist/2)  for col in col_a/col_b >= 0  (obs may then be NULL).
- *        Not available with variant 1.  rvb_env_step uses it for rvb_step_io.obs_h16.
+ *        Not available with variant 1.  rvb_env_post uses it for rvb_step_io.obs_h16.
  * `variant`: 0 = production ("shadow" kernel: enumerates triangles, not (ray, candidate) pairs; needs the layer's block
  * lists, i.e. K <= 255, otherwise the tiled kernel on per-cell lists runs), 1 = simple per-pair kernel kept for
  * cross-checking, 2 = tiled kernel on per-cell lists, 3 = tiled kernel on 3x3-cell block lists.  All four are
@@ -189,21 +189,31 @@ int rvb_reward_reset(const rvb_reward_params* p,
                      double* stats, double* stats_scratch, void* stream);
 
 /* ------------------------------------------------------------------------------------------------
- * One env step with a single host call: the action half of RoverTask.pre_physics_step (rover.py:366-414: Memory.input_state,
- * Ackermann, joint targets) followed by RLTask.post_physics_step (rl_task.py:239-259: progress += 1, get_observations,
- * calculate_metrics, is_done) on the poses in `pos`/`quat` (PhysX is outside this library).  Equivalent to calling
- * rvb_quat_to_euler, rvb_history_push x2, rvb_ackermann, rvb_obs_proprio, rvb_heightmap_raycast (obs fused),
- * rvb_rock_collision and rvb_reward_reset in that order; the rock layer is cast on an internal forked stream, concurrently
- * with the heightmap.  rover_rot of is_done (rover.py:343,615) is taken from the same poses.
- *   lin_hist/ang_hist f32 [N,H] (Memory.tracker, newest first; shifted in place)   progress i64 [N] (incremented in place)
- *   euler f32 [N,3]  heading f32 [N]  steer/vel [N,6]  pos_targets [N,4]  vel_targets [N,6] (the last four optional)
+ * One env step with two host calls, split at the simulator's boundary, for the loop this library is built into:
+ *   obs_t -> policy -> pre_physics_step(a_t) -> simulator steps -> post_physics_step() -> obs_{t+1}.
+ * PhysX is outside this library: a caller without a simulator step between the calls passes the same poses to both.
+ *
+ * rvb_env_pre is the action half of RoverTask.pre_physics_step (rover.py:338-414) on the PRE-physics pose: rover_rot =
+ * tensor_quat_to_eul(quat) (rover.py:343; is_done reads it one post half later, :615-616), Memory.input_state x2 (:379-380,389),
+ * Ackermann + joint targets (:391,400-409): rvb_quat_to_euler, rvb_history_push x2 and rvb_ackermann in one launch.  It reads
+ * no goal, progress or reset state, so it may run before or after the reset half of pre_physics_step.
+ *   quat f32 [N,4] (16-byte aligned)  actions f32 [N,2]  lin_hist/ang_hist f32 [N,H] (shifted in place)  rover_rot f32 [N,3]
+ *   pos_targets f32 [N,4] (FR,RR,FL,RL), vel_targets f32 [N,6] (FR,CR,RR,FL,CL,RL), both optional.
+ *
+ * rvb_env_post is RLTask.post_physics_step (rl_task.py:239-259) on the POST-physics poses in io: progress += 1, get_observations
+ * (euler -> io.euler, heading, proprioceptive columns with this step's action read from lin_hist/ang_hist[:, 0], heightmap
+ * ray-cast into obs or obs_h16, rock layer), calculate_metrics + is_done with the rover_rot of rvb_env_pre.  Equivalent to
+ * calling rvb_quat_to_euler, rvb_obs_proprio, rvb_heightmap_raycast (obs fused), rvb_rock_collision and rvb_reward_reset in
+ * that order; the rock layer is cast on an internal forked stream, concurrently with the heightmap.
+ *   lin_hist/ang_hist f32 [N,H] (Memory.tracker, newest first; as rvb_env_pre left them)   progress i64 [N] (incremented in place)
+ *   euler f32 [N,3]  heading f32 [N]
  *   obs f32 [N,obs_ld>=4+sparse+dense]  dist f16 [N,P]  wheel_dist f16 [N,24]  body_dist f16 [N,2]  rock_collision i64 [N]
  *   (rock outputs and the `rocks` layer may be NULL when curriculum_level < 2); rew, reset, ex_*, stats as rvb_reward_reset.
  * ---------------------------------------------------------------------------------------------- */
 typedef struct rvb_step_io {
-    const float* pos; const float* quat; const float* joints; const float* actions; const float* target;
+    const float* pos; const float* quat; const float* joints; const float* target;
     float* lin_hist; float* ang_hist; int64_t* progress;
-    float* euler; float* heading; float* steer; float* vel; float* pos_targets; float* vel_targets;
+    float* euler; float* heading;
     float* obs; int64_t obs_ld;
     uint16_t* dist; uint16_t* wheel_dist; uint16_t* body_dist; int64_t* rock_collision;
     float* rew; int64_t* reset;
@@ -215,30 +225,13 @@ typedef struct rvb_step_io {
      * recorder then reads the observation from obs_h16 and obs[:, 0:4] (rvb_teacher_record_packed), never from obs[:, 4:]. */
     uint16_t* obs_h16; int64_t obs_h16_ld;
 } rvb_step_io;
-int rvb_env_step(const rvb_terrain* terrain, const rvb_terrain* rocks, const rvb_reward_params* p, const rvb_step_io* io,
-                 const double* pattern, int64_t P, const int32_t* col_a, const int32_t* col_b, int64_t N, int64_t H,
-                 void* stream);
-
-/* The same step split at the simulator's boundary, for the loop this library is built into:
- *   obs_t -> policy -> pre_physics_step(a_t) -> simulator steps -> post_physics_step() -> obs_{t+1}.
- * rvb_env_pre is the action half of RoverTask.pre_physics_step (rover.py:338-414) on the PRE-physics pose: rover_rot =
- * tensor_quat_to_eul(quat) (rover.py:343; is_done reads it one post half later, :615-616), Memory.input_state x2 (:379-380,389),
- * Ackermann + joint targets (:391,400-409).  One launch.  It reads no goal, progress or reset state, so it may run before or
- * after the reset half of pre_physics_step.
- *   quat f32 [N,4] (16-byte aligned)  actions f32 [N,2]  lin_hist/ang_hist f32 [N,H] (shifted in place)  rover_rot f32 [N,3]
- *   steer/vel [N,6], pos_targets [N,4], vel_targets [N,6] optional.
- * rvb_env_post is RLTask.post_physics_step (rl_task.py:239-259) on the POST-physics poses in io: progress += 1, get_observations
- * (euler -> io.euler, heading, proprioceptive columns with this step's action read from lin_hist/ang_hist[:, 0], heightmap
- * ray-cast into obs or obs_h16, rock layer on the forked stream), calculate_metrics + is_done with the rover_rot of rvb_env_pre.
- * io as rvb_env_step; io.actions, steer, vel, pos_targets and vel_targets are not read and may be NULL.  Same kernels as
- * rvb_env_step after its first one, so for an unchanged pose the pair gives rvb_env_step's results bit for bit. */
 int rvb_env_pre(const float* quat, const float* actions, int64_t N, int64_t H, float* lin_hist, float* ang_hist,
-                float* rover_rot, float* steer, float* vel, float* pos_targets, float* vel_targets, int sem, void* stream);
+                float* rover_rot, float* pos_targets, float* vel_targets, int sem, void* stream);
 int rvb_env_post(const rvb_terrain* terrain, const rvb_terrain* rocks, const rvb_reward_params* p, const rvb_step_io* io,
                  const float* rover_rot, const double* pattern, int64_t P, const int32_t* col_a, const int32_t* col_b,
                  int64_t N, int64_t H, void* stream);
 
-/* Device timing of the heightmap ray-cast inside rvb_env_step and rvb_env_post (CUDA events on the caller's stream, calling thread only):
+/* Device timing of the heightmap ray-cast inside rvb_env_post (CUDA events on the caller's stream, calling thread only):
  * enable, run steps, then read the per-step durations in ms (host array; returns the count or <0; synchronises). */
 int rvb_timing_enable(int on);
 int rvb_timing_read(float* ms_host, int cap);

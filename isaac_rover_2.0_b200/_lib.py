@@ -39,8 +39,8 @@ ACTIVATIONS = {"leakyrelu": 0, "relu": 1, "elu": 2, "tanh": 3, "sigmoid": 4, "re
 
 class StepIO(C.Structure):
     """rvb_step_io (include/rover_b200.h)."""
-    _fields_ = [(n, p) for n in ("pos", "quat", "joints", "actions", "target", "lin_hist", "ang_hist", "progress", "euler", "heading",
-                                 "steer", "vel", "pos_targets", "vel_targets", "obs")] + [("obs_ld", i64)] + \
+    _fields_ = [(n, p) for n in ("pos", "quat", "joints", "target", "lin_hist", "ang_hist", "progress", "euler", "heading",
+                                 "obs")] + [("obs_ld", i64)] + \
                [(n, p) for n in ("dist", "wheel_dist", "body_dist", "rock_collision", "rew", "reset", "ex_pos_reward", "ex_collision",
                                  "ex_uprightness", "ex_heading", "ex_motion", "ex_goal_angle", "stats", "stats_scratch", "obs_h16")] + \
                [("obs_h16_ld", i64)]
@@ -67,8 +67,7 @@ _SIGNATURES = {
     "rvb_obs_gather": (C.c_int, [p, i64, i64, p, i64, p, i64, i64, p]),
     "rvb_stats_scratch_len": (i64, [i64]),
     "rvb_reward_reset": (C.c_int, [C.POINTER(RewardParams)] + [p] * 11 + [i64] + [p] * 10 + [p]),
-    "rvb_env_step": (C.c_int, [p, p, C.POINTER(RewardParams), C.POINTER(StepIO), p, i64, p, p, i64, i64, p]),
-    "rvb_env_pre": (C.c_int, [p, p, i64, i64, p, p, p, p, p, p, p, C.c_int, p]),
+    "rvb_env_pre": (C.c_int, [p, p, i64, i64, p, p, p, p, p, C.c_int, p]),
     "rvb_env_post": (C.c_int, [p, p, C.POINTER(RewardParams), C.POINTER(StepIO), p, p, i64, p, p, i64, i64, p]),
     "rvb_timing_enable": (C.c_int, [C.c_int]),
     "rvb_timing_read": (C.c_int, [C.POINTER(f32), C.c_int]),
@@ -101,8 +100,8 @@ def lib_path():
 # kernels launched per entry point (for bench.py's `gpu_launches` claim)
 KERNELS_PER_CALL = {"rvb_terrain_create": 2, "rvb_heightmap_raycast": 4, "rvb_cast_rays": 2, "rvb_ray_distance": 1,
                     "rvb_rock_collision": 1, "rvb_check_collision": 1, "rvb_quat_to_euler": 1, "rvb_ackermann": 1,
-                    "rvb_history_push": 1, "rvb_obs_proprio": 1, "rvb_obs_gather": 1, "rvb_reward_reset": 2, "rvb_env_step": 8,
-                    "rvb_env_pre": 1, "rvb_env_post": 8,
+                    "rvb_history_push": 1, "rvb_obs_proprio": 1, "rvb_obs_gather": 1, "rvb_reward_reset": 2, "rvb_env_pre": 1,
+                    "rvb_env_post": 8,
     "rvb_stone_validate": 1, "rvb_spawn_validate": 1, "rvb_height_lookup": 1, "rvb_build_knn_index": 6, "rvb_reset_targets": 1,
                     "rvb_policy_create": 7, "rvb_policy_forward": 1, "rvb_policy_forward_pair": 1,
                     "rvb_policy_forward_packed": 2,
@@ -150,7 +149,7 @@ def load():
         fn.restype = res
         fn.argtypes = args
         setattr(lib, name, _Counted(fn, KERNELS_PER_CALL[name]) if name in KERNELS_PER_CALL else fn)
-    if lib.rvb_abi_version() != 4:
+    if lib.rvb_abi_version() != 5:
         raise RuntimeError("librover_b200.so ABI version mismatch")
     _lib = lib
     return lib

@@ -32,7 +32,7 @@ int rvb_set_error(int code, const char* what, const char* detail);
 cudaError_t rvb_scratch_alloc(void** p, size_t bytes, cudaStream_t st);
 
 // Side stream + fork / join events of the calling thread for the current device (slot 0: rock layer beside the heightmap in
-// rvb_env_step; slot 1: steep envs beside the shadow kernel), created once per (thread, device, slot) and kept.
+// rvb_env_post; slot 1: steep envs beside the shadow kernel), created once per (thread, device, slot) and kept.
 struct RvbSide {
     cudaStream_t s;
     cudaEvent_t fork, join;

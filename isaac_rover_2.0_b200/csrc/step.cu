@@ -1,45 +1,21 @@
-// Fused env step: everything RLTask.post_physics_step (rl_task.py:239-259) and the action half of
-// RoverTask.pre_physics_step (rover.py:366-414) compute for one step, enqueued by ONE host call:
-//   step_pre_kernel      progress += 1, tensor_quat_to_eul, Memory.input_state x2, Ackermann + joint targets,
-//                        proprioceptive observation columns + heading               (one thread per env)
-//   heightmap ray-cast   Camera.get_depths with the sparse/dense gather fused into obs_buf[:, 4:]
-//   rock collision       Rock_Detection.get_collisions + check_collision, on a forked stream (independent of the ray-cast)
-//   reward_reset         calculate_metrics + is_done + episode statistics (rvb_reward_reset)
-// The per-call entry points of rover_b200.h stay the reference-shaped API; this one removes ~25 Python/ctypes round trips
+// Fused env step: everything the action half of RoverTask.pre_physics_step (rover.py:366-414) and RLTask.post_physics_step
+// (rl_task.py:239-259) compute for one step, enqueued by two host calls, one on each side of the simulator's step:
+//   rvb_env_pre            env_pre_kernel: tensor_quat_to_eul of the pre-physics pose (rover_rot), Memory.input_state x2,
+//                          Ackermann + joint targets                                    (one thread per env)
+//   rvb_env_post           env_post_kernel: progress += 1, euler of the post-physics pose, proprioceptive columns + heading
+//                          (one thread per env), then:
+//     heightmap ray-cast   Camera.get_depths with the sparse/dense gather fused into obs_buf[:, 4:]
+//     rock collision       Rock_Detection.get_collisions + check_collision, on a forked stream (independent of the ray-cast)
+//     reward_reset         calculate_metrics + is_done + episode statistics (rvb_reward_reset)
+// The per-call entry points of rover_b200.h stay the reference-shaped API; this pair removes ~25 Python/ctypes round trips
 // per step (the host side was the bottleneck once the ray-cast dropped below 1.5 ms).
-// The same step split at the simulator's boundary, for a loop in which physics runs between the halves:
-//   rvb_env_pre          env_pre_kernel: tensor_quat_to_eul of the pre-physics pose (rover_rot), Memory.input_state x2,
-//                        Ackermann + joint targets
-//   rvb_env_post         env_post_kernel (progress += 1, euler of the post-physics pose, proprioceptive columns + heading),
-//                        then the ray-cast, rock layer and reward_reset of the fused step (post_body, shared with rvb_env_step)
 #include "task_dev.cuh"
 #include "raycast_common.cuh"
-
-__global__ void step_pre_kernel(rvb_step_io io, int64_t N, int H, int sem) {
-    const int64_t n = blockIdx.x * (int64_t)blockDim.x + threadIdx.x;
-    if (n >= N) return;
-    if (io.progress) io.progress[n] += 1;                                      // rl_task.py:241
-    const float4 q = reinterpret_cast<const float4*>(io.quat)[n];
-    float r, p, y;
-    quat_to_euler_dev(q.x, q.y, q.z, q.w, r, p, y);
-    io.euler[n * 3 + 0] = r; io.euler[n * 3 + 1] = p; io.euler[n * 3 + 2] = y;
-    const float lin = io.actions[n * 2 + 0], ang = io.actions[n * 2 + 1];
-    float* hl = io.lin_hist + n * H;
-    float* ha = io.ang_hist + n * H;
-    for (int i = H - 1; i > 0; --i) { hl[i] = hl[i - 1]; ha[i] = ha[i - 1]; }  // rover.py:76-77
-    hl[0] = lin; ha[0] = ang;
-    float st[6], ve[6];
-    ackermann_dev(lin, ang, sem, st, ve);
-    ackermann_store(n, st, ve, io.steer, io.vel, io.pos_targets, io.vel_targets);
-    obs_proprio_dev(io.pos[n * 3 + 0], io.pos[n * 3 + 1], y, io.target[n * 3 + 0], io.target[n * 3 + 1], lin, ang, sem,
-                    io.obs + n * io.obs_ld, io.heading + n);
-}
 
 // action half alone: rover_rot is the euler of the pose BEFORE physics (rover.py:343), is_done reads it one post half later
 __global__ void env_pre_kernel(const float* __restrict__ quat, const float* __restrict__ actions, int64_t N, int H,
                                float* __restrict__ lin_hist, float* __restrict__ ang_hist, float* __restrict__ rover_rot,
-                               float* __restrict__ steer, float* __restrict__ vel, float* __restrict__ pos_t,
-                               float* __restrict__ vel_t, int sem) {
+                               float* __restrict__ pos_t, float* __restrict__ vel_t, int sem) {
     const int64_t n = blockIdx.x * (int64_t)blockDim.x + threadIdx.x;
     if (n >= N) return;
     const float4 q = reinterpret_cast<const float4*>(quat)[n];
@@ -53,7 +29,7 @@ __global__ void env_pre_kernel(const float* __restrict__ quat, const float* __re
     hl[0] = lin; ha[0] = ang;
     float st[6], ve[6];
     ackermann_dev(lin, ang, sem, st, ve);
-    ackermann_store(n, st, ve, steer, vel, pos_t, vel_t);
+    ackermann_store(n, st, ve, nullptr, nullptr, pos_t, vel_t);
 }
 
 // per-env start of the observation half on the post-physics pose; this step's action is hist[:, 0], pushed by the pre half
@@ -72,7 +48,7 @@ __global__ void env_post_kernel(rvb_step_io io, int64_t N, int H, int sem) {
 #include <vector>
 
 namespace {
-// optional device timing of the heightmap ray-cast inside rvb_env_step (bench.py's roofline figure)
+// optional device timing of the heightmap ray-cast inside rvb_env_post (bench.py's roofline figure)
 struct Timing {
     bool on = false;
     std::vector<cudaEvent_t> ev;     // start, end, start, end, ...
@@ -82,17 +58,39 @@ thread_local Timing g_timing;
 
 }  // namespace
 
-// Everything of the step after its per-env kernel, on the euler that kernel wrote to io.euler: env order, rock layer on the forked
-// stream, heightmap ray-cast, join, reward_reset.  The knobs are read before `first` enqueues the per-env kernel, so that a bad
-// knob fails the call before anything is launched.  rover_rot: the euler is_done reads (io.euler when no physics ran in between).
-template <class First>
-static int post_body(const rvb_terrain* terrain, const rvb_terrain* rocks, const rvb_reward_params* p, const rvb_step_io& io,
-                     const float* rover_rot, const double* pattern, int64_t P, const int32_t* col_a, const int32_t* col_b,
-                     int64_t N, int64_t H, cudaStream_t st, First first) {
+extern "C" int rvb_env_pre(const float* quat, const float* actions, int64_t N, int64_t H, float* lin_hist, float* ang_hist,
+                           float* rover_rot, float* pos_targets, float* vel_targets, int sem, void* stream) {
+    RVB_REQUIRE(N >= 0, "rvb_env_pre: N < 0");
+    if (N == 0) return RVB_OK;
+    RVB_REQUIRE(quat && actions && lin_hist && ang_hist && rover_rot, "rvb_env_pre: null pointer");
+    RVB_REQUIRE(((uintptr_t)quat & 15) == 0, "rvb_env_pre: quat must be 16-byte aligned");
+    RVB_REQUIRE(H >= 2 && H <= 64, "rvb_env_pre: history length out of range");
+    env_pre_kernel<<<(unsigned)ceil_div(N, 256), 256, 0, as_stream(stream)>>>(quat, actions, N, (int)H, lin_hist, ang_hist, rover_rot,
+                                                                             pos_targets, vel_targets, sem);
+    RVB_LAUNCH_CHECK();
+    return RVB_OK;
+}
+
+extern "C" int rvb_env_post(const rvb_terrain* terrain, const rvb_terrain* rocks, const rvb_reward_params* p, const rvb_step_io* io_,
+                            const float* rover_rot, const double* pattern, int64_t P, const int32_t* col_a, const int32_t* col_b,
+                            int64_t N, int64_t H, void* stream) {
+    RVB_REQUIRE(N >= 0, "rvb_env_post: N < 0");
+    if (N == 0) return RVB_OK;
+    RVB_REQUIRE(terrain && p && io_ && rover_rot && pattern && col_a && col_b, "rvb_env_post: null pointer");
+    const rvb_step_io io = *io_;
+    RVB_REQUIRE(io.pos && io.quat && io.joints && io.target && io.lin_hist && io.ang_hist && io.euler && io.heading && io.obs &&
+                    io.dist && io.rew && io.reset && io.progress, "rvb_env_post: null pointer in rvb_step_io");
+    RVB_REQUIRE(((uintptr_t)io.quat & 15) == 0, "rvb_env_post: quat must be 16-byte aligned");
+    RVB_REQUIRE(H >= 2 && H <= 64 && io.obs_ld >= 4, "rvb_env_post: bad history length or obs_ld");
+    RVB_REQUIRE(!io.obs_h16 || io.obs_h16_ld > 0, "rvb_env_post: obs_h16 needs obs_h16_ld");
+    RVB_REQUIRE(p->curriculum_level < 2 || (rocks && io.wheel_dist && io.body_dist && io.rock_collision),
+                "rvb_env_post: curriculum_level >= 2 needs the rock layer and its outputs");
+    cudaStream_t st = as_stream(stream);
+    // the knobs are read before the first launch, so that a bad knob fails the call before anything is launched
     RaycastKnobs knobs;
     const int krc = read_raycast_knobs(knobs);
     if (krc != RVB_OK) return krc;
-    first();
+    env_post_kernel<<<(unsigned)ceil_div(N, 256), 256, 0, st>>>(io, N, (int)H, p->sem);
     RVB_LAUNCH_CHECK();
     cudaEvent_t t0 = nullptr, t1 = nullptr;
     if (g_timing.on) {
@@ -143,58 +141,6 @@ static int post_body(const rvb_terrain* terrain, const rvb_terrain* rocks, const
                             io.joints, io.progress, p->curriculum_level >= 2 ? io.rock_collision : nullptr, N, io.rew, io.reset,
                             io.ex_pos_reward, io.ex_collision, io.ex_uprightness, io.ex_heading, io.ex_motion, io.ex_goal_angle,
                             io.stats, io.stats_scratch, st);
-}
-
-extern "C" int rvb_env_step(const rvb_terrain* terrain, const rvb_terrain* rocks, const rvb_reward_params* p,
-                            const rvb_step_io* io_, const double* pattern, int64_t P, const int32_t* col_a,
-                            const int32_t* col_b, int64_t N, int64_t H, void* stream) {
-    RVB_REQUIRE(N >= 0, "rvb_env_step: N < 0");
-    if (N == 0) return RVB_OK;
-    RVB_REQUIRE(terrain && p && io_ && pattern && col_a && col_b, "rvb_env_step: null pointer");
-    const rvb_step_io io = *io_;
-    RVB_REQUIRE(io.pos && io.quat && io.joints && io.actions && io.target && io.lin_hist && io.ang_hist && io.euler && io.heading &&
-                    io.obs && io.dist && io.rew && io.reset && io.progress, "rvb_env_step: null pointer in rvb_step_io");
-    RVB_REQUIRE(((uintptr_t)io.quat & 15) == 0, "rvb_env_step: quat must be 16-byte aligned");
-    RVB_REQUIRE(H >= 2 && H <= 64 && io.obs_ld >= 4, "rvb_env_step: bad history length or obs_ld");
-    RVB_REQUIRE(!io.obs_h16 || io.obs_h16_ld > 0, "rvb_env_step: obs_h16 needs obs_h16_ld");
-    RVB_REQUIRE(p->curriculum_level < 2 || (rocks && io.wheel_dist && io.body_dist && io.rock_collision),
-                "rvb_env_step: curriculum_level >= 2 needs the rock layer and its outputs");
-    cudaStream_t st = as_stream(stream);
-    // rover_rot = euler: no physics between the halves
-    return post_body(terrain, rocks, p, io, io.euler, pattern, P, col_a, col_b, N, H, st,
-                     [&] { step_pre_kernel<<<(unsigned)ceil_div(N, 256), 256, 0, st>>>(io, N, (int)H, p->sem); });
-}
-
-extern "C" int rvb_env_pre(const float* quat, const float* actions, int64_t N, int64_t H, float* lin_hist, float* ang_hist,
-                           float* rover_rot, float* steer, float* vel, float* pos_targets, float* vel_targets, int sem, void* stream) {
-    RVB_REQUIRE(N >= 0, "rvb_env_pre: N < 0");
-    if (N == 0) return RVB_OK;
-    RVB_REQUIRE(quat && actions && lin_hist && ang_hist && rover_rot, "rvb_env_pre: null pointer");
-    RVB_REQUIRE(((uintptr_t)quat & 15) == 0, "rvb_env_pre: quat must be 16-byte aligned");
-    RVB_REQUIRE(H >= 2 && H <= 64, "rvb_env_pre: history length out of range");
-    env_pre_kernel<<<(unsigned)ceil_div(N, 256), 256, 0, as_stream(stream)>>>(quat, actions, N, (int)H, lin_hist, ang_hist, rover_rot,
-                                                                             steer, vel, pos_targets, vel_targets, sem);
-    RVB_LAUNCH_CHECK();
-    return RVB_OK;
-}
-
-extern "C" int rvb_env_post(const rvb_terrain* terrain, const rvb_terrain* rocks, const rvb_reward_params* p, const rvb_step_io* io_,
-                            const float* rover_rot, const double* pattern, int64_t P, const int32_t* col_a, const int32_t* col_b,
-                            int64_t N, int64_t H, void* stream) {
-    RVB_REQUIRE(N >= 0, "rvb_env_post: N < 0");
-    if (N == 0) return RVB_OK;
-    RVB_REQUIRE(terrain && p && io_ && rover_rot && pattern && col_a && col_b, "rvb_env_post: null pointer");
-    const rvb_step_io io = *io_;
-    RVB_REQUIRE(io.pos && io.quat && io.joints && io.target && io.lin_hist && io.ang_hist && io.euler && io.heading && io.obs &&
-                    io.dist && io.rew && io.reset && io.progress, "rvb_env_post: null pointer in rvb_step_io");
-    RVB_REQUIRE(((uintptr_t)io.quat & 15) == 0, "rvb_env_post: quat must be 16-byte aligned");
-    RVB_REQUIRE(H >= 2 && H <= 64 && io.obs_ld >= 4, "rvb_env_post: bad history length or obs_ld");
-    RVB_REQUIRE(!io.obs_h16 || io.obs_h16_ld > 0, "rvb_env_post: obs_h16 needs obs_h16_ld");
-    RVB_REQUIRE(p->curriculum_level < 2 || (rocks && io.wheel_dist && io.body_dist && io.rock_collision),
-                "rvb_env_post: curriculum_level >= 2 needs the rock layer and its outputs");
-    cudaStream_t st = as_stream(stream);
-    return post_body(terrain, rocks, p, io, rover_rot, pattern, P, col_a, col_b, N, H, st,
-                     [&] { env_post_kernel<<<(unsigned)ceil_div(N, 256), 256, 0, st>>>(io, N, (int)H, p->sem); });
 }
 
 extern "C" int rvb_timing_enable(int on) {

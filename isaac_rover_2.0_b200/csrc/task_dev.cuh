@@ -4,7 +4,7 @@
 
 #include "common.cuh"
 
-// calculate_metrics + is_done with the episode statistics (task.cu; rvb_reward_reset and the end of rvb_env_step).
+// calculate_metrics + is_done with the episode statistics (task.cu; rvb_reward_reset and the end of rvb_env_post).
 // hs: element stride between consecutive envs in lin / lin_prev / ang / ang_prev (1 for packed columns, H for [N,H] histories)
 int launch_reward_reset(const rvb_reward_params* p, const float* pos, const float* target, const float* heading,
                         const float* rover_rot, const float* lin, const float* lin_prev, const float* ang,

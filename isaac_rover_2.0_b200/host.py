@@ -1,7 +1,7 @@
 """Host-buffer front end of the hot path: the call a simulator that keeps its state in HOST memory makes.
 
 `submit()` enqueues one env step: pinned host -> device copies of this step's poses / joints / actions, the device hot path
-(RoverTask.hot_step, one library call), and -- on a second stream -- device -> pinned host copies of obs_buf / rew_buf /
+(RoverTask.hot_step, two library calls), and -- on a second stream -- device -> pinned host copies of obs_buf / rew_buf /
 reset_buf.  `result(slot)` waits for that step's copies and returns the host tensors.  Two slots (double buffering): the
 28.7 MB observation read-back of step i overlaps the kernels of step i+1, and the inputs of step i+1 are uploaded on a third
 stream into the other slot's device buffers while step i still computes (measured: small uploads queued on the compute stream

@@ -208,49 +208,26 @@ class RoverTask():
         device_reset=True runs the reset half of pre_physics_step first (rover.py:356-361: book-keeping, goal
         re-sampling against stone_info, target heights) for every env whose reset_buf is set, on the device
         (rvb_reset_targets; pose resets stay with the simulator: `_rover.reset_idx_masked(mask, initial_pos)` when the
-        view offers it).  fused=True enqueues the rest of the step with ONE library call (rvb_env_step); fused=False makes
-        the reference's sequence of calls (same results, ~25 host round trips).  The observation hooks and the teacher
-        recorder (rover.py:298-317,326-329) run on both paths.  reset_mask: the mask to consume instead of reset_buf (i64 [N],
-        read only -- used by HostPipeline, whose reset_buf rotates between slots)."""
+        view offers it).  fused=True enqueues the rest of the step with two library calls (rvb_env_pre + rvb_env_post) on
+        the pose the view holds after the reset half; fused=False makes the reference's sequence of calls (same results,
+        ~25 host round trips).  The observation hooks and the teacher recorder (rover.py:298-317,326-329) run on both paths.
+        reset_mask: the mask to consume instead of reset_buf (i64 [N], read only -- used by HostPipeline, whose reset_buf
+        rotates between slots)."""
         self.global_step += 1                                       # rover.py:341
-        if device_reset:
-            mask = self.reset_buf if reset_mask is None else reset_mask
-            self._mark_reset_info(mask)
-            if hasattr(self._rover, "reset_idx_masked"):
-                self._rover.reset_idx_masked(mask.clone(), self.initial_pos)
-            self.reset_targets_device(reset_mask=reset_mask)
         if fused:
-            return self._hot_step_fused(actions)
-        _, quat = self._rover.get_world_poses()
-        self.rover_rot = tensor_quat_to_eul(quat)
-        self.apply_actions(actions)
-        return self.post_physics_step()
-
-    def _hot_step_fused(self, actions):
-        pos, quat = self._rover.get_world_poses()
-        joints = self._rover.get_joint_positions()
-        pos, quat, joints = _f32(pos), _f32(quat), _f32(joints)
-        act = self._actions_f32(actions)
-        _lib.require_cuda(pos, quat, joints, act)
-        self._refuse_hooks_with_obs16("hot_step")
-        if self.save_teacher_data:                                  # rover.py:373-375, then :298-317 BEFORE obs_buf is refreshed
-            self._teacher_actions = act[:, 0:2]
-            if self.teacher_recorder is not None:
-                self.teacher_recorder.record(self.reset_info, self._teacher_actions, self._teacher_obs())
-        fb = self._step_buffers()
-        want_rocks = self.curriculum_level >= 2
-        io = self._step_io(pos, quat, joints, act, fb["pos_t"], fb["vel_t"], want_rocks)
-        prm = self._params()
-        cam = self.Camera
-        with torch.cuda.device(torch.device(self._device)):
-            _lib.check(self._lib.rvb_env_step(cam.layer.handle, self.Rock_detector.layer.handle if want_rocks else None,
-                                              C.byref(prm), C.byref(io), _lib.ptr(cam.heightmap_distribution), self.num_exteroceptive,
-                                              _lib.ptr(cam._col_a), _lib.ptr(cam._col_b), self.num_envs, self.linear_velocity.horizon,
-                                              self._stream()))
-        self._after_post(pos, want_rocks)
-        self.rover_rot = fb["euler"]
-        self._hand_targets(fb["pos_t"], fb["vel_t"])
-        return self.obs_buf, self.rew_buf, self.reset_buf, self.extras
+            self._refuse_hooks_with_obs16("hot_step")
+        if device_reset:
+            self._reset_half(reset_mask=reset_mask)
+        if not fused:
+            _, quat = self._rover.get_world_poses()
+            self.rover_rot = tensor_quat_to_eul(quat)
+            self.apply_actions(actions)
+            return self.post_physics_step()
+        pos, quat, joints = self._view_state()
+        self._action_half(actions, quat)
+        out = self._observation_half(pos, quat, joints)
+        self._hand_targets()
+        return out
 
     # ------------------------------------------------------------------ the fused step split at the simulator's boundary
     def pre_physics_step_fused(self, actions, max_attempts=64) -> None:
@@ -259,26 +236,12 @@ class RoverTask():
         now.  Same side effects as pre_physics_step_device."""
         self.global_step += 1
         self.rover_loc, quat = self._rover.get_world_poses()
-        quat = _f32(quat)
-        act = self._actions_f32(actions)
-        _lib.require_cuda(quat, act)
-        if self.save_teacher_data:                                  # rover.py:373-375
-            self._teacher_actions = act[:, 0:2]
-        fb = self._step_buffers()
         # The action half is enqueued BEFORE the reset half, so rover_rot is the pose before the simulator's pose reset, as
         # rover.py:343 takes it before :356.  Moving it ahead changes nothing else: the reset half writes goal targets, progress,
         # reset flags and reset_info, none of which the action half (histories, steering, wheel velocities) reads or writes.
-        with torch.cuda.device(torch.device(self._device)):
-            _lib.check(self._lib.rvb_env_pre(_lib.ptr(quat), _lib.ptr(act), self.num_envs, self.linear_velocity.horizon,
-                                             _lib.ptr(self.linear_velocity.tracker), _lib.ptr(self.angular_velocity.tracker),
-                                             _lib.ptr(fb["rot"]), None, None, _lib.ptr(fb["pos_t"]), _lib.ptr(fb["vel_t"]), self.sem,
-                                             self._stream()))
-        self.rover_rot = fb["rot"]
-        self._mark_reset_info()
-        if hasattr(self._rover, "reset_idx_masked"):
-            self._rover.reset_idx_masked(self.reset_buf.clone(), self.initial_pos)
-        self.reset_targets_device(max_attempts=max_attempts)
-        self._hand_targets(fb["pos_t"], fb["vel_t"])               # after the resets, as apply_actions does
+        self._action_half(actions, _f32(quat))
+        self._reset_half(max_attempts=max_attempts)
+        self._hand_targets()                                        # after the resets, as apply_actions does
 
     def post_physics_step_fused(self):
         """post_physics_step (rl_task.py:239-259) after pre_physics_step_fused and the simulator's step: ONE library call
@@ -287,18 +250,54 @@ class RoverTask():
         if not self._is_playing():                                  # rl_task.py:241 comes before the guard at :250
             self.progress_buf[:] += 1
             return self.obs_buf, self.rew_buf, self.reset_buf, self.extras
+        pos, quat, joints = self._view_state()
+        self._refuse_hooks_with_obs16("post_physics_step_fused")
+        if self.rover_rot is None:
+            raise RuntimeError("post_physics_step_fused: no rover_rot; the pre-physics half has not run")
+        return self._observation_half(pos, quat, joints)
+
+    def _reset_half(self, reset_mask=None, max_attempts=64):
+        """The reset half of pre_physics_step on the device (rover.py:356-361) for the envs set in reset_mask (default reset_buf):
+        reset_info, the view's pose reset, then reset_targets_device."""
+        mask = self.reset_buf if reset_mask is None else reset_mask
+        # rover.py:420-422 without the host-side nonzero(): when any env resets, the reference sets reset_info of EVERY env
+        if self.save_teacher_data:
+            any_reset = (mask != 0).any().to(self.reset_info.dtype)
+            torch.maximum(self.reset_info, any_reset.expand_as(self.reset_info), out=self.reset_info)
+        if hasattr(self._rover, "reset_idx_masked"):
+            self._rover.reset_idx_masked(mask.clone(), self.initial_pos)
+        self.reset_targets_device(max_attempts=max_attempts, reset_mask=reset_mask)
+
+    def _view_state(self):
+        """The poses and joint positions the view holds now, as contiguous f32 device tensors."""
         pos, quat = self._rover.get_world_poses()
         joints = self._rover.get_joint_positions()
         pos, quat, joints = _f32(pos), _f32(quat), _f32(joints)
         _lib.require_cuda(pos, quat, joints)
-        self._refuse_hooks_with_obs16("post_physics_step_fused")
-        if self.rover_rot is None:
-            raise RuntimeError("post_physics_step_fused: no rover_rot; the pre-physics half has not run")
-        self._step_buffers()
+        return pos, quat, joints
+
+    def _action_half(self, actions, quat):
+        """rvb_env_pre on `quat`: rover_rot, both histories and the joint targets, which _hand_targets gives to the view."""
+        act = self._actions_f32(actions)
+        _lib.require_cuda(quat, act)
+        if self.save_teacher_data:                                  # rover.py:373-375
+            self._teacher_actions = act[:, 0:2]
+        fb = self._step_buffers()
+        with torch.cuda.device(torch.device(self._device)):
+            _lib.check(self._lib.rvb_env_pre(_lib.ptr(quat), _lib.ptr(act), self.num_envs, self.linear_velocity.horizon,
+                                             _lib.ptr(self.linear_velocity.tracker), _lib.ptr(self.angular_velocity.tracker),
+                                             _lib.ptr(fb["rot"]), _lib.ptr(fb["pos_t"]), _lib.ptr(fb["vel_t"]), self.sem,
+                                             self._stream()))
+        self.rover_rot = fb["rot"]
+
+    def _observation_half(self, pos, quat, joints):
+        """rvb_env_post on the view's state, is_done on rover_rot; the teacher recorder's row before it, the observation hooks
+        (rover.py:326-329), attributes and extras after it."""
+        fb = self._step_buffers()
         if self.save_teacher_data and self.teacher_recorder is not None:       # rover.py:298-317: BEFORE obs_buf is refreshed
             self.teacher_recorder.record(self.reset_info, self._teacher_actions, self._teacher_obs())
         want_rocks = self.curriculum_level >= 2
-        io = self._step_io(pos, quat, joints, None, None, None, want_rocks)
+        io = self._step_io(pos, quat, joints, want_rocks)
         prm = self._params()
         cam = self.Camera
         with torch.cuda.device(torch.device(self._device)):
@@ -306,7 +305,15 @@ class RoverTask():
                                               C.byref(prm), C.byref(io), _lib.ptr(self.rover_rot), _lib.ptr(cam.heightmap_distribution),
                                               self.num_exteroceptive, _lib.ptr(cam._col_a), _lib.ptr(cam._col_b), self.num_envs,
                                               self.linear_velocity.horizon, self._stream()))
-        self._after_post(pos, want_rocks)
+        if not want_rocks:                                          # no rock kernel was launched
+            _lib.launch_count -= 1
+        if self.obs_hooks is not None:
+            self.obs_hooks.apply(self.obs_buf, epoch=self.global_step, env_offset=self.env_offset)
+        self.rover_positions, self.rover_rotation = pos, fb["euler"]
+        self.rock_wheel_dist, self.rock_body_dist = (fb["wheel"], fb["body"]) if want_rocks else (None, None)
+        self.extras.update(self._ex)
+        self.extras["torque_penalty_driving"] = self.linear_velocity.tracker[:, 0, 0]      # rover.py:530-531
+        self.extras["torque_penalty_steering"] = self.angular_velocity.tracker[:, 0, 0]
         return self.obs_buf, self.rew_buf, self.reset_buf, self.extras
 
     def _actions_f32(self, actions):
@@ -338,12 +345,12 @@ class RoverTask():
                 pos_t=torch.empty((N, 4), device=dev), vel_t=torch.empty((N, 6), device=dev), rot=torch.empty((N, 3), device=dev))
         return self._fused
 
-    def _step_io(self, pos, quat, joints, act, pos_t, vel_t, want_rocks):
+    def _step_io(self, pos, quat, joints, want_rocks):
         fb = self._fused
         e = self._ex
-        return _lib.StepIO(*[_lib.ptr(t) for t in (pos, quat, joints, act, self.target_positions, self.linear_velocity.tracker,
+        return _lib.StepIO(*[_lib.ptr(t) for t in (pos, quat, joints, self.target_positions, self.linear_velocity.tracker,
                                                     self.angular_velocity.tracker, self.progress_buf, fb["euler"], self.heading_diff,
-                                                    None, None, pos_t, vel_t, self.obs_buf)],
+                                                    self.obs_buf)],
                            self.obs_buf.stride(0),
                            *[_lib.ptr(t) for t in (fb["dist"], fb["wheel"] if want_rocks else None, fb["body"] if want_rocks else None,
                                                     self.rock_collison if want_rocks else None, self.rew_buf, self.reset_buf,
@@ -352,21 +359,9 @@ class RoverTask():
                                                     e["goal_angle_penalty"], self.stats, self._stats_scratch, self.obs16_buf)],
                            0 if self.obs16_buf is None else self.obs16_buf.stride(0))
 
-    def _after_post(self, pos, want_rocks):
-        """What follows rvb_env_step / rvb_env_post: observation hooks (rover.py:326-329), attributes, extras."""
-        fb = self._fused
-        if not want_rocks:                                          # no rock kernel was launched
-            _lib.launch_count -= 1
-        if self.obs_hooks is not None:
-            self.obs_hooks.apply(self.obs_buf, epoch=self.global_step, env_offset=self.env_offset)
-        self.rover_positions, self.rover_rotation = pos, fb["euler"]
-        self.rock_wheel_dist, self.rock_body_dist = (fb["wheel"], fb["body"]) if want_rocks else (None, None)
-        self.extras.update(self._ex)
-        self.extras["torque_penalty_driving"] = self.linear_velocity.tracker[:, 0, 0]      # rover.py:530-531
-        self.extras["torque_penalty_steering"] = self.angular_velocity.tracker[:, 0, 0]
-
-    def _hand_targets(self, pos_t, vel_t):
-        """rover.py:412-414: the joint targets go to the view."""
+    def _hand_targets(self):
+        """rover.py:412-414: the joint targets of the action half go to the view."""
+        pos_t, vel_t = self._fused["pos_t"], self._fused["vel_t"]
         self.joint_position_targets, self.joint_velocity_targets = pos_t, vel_t
         if hasattr(self._rover, "set_joint_position_targets"):
             self._rover.set_joint_position_targets(pos_t, indices=None, joint_indices=getattr(self._rover, "actuated_pos_indices", None))
@@ -432,17 +427,8 @@ class RoverTask():
         self.global_step += 1
         self.rover_loc, quat = self._rover.get_world_poses()
         self.rover_rot = tensor_quat_to_eul(quat)
-        self._mark_reset_info()
-        if hasattr(self._rover, "reset_idx_masked"):
-            self._rover.reset_idx_masked(self.reset_buf.clone(), self.initial_pos)
-        self.reset_targets_device(max_attempts=max_attempts)
+        self._reset_half(max_attempts=max_attempts)
         self.apply_actions(actions)
-
-    def _mark_reset_info(self, mask=None):
-        """rover.py:420-422 without the host-side nonzero(): when any env resets, the reference sets reset_info of EVERY env."""
-        if self.save_teacher_data:
-            any_reset = ((self.reset_buf if mask is None else mask) != 0).any().to(self.reset_info.dtype)
-            torch.maximum(self.reset_info, any_reset.expand_as(self.reset_info), out=self.reset_info)
 
     def reset_targets_device(self, radius=8.0, thr=1.0, max_attempts=64, epoch=None, reset_mask=None):
         """reset_idx book-keeping + set_targets (rover.py:451-452, 566-584) for every env with reset_buf != 0, on the device.

@@ -14,7 +14,7 @@ def declared_symbols():
     return sorted(set(re.findall(r"\b(rvb_[a-z0-9_]+)\s*\(", src)))
 
 
-def test_header_symbols_exported():
+def test_header_symbols_exported_abi5():
     import isaac_rover_b200
     from isaac_rover_b200 import _lib
     lib = _lib.load()
@@ -26,7 +26,8 @@ def test_header_symbols_exported():
     assert set(names) == set(_lib.EXPORTS), set(names) ^ set(_lib.EXPORTS)
     for n in ("rvb_terrain_create", "rvb_heightmap_raycast", "rvb_rock_collision"):        # their "2" forms were merged into them
         assert not hasattr(raw, n + "2"), "removed entry point still exported: " + n + "2"
-    assert lib.rvb_abi_version() == 4
+    assert not hasattr(raw, "rvb_env_step"), "removed entry point still exported: rvb_env_step"    # the pair pre + post replaced it
+    assert lib.rvb_abi_version() == 5
 
 
 def test_argument_validation_without_gpu():

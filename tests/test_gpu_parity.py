@@ -722,7 +722,7 @@ def test_benchmark_world_matches_oracle(R, O, world200):
 
 
 def test_fused_step_equals_call_sequence(R, world20):
-    """rvb_env_step (one host call, rock layer on a forked stream) == the reference-shaped sequence of calls, for three
+    """The fused step (rvb_env_pre + rvb_env_post, rock layer on a forked stream) == the reference-shaped sequence of calls, for three
     consecutive steps (history shift, progress counter and statistics included); then the pipelined host front end."""
     w = world20
     N = 300

@@ -16,7 +16,7 @@ def lib():
 
 
 def _pre(lib, quat=FAKE, actions=FAKE, N=4, H=3, lin=FAKE, ang=FAKE, rot=FAKE):
-    return lib.rvb_env_pre(quat, actions, N, H, lin, ang, rot, None, None, None, None, 0, None)
+    return lib.rvb_env_pre(quat, actions, N, H, lin, ang, rot, None, None, 0, None)
 
 
 def _io(**kw):
@@ -25,8 +25,7 @@ def _io(**kw):
     for name, _ in _lib.StepIO._fields_:
         setattr(io, name, FAKE)
     io.obs_ld, io.obs_h16_ld = 1750, 0
-    for name in ("actions", "steer", "vel", "pos_targets", "vel_targets", "obs_h16"):       # not read by the post half
-        setattr(io, name, None)
+    io.obs_h16 = None                                               # the packed observation is optional
     for name, v in kw.items():
         setattr(io, name, v)
     return io
@@ -44,7 +43,7 @@ def _refused(lib, rc, what):
     assert what in msg, msg
 
 
-def test_env_pre_validation_without_gpu(lib):
+def test_env_pre_validation_abi5_without_gpu(lib):
     assert _pre(lib, N=0) == 0                                    # nothing to do
     _refused(lib, _pre(lib, N=-1), b"N < 0")
     for k in ("quat", "actions", "lin", "ang", "rot"):

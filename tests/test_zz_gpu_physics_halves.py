@@ -144,7 +144,9 @@ def test_packed_post_half(R, world20):
 
 @pytest.mark.parametrize("level", [1, 2])
 def test_unchanged_pose_equals_hot_step(R, world20, level):
-    """With no physics between the halves the pair is rvb_env_step: the bits of hot_step(device_reset=True)."""
+    """With no physics between the halves, the pair in a simulator loop's order (action half, then reset half) gives the bits of
+    hot_step(device_reset=True), which runs the reset half first and then the action half (this view moves no env on a reset, so
+    both orders read the same pose)."""
     st = R.synth.make_env_state(world20, N, seed=47)
     pair, step = [R.synth.make_task(world20, st, device="cuda:0", level=level) for _ in range(2)]
     g = torch.Generator().manual_seed(5)

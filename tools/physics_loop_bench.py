@@ -3,7 +3,8 @@ post_physics_step() -> obs_{t+1}, with a stand-in for physics that only swaps th
   (a) reference  pre_physics_step_device + post_physics_step   (the reference-shaped sequence of library calls)
   (b) fused      pre_physics_step_fused + post_physics_step_fused   (rvb_env_pre + rvb_env_post)
   (b16)          (b) with the packed fp16 observation (obs16_buf)
-  (c) hot_step   hot_step(device_reset=True)   (rvb_env_step: no physics between the halves; what bench.py times)
+  (c) hot_step   hot_step(device_reset=True)   (rvb_env_pre + rvb_env_post with no physics between them, the reset half first;
+                                                what bench.py times)
 Benchmark world (200 m, K = 200, 2000 stones), curriculum level 2, device-side reset on, one task per size.  The arms alternate
 round by round on the same task, so they see the same state distribution and the same clocks.  Every window is bracketed by CUDA
 events on the task's stream after a synchronise, so host time that holds the stream back is part of what is measured.
