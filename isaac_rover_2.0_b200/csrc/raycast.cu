@@ -110,51 +110,34 @@ cast_simple_kernel(const int32_t* __restrict__ index, const TriRec* __restrict__
 }
 
 static int launch_cast_simple(const rvb_terrain* t, const __half* src16, const __half* dneg16, int64_t R,
-                              int64_t rays_per_dir, uint16_t* dist, int32_t* hit_slot, int32_t* hit_tri, uint16_t* pt,
+                              int64_t rays_per_dir, __half* dist, int32_t* hit_slot, int32_t* hit_tri, __half* pt,
                               float* obs, int64_t obs_ld, const int32_t* col_a, const int32_t* col_b, cudaStream_t st) {
     const int64_t blocks = ceil_div(R * 32, 256);
     RVB_REQUIRE(blocks < ((int64_t)1 << 31), "cast: too many rays for one launch");
     cast_simple_kernel<<<(unsigned)blocks, 256, 0, st>>>(t->index, t->recs, (int)t->G0, (int)t->G1, (int)t->K, (int)t->Ks, t->res,
                                                          1.0f / t->res, t->shift_x, t->shift_y, t->sem, src16, dneg16, R,
-                                                         rays_per_dir, (__half*)dist, hit_slot, hit_tri, (__half*)pt, obs,
-                                                         obs_ld, col_a, col_b);
+                                                         rays_per_dir, dist, hit_slot, hit_tri, pt, obs, obs_ld, col_a, col_b);
     RVB_LAUNCH_CHECK();
     return RVB_OK;
 }
 
-int heightmap_raycast(const rvb_terrain* t, const float* pos, const float* euler, const float* trig, const double* pattern,
-                      int64_t P, int64_t N, uint16_t* dist, int32_t* hit_slot, int32_t* hit_tri, uint16_t* pt, uint16_t* sources,
-                      float* obs, int64_t obs_ld, uint16_t* obs_h16, int64_t obs_h16_ld, int obs_h16_col0, const int32_t* col_a,
-                      const int32_t* col_b, int variant, const RaycastKnobs& knobs, const int32_t* order, cudaStream_t st) {
-    RVB_REQUIRE(N >= 0 && P > 0 && P <= 65535, "rvb_heightmap_raycast: need N >= 0, 0 < P <= 65535");
-    if (N == 0) return RVB_OK;
-    RVB_REQUIRE(t && pos && euler && pattern && dist, "rvb_heightmap_raycast: null pointer");
-    RVB_REQUIRE(!obs || (col_a && col_b && obs_ld > 0), "rvb_heightmap_raycast: obs needs col_a, col_b, obs_ld");
-    RVB_REQUIRE(!obs_h16 || (col_a && col_b && obs_h16_ld > 0 && obs_h16_col0 >= 0), "rvb_heightmap_raycast: obs_h16 needs col_a, col_b, obs_h16_ld");
-    RVB_REQUIRE(variant >= 0 && variant <= 3, "rvb_heightmap_raycast: variant must be 0, 1, 2 or 3");
-    RVB_REQUIRE(!obs_h16 || variant != 1, "rvb_heightmap_raycast: the per-pair cross-check kernel (variant 1) has no packed output");
-    RVB_REQUIRE(variant != 2 || t->index != nullptr, "rvb_heightmap_raycast: variant 2 reads the index the layer released (rvb_terrain_release_index)");
+int heightmap_raycast(const rvb_terrain* t, const rc::TiledParams& q, int64_t N, int variant, const RaycastKnobs& knobs,
+                      const int32_t* order, cudaStream_t st) {
     if (variant != 1) {
-        rc::TiledParams q;
-        const int frc = fill_tiled_params(t, pos, euler, trig, pattern, P, N, dist, hit_slot, hit_tri, pt, sources, obs, obs_ld,
-                                          obs_h16, obs_h16_ld, obs_h16_col0, col_a, col_b, q);
-        if (frc != RVB_OK) return frc;
         // a layer with more than 2 % of triangles the shadow kernel has no bound for (terrain.cu: n_ill): the tiled kernel is the faster one
         const bool shadow_ok = knobs.force >= 0 ? knobs.force == 1 : t->n_ill * 50 <= t->T;
         if (variant == 0 && t->sb_ids != nullptr && shadow_ok) return launch_shadow(q, N, knobs, order, st);
         return launch_tiled(q, t->blk_ids != nullptr && variant != 2, N * q.tiles, st);
     }
-    RVB_REQUIRE(t->index != nullptr, "rvb_heightmap_raycast: variant 1 reads the index the layer released (rvb_terrain_release_index)");
-    RVB_REQUIRE(N <= 65535, "rvb_heightmap_raycast: variant 1 handles at most 65535 envs per call");
-    __half* src16 = (__half*)sources;
+    __half* src16 = q.sources;
     RvbTemp<__half> scratch;          // the N directions, then (without `sources`) the N * P sources
-    RVB_CUDA(scratch.alloc_pool(3 * (size_t)N + (sources ? 0 : 3 * (size_t)N * P), st));
+    RVB_CUDA(scratch.alloc_pool(3 * (size_t)N + (src16 ? 0 : 3 * (size_t)N * q.P), st));
     __half* dneg = scratch.p;
-    if (!sources) src16 = scratch.p + 3 * N;
-    dim3 grid((unsigned)ceil_div(P, 256), (unsigned)N);
-    hm_setup_kernel<<<grid, 256, 0, st>>>(pos, euler, trig, pattern, (int)P, src16, dneg);
+    if (!src16) src16 = scratch.p + 3 * N;
+    dim3 grid((unsigned)ceil_div(q.P, 256), (unsigned)N);
+    hm_setup_kernel<<<grid, 256, 0, st>>>(q.pos, q.euler, q.trig, q.pattern, q.P, src16, dneg);
     RVB_LAUNCH_CHECK();
-    return launch_cast_simple(t, src16, dneg, N * P, P, dist, hit_slot, hit_tri, pt, obs, obs_ld, col_a, col_b, st);
+    return launch_cast_simple(t, src16, dneg, N * q.P, q.P, q.dist, q.hit_slot, q.hit_tri, q.pt, q.obs, q.obs_ld, q.col_a, q.col_b, st);
 }
 
 extern "C" int rvb_heightmap_raycast(const rvb_terrain* t, const float* pos, const float* euler, const float* trig,
@@ -165,8 +148,14 @@ extern "C" int rvb_heightmap_raycast(const rvb_terrain* t, const float* pos, con
     RaycastKnobs knobs;
     const int krc = read_raycast_knobs(knobs);
     if (krc != RVB_OK) return krc;
-    return heightmap_raycast(t, pos, euler, trig, pattern, P, N, dist, hit_slot, hit_tri, pt, sources, obs, obs_ld, obs_h16,
-                             obs_h16_ld, obs_h16_col0, col_a, col_b, variant, knobs, nullptr, as_stream(stream));
+    rc::TiledParams q{};
+    q.pos = pos; q.euler = euler; q.trig = trig; q.pattern = pattern;
+    q.dist = (__half*)dist; q.hit_slot = hit_slot; q.hit_tri = hit_tri; q.pt = (__half*)pt; q.sources = (__half*)sources;
+    q.obs = obs; q.obs_ld = obs_ld; q.col_a = col_a; q.col_b = col_b;
+    q.obs16 = (__half*)obs_h16; q.obs16_ld = obs_h16_ld; q.obs16_col0 = obs_h16_col0;
+    const int prc = fill_tiled_params(t, P, N, variant, q);
+    if (prc != RVB_OK || N == 0) return prc;
+    return heightmap_raycast(t, q, N, variant, knobs, nullptr, as_stream(stream));
 }
 
 extern "C" int rvb_cast_rays(const rvb_terrain* t, const uint16_t* sources, const uint16_t* directions, int64_t R,
@@ -179,7 +168,8 @@ extern "C" int rvb_cast_rays(const rvb_terrain* t, const uint16_t* sources, cons
     RvbTemp<__half> dneg;
     RVB_CUDA(dneg.alloc_pool(3 * (size_t)R, st));
     normalize_dirs_kernel<<<(unsigned)ceil_div(R, 256), 256, 0, st>>>((const __half*)directions, R, dneg.p);
-    return launch_cast_simple(t, (const __half*)sources, dneg.p, R, 1, dist, hit_slot, hit_tri, pt, nullptr, 0, nullptr, nullptr, st);
+    return launch_cast_simple(t, (const __half*)sources, dneg.p, R, 1, (__half*)dist, hit_slot, hit_tri, (__half*)pt, nullptr, 0, nullptr,
+                              nullptr, st);
 }
 
 // ------------------------------------------------------------------------------------------------

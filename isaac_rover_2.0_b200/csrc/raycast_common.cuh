@@ -19,29 +19,27 @@ struct RaycastKnobs {
 int read_raycast_knobs(RaycastKnobs& k);
 
 namespace rc { struct TiledParams; }
-// rvb_heightmap_raycast (raycast.cu) fills one parameter block from its arguments and hands it to a launcher.
-// fill_tiled_params (raycast_tiled.cu): the layer's lists and grid, the call's inputs and outputs, the tiling of the P rays.
-int fill_tiled_params(const rvb_terrain* t, const float* pos, const float* euler, const float* trig, const double* pattern,
-                      int64_t P, int64_t N, uint16_t* dist, int32_t* hit_slot, int32_t* hit_tri, uint16_t* pt,
-                      uint16_t* sources, float* obs, int64_t obs_ld, uint16_t* obs_h16, int64_t obs_h16_ld, int obs_h16_col0,
-                      const int32_t* col_a, const int32_t* col_b, rc::TiledParams& q);
+// rvb_heightmap_raycast (raycast.cu) and rvb_env_post (step.cu) set the call's inputs and outputs in one parameter block and hand
+// it to heightmap_raycast.
+// fill_tiled_params (raycast_tiled.cu): checks a ray-cast of P rays over N envs with `variant` and q's inputs and outputs, and
+// fills in the rest of q (zero-initialised by the caller): the layer's lists and grid, P and the tiling of the P rays.  With
+// N == 0 it checks N and P alone and leaves q as it is.
+int fill_tiled_params(const rvb_terrain* t, int64_t P, int64_t N, int variant, rc::TiledParams& q);
 // launch_tiled (raycast_tiled.cu): q.work_list / q.work_count set: `grid` CTAs loop over the list; otherwise one CTA per
 // (env, tile).  `blocks`: the 3x3-cell block lists instead of the K-contiguous index.
 int launch_tiled(const rc::TiledParams& q, bool blocks, int64_t grid, cudaStream_t st);
-// build_env_order (raycast_shadow.cu): order[0 .. N) = the envs in the order the shadow kernel and the rock kernel cast them:
-// envs with tilted rays first (the slow CTAs of the shadow kernel must not start last), within each class by map position
-// (Z-order of 0.8 m cells of t's grid), so that the envs resident on the GPU at one time share their terrain data in L2.
-// Deterministic: equal keys keep index order.
-int build_env_order(const rvb_terrain* t, const float* pos, const float* euler, const float* trig, int64_t N, float cos_steep,
-                    int32_t* order, cudaStream_t st);
+// build_env_order (raycast_shadow.cu): order[0 .. N) = the envs of q (filled by fill_tiled_params) in the order the shadow kernel
+// and the rock kernel cast them: envs with tilted rays first (the slow CTAs of the shadow kernel must not start last), within
+// each class by map position (Z-order of 0.8 m cells of the layer's grid), so that the envs resident on the GPU at one time share
+// their terrain data in L2.  Deterministic: equal keys keep index order.
+int build_env_order(const rc::TiledParams& q, int64_t N, float cos_steep, int32_t* order, cudaStream_t st);
 // launch_shadow (raycast_shadow.cu): the shadow kernel over N envs in `order` (null: it builds the order itself), with the tiled
 // kernel for the envs and tiles it leaves.
 int launch_shadow(rc::TiledParams q, int64_t N, const RaycastKnobs& knobs, const int32_t* order, cudaStream_t st);
-// heightmap_raycast (raycast.cu): rvb_heightmap_raycast with the knobs already read and the env order of the shadow kernel (or null).
-int heightmap_raycast(const rvb_terrain* t, const float* pos, const float* euler, const float* trig, const double* pattern,
-                      int64_t P, int64_t N, uint16_t* dist, int32_t* hit_slot, int32_t* hit_tri, uint16_t* pt, uint16_t* sources,
-                      float* obs, int64_t obs_ld, uint16_t* obs_h16, int64_t obs_h16_ld, int obs_h16_col0, const int32_t* col_a,
-                      const int32_t* col_b, int variant, const RaycastKnobs& knobs, const int32_t* order, cudaStream_t st);
+// heightmap_raycast (raycast.cu): the ray-cast of q (filled by fill_tiled_params) with the knobs already read and, for the shadow
+// route, the env order of the shadow kernel (or null).
+int heightmap_raycast(const rvb_terrain* t, const rc::TiledParams& q, int64_t N, int variant, const RaycastKnobs& knobs,
+                      const int32_t* order, cudaStream_t st);
 // rock_collision (rock.cu): rvb_rock_collision with the envs taken in `order` (null: index order); outputs stay indexed by env.
 int rock_collision(const rvb_terrain* t, const float* pos, const float* euler, const float* trig, const float* joints,
                    const float* joint_trig, int64_t N, uint16_t* wheel_dist, uint16_t* body_dist, int32_t* hit_tri,

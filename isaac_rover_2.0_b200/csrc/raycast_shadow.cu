@@ -37,7 +37,6 @@
 #include <ctype.h>
 #include <errno.h>
 #include <stdlib.h>
-#include <string.h>
 
 #include <cub/device/device_radix_sort.cuh>
 
@@ -977,16 +976,10 @@ static int sort_envs(const rc::TiledParams& q, int64_t N, int32_t* order, int* s
     return RVB_OK;
 }
 
-int build_env_order(const rvb_terrain* t, const float* pos, const float* euler, const float* trig, int64_t N, float cos_steep,
-                    int32_t* order, cudaStream_t st) {
-    RVB_REQUIRE(t && t->G0 >= 1 && t->G1 >= 1 && t->G0 <= (1 << 18) && t->G1 <= (1 << 18), "env order: grid wider than 2^18 cells");
-    rc::TiledParams q;
-    memset(&q, 0, sizeof(q));
-    q.G0 = (int)t->G0; q.G1 = (int)t->G1;
-    q.res = t->res; q.inv_res = 1.0f / t->res; q.shift_x = t->shift_x; q.shift_y = t->shift_y; q.sem = t->sem;
-    q.pos = pos; q.euler = euler; q.trig = trig;
-    q.cos_steep = cos_steep;
-    return sort_envs(q, N, order, nullptr, nullptr, st);
+int build_env_order(const rc::TiledParams& q, int64_t N, float cos_steep, int32_t* order, cudaStream_t st) {
+    rc::TiledParams c = q;
+    c.cos_steep = cos_steep;
+    return sort_envs(c, N, order, nullptr, nullptr, st);
 }
 
 int launch_shadow(rc::TiledParams q, int64_t N, const RaycastKnobs& knobs, const int32_t* order, cudaStream_t st) {
@@ -1032,7 +1025,9 @@ int launch_shadow(rc::TiledParams q, int64_t N, const RaycastKnobs& knobs, const
     RVB_CUDA(rvb_side_stream(1, &side));
     if (order) {
         // the caller's order (the fused step builds one for the ray-cast and the rock kernel): this launch only makes the steep
-        // list, whose slots depend on this call's tiling (it recomputes every env's ray direction, one thread per env)
+        // list.  The caller's classify launch could make it too, but its count would then need a memset in front of the caller's
+        // fork of the rock kernel, on the step's critical path; this launch runs after the fork, while the shadow kernel waits for
+        // the rock kernel's CTAs, and costs nothing measurable (profiles/r8_env_plan_check.txt)
         hm_classify_kernel<<<(unsigned)ceil_div(N, 256), 256, 0, st>>>(q, N, 0, nullptr, nullptr, counts, steep_list);
         RVB_LAUNCH_CHECK();
         q.order = order;

@@ -21,8 +21,6 @@
 //      (NaN first, ties -> lowest slot), merged across candidate chunks with a shared-memory atomicMin;
 //   6. epilogue in ray order: coalesced stores of dist / hit slot / hit triangle / pt / sources and the fused
 //      sparse+dense observation columns (heightmap_distribution.py:126-133, rover.py:324-325).
-#include <string.h>
-
 #include "raycast_common.cuh"
 
 namespace {
@@ -357,28 +355,31 @@ size_t tiled_smem_bytes(int RT) {
 
 }  // namespace
 
-int fill_tiled_params(const rvb_terrain* t, const float* pos, const float* euler, const float* trig, const double* pattern,
-                      int64_t P, int64_t N, uint16_t* dist, int32_t* hit_slot, int32_t* hit_tri, uint16_t* pt,
-                      uint16_t* sources, float* obs, int64_t obs_ld, uint16_t* obs_h16, int64_t obs_h16_ld, int obs_h16_col0,
-                      const int32_t* col_a, const int32_t* col_b, rc::TiledParams& q) {
-    RVB_REQUIRE(t->G0 <= 32767 && t->G1 <= 65535, "heightmap ray-cast: grid larger than 32767 x 65535 cells");
-    RVB_REQUIRE(t->K <= 16383, "heightmap ray-cast: K > 16383");
-    RVB_REQUIRE(t->G0 * t->G1 < ((int64_t)1 << 32), "heightmap ray-cast: more than 2^32 cells");
-    memset(&q, 0, sizeof(q));
+int fill_tiled_params(const rvb_terrain* t, int64_t P, int64_t N, int variant, rc::TiledParams& q) {
+    RVB_REQUIRE(N >= 0 && P > 0 && P <= 65535, "rvb_heightmap_raycast: need N >= 0, 0 < P <= 65535");
+    if (N == 0) return RVB_OK;
+    RVB_REQUIRE(t && q.pos && q.euler && q.pattern && q.dist, "rvb_heightmap_raycast: null pointer");
+    RVB_REQUIRE(!q.obs || (q.col_a && q.col_b && q.obs_ld > 0), "rvb_heightmap_raycast: obs needs col_a, col_b, obs_ld");
+    RVB_REQUIRE(!q.obs16 || (q.col_a && q.col_b && q.obs16_ld > 0 && q.obs16_col0 >= 0), "rvb_heightmap_raycast: obs_h16 needs col_a, col_b, obs_h16_ld");
+    RVB_REQUIRE(variant >= 0 && variant <= 3, "rvb_heightmap_raycast: variant must be 0, 1, 2 or 3");
+    RVB_REQUIRE(!q.obs16 || variant != 1, "rvb_heightmap_raycast: the per-pair cross-check kernel (variant 1) has no packed output");
+    RVB_REQUIRE(variant != 2 || t->index != nullptr, "rvb_heightmap_raycast: variant 2 reads the index the layer released (rvb_terrain_release_index)");
+    if (variant == 1) {
+        RVB_REQUIRE(t->index != nullptr, "rvb_heightmap_raycast: variant 1 reads the index the layer released (rvb_terrain_release_index)");
+        RVB_REQUIRE(N <= 65535, "rvb_heightmap_raycast: variant 1 handles at most 65535 envs per call");
+    } else {
+        RVB_REQUIRE(t->G0 <= 32767 && t->G1 <= 65535, "heightmap ray-cast: grid larger than 32767 x 65535 cells");
+        RVB_REQUIRE(t->K <= 16383, "heightmap ray-cast: K > 16383");
+        RVB_REQUIRE(t->G0 * t->G1 < ((int64_t)1 << 32), "heightmap ray-cast: more than 2^32 cells");
+    }
     q.index = t->index; q.recs = t->recs; q.s1 = t->s1recs;
     q.blk_off = t->blk_off; q.blk_ids = t->blk_ids; q.blk_slots = t->blk_slots; q.nBy = t->nBy;
     q.sb_off = t->sb_off; q.sb_ids = t->sb_ids; q.sb_slot9 = t->sb_slot9; q.sb_chunk = t->sb_chunk; q.nSBy = t->nSBy;
     q.G0 = (int)t->G0; q.G1 = (int)t->G1; q.K = (int)t->K; q.Ks = (int)t->Ks;
     q.res = t->res; q.inv_res = 1.0f / t->res; q.shift_x = t->shift_x; q.shift_y = t->shift_y; q.sem = t->sem;
-    q.pos = pos; q.euler = euler; q.trig = trig; q.pattern = pattern;
     q.P = (int)P;
     q.tiles = (int)ceil_div(P, RT_MAX);
     q.tile_size = (int)ceil_div(P, q.tiles);
-    q.dist = (__half*)dist; q.hit_slot = hit_slot; q.hit_tri = hit_tri; q.pt = (__half*)pt; q.sources = (__half*)sources;
-    q.obs = obs; q.obs_ld = obs_ld; q.col_a = col_a; q.col_b = col_b;
-    if (obs_h16) {
-        q.obs16 = (__half*)obs_h16; q.obs16_ld = obs_h16_ld; q.obs16_col0 = obs_h16_col0;
-    }
     RVB_REQUIRE(N * q.tiles < ((int64_t)1 << 31), "heightmap ray-cast: too many (env, tile) blocks for one launch");
     return RVB_OK;
 }

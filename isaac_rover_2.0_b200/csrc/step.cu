@@ -86,10 +86,19 @@ extern "C" int rvb_env_post(const rvb_terrain* terrain, const rvb_terrain* rocks
     RVB_REQUIRE(p->curriculum_level < 2 || (rocks && io.wheel_dist && io.body_dist && io.rock_collision),
                 "rvb_env_post: curriculum_level >= 2 needs the rock layer and its outputs");
     cudaStream_t st = as_stream(stream);
-    // the knobs are read before the first launch, so that a bad knob fails the call before anything is launched
+    // the knobs are read and the ray-cast's arguments checked before the first launch, so that a bad knob or argument fails the
+    // call before anything is launched
     RaycastKnobs knobs;
     const int krc = read_raycast_knobs(knobs);
     if (krc != RVB_OK) return krc;
+    // packed observation requested: the heightmap columns go to obs_h16 (fp16, what they are by construction) and the f32
+    // columns 4.. of obs are left alone
+    rc::TiledParams q{};
+    q.pos = io.pos; q.euler = io.euler; q.pattern = pattern; q.dist = (__half*)io.dist;
+    q.obs = io.obs_h16 ? nullptr : io.obs; q.obs_ld = io.obs_ld; q.col_a = col_a; q.col_b = col_b;
+    q.obs16 = (__half*)io.obs_h16; q.obs16_ld = io.obs_h16_ld; q.obs16_col0 = 4;
+    const int prc = fill_tiled_params(terrain, P, N, 0, q);
+    if (prc != RVB_OK) return prc;
     env_post_kernel<<<(unsigned)ceil_div(N, 256), 256, 0, st>>>(io, N, (int)H, p->sem);
     RVB_LAUNCH_CHECK();
     cudaEvent_t t0 = nullptr, t1 = nullptr;
@@ -111,7 +120,7 @@ extern "C" int rvb_env_post(const rvb_terrain* terrain, const rvb_terrain* rocks
     // waits for the rock kernel before the order goes back to the pool
     RvbTemp<int32_t> order;
     RVB_CUDA(order.alloc_pool((size_t)N, st));
-    const int orc = build_env_order(terrain, io.pos, io.euler, nullptr, N, knobs.cos_steep, order.p, st);
+    const int orc = build_env_order(q, N, knobs.cos_steep, order.p, st);
     if (orc != RVB_OK) return orc;
     const bool with_rocks = rocks && io.wheel_dist && io.body_dist;
     RvbJoinGuard guard(st);          // on every exit path below: st waits for the rock layer's kernel
@@ -126,10 +135,7 @@ extern "C" int rvb_env_post(const rvb_terrain* terrain, const rvb_terrain* rocks
         RVB_CUDA(cudaEventRecord(side->join, side->s));
         guard.join = side->join;
     }
-    // packed observation requested: the heightmap columns go to obs_h16 (fp16, what they are by construction) and the f32
-    // columns 4.. of obs are left alone
-    int rc = heightmap_raycast(terrain, io.pos, io.euler, nullptr, pattern, P, N, io.dist, nullptr, nullptr, nullptr, nullptr,
-                               io.obs_h16 ? nullptr : io.obs, io.obs_ld, io.obs_h16, io.obs_h16_ld, 4, col_a, col_b, 0, knobs, order.p, st);
+    const int rc = heightmap_raycast(terrain, q, N, 0, knobs, order.p, st);
     if (rc != RVB_OK) return rc;
     if (t1) RVB_CUDA(cudaEventRecord(t1, st));
     if (guard.join) {
